@@ -2,6 +2,7 @@
 """Benchmark of the env-step hot path (BASELINE.json: env-steps/sec, whole box, device-timed).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--scene ball|space] [--envs 65536] [--impl reference]
+                    [--dump-outputs DIR]
 
 Own arm (default): one process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE), each rank steps its own shard of
 `--envs` environments with device-generated random actions (get_random_action, safe_motions_base.py:1327-1328) and
@@ -11,6 +12,8 @@ flushed between timed steps, the max over ranks is taken and rank 0 prints ONE J
 observations / rewards / dones out, copies inside the timed region.
 `--impl reference` times the CPU restatement of the reference path (oracle/, all host threads) on the same workload;
 the real PyBullet/klimits env cannot be installed in this image (no network, SURVEY.md section 8c).
+`--dump-outputs DIR` writes what the last timed step returned (obs, reward, done, info of the headline scene) as
+DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -249,6 +252,26 @@ def _emit(line):
     os.write(_STDOUT_FD if _STDOUT_FD is not None else 1, (line + "\n").encode())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT_BYTES, suffix=""):
+    """Writes each per-env array (first axis: env) as <path>/<name><suffix>.npy, float64 kept, everything else as
+    float32.  When they exceed `limit` bytes together, every array keeps the same fixed, seeded sample of env rows and
+    the sampled env indices go to env_index<suffix>.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64 if np.asarray(v).dtype == np.float64 else np.float32)
+              for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes for v in arrays.values()) // max(n, 1)
+    if n * row_bytes > limit:
+        rows = np.sort(np.random.default_rng(0).choice(n, limit // (row_bytes + 8), replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), v)
+
+
 def bind_to_gpu_cpus(local_rank):
     """Pins this rank to the CPUs nearest to its GPU (NVML's ideal affinity) before any pinned host buffer exists, so
     that the staging buffers of the host-buffer step are first touched on the GPU's own NUMA node.  Returns what was
@@ -290,7 +313,13 @@ def main():
     ap.add_argument("--scenes", default="space,space_bm,ball,human",
                     help="further scenes measured (device-timed, shorter) after the main one and reported under 'scenes'")
     ap.add_argument("--no-scenes", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write obs, reward, done and info of the last timed step of the headline scene as DIR/<name>.npy "
+                         "(float32, at most 64 MiB in all: a fixed, seeded sample of envs beyond that; with several "
+                         "ranks each rank writes <name>_rank<r>.npy)")
     args = ap.parse_args()
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the device step (--impl b200)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -304,11 +333,9 @@ def main():
             return 0
         # bounded sample: small shards so that `steps` finish within minutes on the host cores
         per_thread = 1024 if args.scene.startswith("ball") else 8 if args.scene.startswith("human") else 64
-
-        # each of the K "steps" the driver asks for is one oracle step of the bounded sample; K is capped so that the
-        # run ends within minutes
-        steps = max(1, min(args.steps, 40))
-        val, dt, total, steps = cpu_reference_run(args.scene, per_thread, steps, min(max(args.warmup, 1), 2), threads)
+        # each of the K steps is one oracle step of the bounded sample
+        val, dt, total, steps = cpu_reference_run(args.scene, per_thread, args.steps, min(max(args.warmup, 1), 2),
+                                                  threads)
         sample = "{} host threads x {} envs x {} steps of the same scene ({} env-steps in {:.1f} s)".format(
             threads, per_thread, steps, total, dt)
         _emit(json.dumps({
@@ -331,7 +358,8 @@ def main():
     dev = torch.device("cuda", local_rank)
     fma_peaks = measure_fma_peaks(local_rank)
     main = measure_scene(args.scene, args, dev, rank, world, local_rank, fma_peaks, steps=args.steps,
-                         full=True, with_cpu=(rank == 0 and world == 1 and not args.no_cpu_baseline))
+                         full=True, with_cpu=(rank == 0 and world == 1 and not args.no_cpu_baseline),
+                         dump=args.dump_outputs)
     # the other scenes of BASELINE.json on the same box, so that the driver's record carries the north-star scene (Space,
     # also with the robot of the shipped checkpoints) next to the headline workload: shorter runs, device-timed only
     extra = {}
@@ -395,9 +423,9 @@ def measure_fma_peaks(device_index):
     return {"fp32": f32.value, "fp64": f64.value}
 
 
-def measure_scene(scene_name, args, dev, rank, world, local_rank, fma_peaks, steps, full, with_cpu):
+def measure_scene(scene_name, args, dev, rank, world, local_rank, fma_peaks, steps, full, with_cpu, dump=None):
     """One workload on this rank's GPU: K device-timed steps (max over ranks), roofline of the dominant kernel, and (full)
-    the end-to-end number through the host-buffer API."""
+    the end-to-end number through the host-buffer API.  dump: directory for the outputs of the last timed step."""
     import torch
     import torch.distributed as dist
     from safemotionsrisk_b200.vec_env import SafeMotionsVecEnv
@@ -420,7 +448,7 @@ def measure_scene(scene_name, args, dev, rank, world, local_rank, fma_peaks, ste
         config["workload"] += " + state-action risk network and backup policy in the step loop"
 
     def one_step():
-        env.step_random()
+        return env.step_random()
     sampler = ClockSampler(local_rank) if rank == 0 else None   # started early: nvidia-smi needs ~0.1 s to its first sample
     env.reset()
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
@@ -436,10 +464,13 @@ def measure_scene(scene_name, args, dev, rank, world, local_rank, fma_peaks, ste
     for i in range(steps):
         flush.fill_(i & 0xff)  # evict the env state from L2 (outside the timed region of the step)
         starts[i].record()
-        one_step()
+        last = one_step()
         ends[i].record()
     torch.cuda.synchronize(dev)
     t_wall1 = time.time()
+    if dump is not None:   # read before the counter and kernel-timing passes below step the env again
+        dump_outputs(dump, {k: t.cpu().numpy() for k, t in zip(("obs", "reward", "done", "info"), last)},
+                     limit=DUMP_LIMIT_BYTES // world, suffix="_rank{}".format(rank) if world > 1 else "")
     launches = env.launch_count() - launches0
     step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     total_ms = float(sum(step_ms))

@@ -479,6 +479,26 @@ int smenv_measure_fma_peaks(int device, double* tflops_fp32, double* tflops_fp64
 int smenv_debug_build_lut(const float* xyz, int n, int res, uint32_t* out, int capacity);
 int smenv_debug_lut_cell(float dx, float dy, float dz, int res);
 
+/* Bounding volumes of the human's braking-trajectory check as human_brake_plan_kernel reads them (frame coordinates,
+ * margins included).  Link-group pair g: the pairs (a, b) with a in [gp_a0, gp_a0 + gp_na) on frame gp_fa and b in
+ * [gp_b0, gp_b0 + gp_nb) on frame gp_fb (human frame index; -1 = world, i.e. the table).  Side A is covered by the capsule
+ * of its arm frame (hf_*, arm frames 3, 4, 7, 8 in this order); side B by gp_sb / gp_srb (trunk, frame 0), by the box
+ * gp_bmin / gp_bmax (table, world frame) or by its arm frame's capsule.  Against the table the kernel replaces an arm
+ * capsule by two spheres of radius hf_cover_rad at 1/4 and 3/4 of its segment. */
+typedef struct SmHumanBounds {
+    int32_t n_gp;
+    int32_t gp_fa[8], gp_fb[8], gp_a0[8], gp_na[8], gp_b0[8], gp_nb[8];
+    float gp_ca[8][3], gp_ra[8], gp_cb[8][3], gp_rb[8];   /* bounding spheres of both sides */
+    float gp_bmin[8][3], gp_bmax[8][3];                   /* box of side B */
+    float gp_sa[8][6], gp_sra[8], gp_sb[8][6], gp_srb[8]; /* capsules of both sides: segment end points, radius */
+    int32_t hf_s0[4], hf_sn[4];                           /* shape range of arm frame i */
+    float hf_seg[4][6], hf_rad[4], hf_cover_rad[4];
+} SmHumanBounds;
+
+/* Host-only (no GPU needed): the bounding volumes above for a scene with the human enabled, built by the same code as
+ * smenv_create.  Returns SM_OK or a negative status (the scene is refused for the same reasons as by smenv_create). */
+int smenv_debug_human_bounds(const SmScene* scene, SmHumanBounds* out);
+
 /* Debug: trace of one GJK call between shapes ia and ib for one env state given on the host (trace: 32 x 8 floats per
  * iteration = simplex size, |v|^2, v.w, support ids, v; result: distance, iterations, then the 9 robot frames). */
 int smenv_debug_gjk(SmEnv* env, const double* kin_host, const double* obst_host, int ia, int ib, float upper,

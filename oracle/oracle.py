@@ -88,6 +88,18 @@ def distances(scene, q, obst):
     return ds.value, dse.value, dm.value
 
 
+def distances_h(scene, q, obst, hq):
+    """(d_static, d_self, d_moving) raw (before the 1 mm clamp) for one env of the Human scene, the human at joint
+    angles hq [8]."""
+    q = np.ascontiguousarray(q, dtype=np.float64)
+    ob = np.ascontiguousarray(obst, dtype=np.float64)
+    hq = np.ascontiguousarray(hq, dtype=np.float64)
+    ds, dse, dm = C.c_double(), C.c_double(), C.c_double()
+    lib().smo_distances_h(scene.pointer(), _p(q, C.c_double), _p(ob, C.c_double), _p(hq, C.c_double), C.byref(ds),
+                          C.byref(dse), C.byref(dm))
+    return ds.value, dse.value, dm.value
+
+
 def observation(scene, kin, obst):
     kin = np.ascontiguousarray(kin, dtype=np.float64)
     ob = np.ascontiguousarray(obst, dtype=np.float64)
@@ -118,6 +130,8 @@ class OracleEnvs:
             self.hbrake = np.zeros((n, abi.SM_HBRAKE_STEPS * abi.SM_HUMAN_JOINTS))
             self.hobs = np.zeros((n, abi.SM_HOBS_STRIDE), dtype=np.float32)
             self.hinfo = np.zeros((n, 4), dtype=np.int32)
+            # smallest |d_min - brake_safety| over the poses the last step's braking check visited (inf: no check)
+            self.hmargin = np.full(n, np.inf)
 
     def set_human_state(self, hq, hv, ha, first_target, active_arm):
         """Start state of the nested env: joint state [n, 8], first target point [n, 3] of arm active_arm [n]."""
@@ -146,7 +160,7 @@ class OracleEnvs:
                                    _p(hact, C.c_float), _p(nt, C.c_double) if nt is not None else None,
                                    _p(self.obs, C.c_float), _p(self.hobs, C.c_float), _p(self.reward, C.c_float),
                                    _p(self.done, C.c_uint8), _p(self.term, C.c_int32), _p(self.info, C.c_float),
-                                   _p(self.hinfo, C.c_int32))
+                                   _p(self.hinfo, C.c_int32), _p(self.hmargin, C.c_double))
         return self.obs, self.reward, self.done, self.term, self.info
 
     def set_state(self, q, v, a, obst=None, first_target=None):
@@ -219,16 +233,36 @@ def human_pose_collides(scene, hq):
     return bool(lib().smo_human_pose_collides(scene.pointer(), _p(hq, C.c_double)))
 
 
+def _check_braking(scene, q, v, a, a_target):
+    q, v, a, at = (np.ascontiguousarray(x, dtype=np.float64) for x in (q, v, a, a_target))
+    acc = np.zeros((abi.SM_HBRAKE_STEPS, 8))
+    k, poses, coll, margin = C.c_int(), C.c_int(), C.c_int(), C.c_double()
+    ex = lib().smo_human_check_braking(scene.pointer(), _p(q, C.c_double), _p(v, C.c_double), _p(a, C.c_double),
+                                       _p(at, C.c_double), _p(acc, C.c_double), C.byref(k), C.byref(poses),
+                                       C.byref(coll), C.byref(margin))
+    return bool(ex), acc[:min(k.value, abi.SM_HBRAKE_STEPS)], poses.value, coll.value, margin.value
+
+
 def human_check_braking(scene, q, v, a, a_target):
     """(execute braking?, braking accelerations [k, 8], poses visited, first colliding pose) of the nested env's
     braking-trajectory check (ctlp.py:3026-3207)."""
-    q, v, a, at = (np.ascontiguousarray(x, dtype=np.float64) for x in (q, v, a, a_target))
-    acc = np.zeros((abi.SM_HBRAKE_STEPS, 8))
-    k, poses, coll = C.c_int(), C.c_int(), C.c_int()
-    ex = lib().smo_human_check_braking(scene.pointer(), _p(q, C.c_double), _p(v, C.c_double), _p(a, C.c_double),
-                                       _p(at, C.c_double), _p(acc, C.c_double), C.byref(k), C.byref(poses),
-                                       C.byref(coll))
-    return bool(ex), acc[:min(k.value, abi.SM_HBRAKE_STEPS)], poses.value, coll.value
+    return _check_braking(scene, q, v, a, a_target)[:4]
+
+
+def human_check_braking_margin(scene, q, v, a, a_target):
+    """How far the braking-trajectory check of human_check_braking is from flipping: the smallest |d_min - brake_safety|
+    over the poses it visited, d_min the smallest pair distance of a pose (exact up to 1e-3 m, a lower bound beyond)."""
+    return _check_braking(scene, q, v, a, a_target)[4]
+
+
+def human_brake_pair_distances(scene, hq):
+    """Distance of every pair of the braking check (scene.struct.human.brake_pairs order) at pose hq [8], margins
+    subtracted, without early stop: [n_brake_pairs]."""
+    h = scene.struct.human
+    hq = np.ascontiguousarray(hq, dtype=np.float64)
+    out = np.zeros(h.n_brake_pairs)
+    lib().smo_human_brake_pair_distances(scene.pointer(), _p(hq, C.c_double), _p(out, C.c_double))
+    return out
 
 
 def target_link_point(scene, q):

@@ -685,6 +685,8 @@ typedef struct SmoHumanIO {
     int32_t braked;            /* out: 1 if the stored braking trajectory was executed */
     int32_t brake_poses;       /* out: poses the braking-trajectory check visited */
     int32_t brake_collision;   /* out: 1-based index of the first pose in collision, 0 = none, -1 = timeout */
+    double brake_margin;       /* out: smallest |d_min - brake_safety| over the poses the check visited (see
+                                  smo_human_check_braking) */
     double a1[SM_HUMAN_JOINTS];/* out: end acceleration of the step */
 } SmoHumanIO;
 
@@ -748,6 +750,33 @@ int smo_human_pose_collides(const SmScene* sc, const double* hq) {
         if (d < h->brake_safety) return 1;
     }
     return 0;
+}
+
+/* smallest distance over the pairs of the braking check at pose hq: exact below brake_safety + 1e-3, above that a lower
+ * bound (the GJK search of a pair stops once it is proven that far).  d_min < brake_safety exactly where
+ * smo_human_pose_collides reports a collision (same pair distances). */
+static double human_brake_dmin(const SmScene* sc, const double* hq) {
+    const SmHuman* h = &sc->human;
+    Xf world[1 + SM_MAX_JOINTS], fr[SM_MAX_OBST_FRAMES];
+    xf_identity(&world[0]);
+    smo_human_fk(sc, hq, fr);
+    double dmin = INFINITY;
+    for (int i = 0; i < h->n_brake_pairs; ++i) {
+        double d = pair_distance(sc, h->brake_pairs[i][0], h->brake_pairs[i][1], world, fr, h->brake_safety + 1e-3);
+        if (d < dmin) dmin = d;
+    }
+    return dmin;
+}
+
+/* distance of every pair of the braking check (human.brake_pairs order) at pose hq, GJK without early stop (test hook:
+ * the tests find the pair and link-group pair that decide a pose, and its clearance d - brake_safety) */
+void smo_human_brake_pair_distances(const SmScene* sc, const double* hq, double* out /* [n_brake_pairs] */) {
+    const SmHuman* h = &sc->human;
+    Xf world[1 + SM_MAX_JOINTS], fr[SM_MAX_OBST_FRAMES];
+    xf_identity(&world[0]);
+    smo_human_fk(sc, hq, fr);
+    for (int i = 0; i < h->n_brake_pairs; ++i)
+        out[i] = pair_distance(sc, h->brake_pairs[i][0], h->brake_pairs[i][1], world, fr, 0.0);
 }
 
 /* BrakingTrajectoryGenerator.get_braking_acceleration for one joint (utils/braking_trajectory_generator.py:44-78): a
@@ -818,17 +847,22 @@ static int human_braking_acceleration(const SmScene* sc, const double* q, const 
 /* check_braking_trajectory_method / _check_if_braking_trajectory_is_collision_free (ctlp.py:3026-3053, :3155-3207):
  * execute the next step with a_target, then brake; every step is checked at brake_checks poses.  Returns 1 if the
  * braking trajectory has to be executed instead (collision or timeout).  brake_acc receives the braking accelerations
- * b_1 .. b_k that follow a_target (the part adapt_action keeps, ctlp.py:3096-3119), *k_out their number. */
+ * b_1 .. b_k that follow a_target (the part adapt_action keeps, ctlp.py:3096-3119), *k_out their number.
+ * *margin_out (if not NULL) receives the smallest |d_min - brake_safety| over the poses visited, d_min the smallest pair
+ * distance of a pose (human_brake_dmin: exact up to 1e-3 m, a lower bound beyond): how far the decision is from flipping
+ * under a small error of the distances. */
 int smo_human_check_braking(const SmScene* sc, const double* q0, const double* v0, const double* a0,
                             const double* a_target, double* brake_acc /* [SM_HBRAKE_STEPS][8] */, int* k_out,
-                            int* poses_out, int* collision_out) {
+                            int* poses_out, int* collision_out, double* margin_out) {
     const SmHuman* h = &sc->human;
     const int nj = h->n_joints, C = h->brake_checks;
     double ts = sc->ts;
     double q[SM_HUMAN_JOINTS], v[SM_HUMAN_JOINTS], as[SM_HUMAN_JOINTS], ae[SM_HUMAN_JOINTS];
     memcpy(q, q0, sizeof(q)); memcpy(v, v0, sizeof(v)); memcpy(as, a0, sizeof(as)); memcpy(ae, a_target, sizeof(ae));
     int k = 0, poses = 0;
+    double margin = INFINITY;
     *collision_out = 0;
+    if (margin_out) *margin_out = margin;
     for (;;) {
         /* np.linspace(ts / C, ts, C) */
         double pend[SM_HUMAN_JOINTS];
@@ -839,7 +873,10 @@ int smo_human_check_braking(const SmScene* sc, const double* q0, const double* v
             double pm[SM_HUMAN_JOINTS];
             for (int j = 0; j < nj; ++j) { double vv, aa; interpolate(sc, q[j], v[j], as[j], ae[j], t, &pm[j], &vv, &aa); }
             ++poses;
-            if (smo_human_pose_collides(sc, pm)) { *collision_out = poses; *k_out = k; *poses_out = poses; return 1; }
+            const double dmin = human_brake_dmin(sc, pm);
+            if (fabs(dmin - h->brake_safety) < margin) margin = fabs(dmin - h->brake_safety);
+            if (margin_out) *margin_out = margin;
+            if (dmin < h->brake_safety) { *collision_out = poses; *k_out = k; *poses_out = poses; return 1; }
             if (m == C) memcpy(pend, pm, sizeof(pm));
         }
         /* _compute_next_braking_trajectory_time_step (ctlp.py:3467-3493) */
@@ -864,12 +901,12 @@ static void human_pre_step(const SmScene* sc, SmoHumanIO* H) {
     int32_t code[SM_HUMAN_JOINTS];
     smo_human_safe_range(sc, q, v, a, lo, hi, code);
     for (int j = 0; j < h->n_joints; ++j) H->a1[j] = lo[j] + 0.5 * (H->uh[j] + 1.0) * (hi[j] - lo[j]);
-    H->braked = 0; H->brake_poses = 0; H->brake_collision = 0;
+    H->braked = 0; H->brake_poses = 0; H->brake_collision = 0; H->brake_margin = INFINITY;
     H->hstate[SM_HS_STEPS] += 1.0;
     if (!h->check_braking) return;
     double bacc[SM_HBRAKE_STEPS * SM_HUMAN_JOINTS];
     int k = 0, poses = 0, coll = 0;
-    int execute = smo_human_check_braking(sc, q, v, a, H->a1, bacc, &k, &poses, &coll);
+    int execute = smo_human_check_braking(sc, q, v, a, H->a1, bacc, &k, &poses, &coll, &H->brake_margin);
     H->brake_poses = poses; H->brake_collision = coll;
     int count = (int)H->hstate[SM_HS_BRAKE_COUNT];
     if (execute) { /* get_braking_acceleration (ctlp.py:3000-3024): next acceleration of the stored trajectory */
@@ -1275,11 +1312,12 @@ void smo_step_human(const SmScene* sc, double* kin, double* ob, SmoHumanIO* H, i
 }
 
 /* batch driver of the Human scene.  hactions [n][8]; next_target [n][3] or NULL; hinfo [n][4] = braked, poses visited by
- * the braking-trajectory check, first colliding pose (0 none, -1 timeout), reserved */
+ * the braking-trajectory check, first colliding pose (0 none, -1 timeout), reserved; hmargin [n] or NULL: the check's
+ * smallest |d_min - brake_safety| over the poses it visited (infinite if it did not run) */
 void smo_step_batch_human(const SmScene* sc, int n, double* kin, double* ob, double* hkin, double* hstate, double* hbrake,
                           int32_t* episode, double* ep_return, const float* actions, const float* hactions,
                           const double* next_target, float* obs, float* hobs, float* reward, uint8_t* done,
-                          int32_t* term, float* info, int32_t* hinfo) {
+                          int32_t* term, float* info, int32_t* hinfo, double* hmargin) {
     for (int e = 0; e < n; ++e) {
         double u[SM_MAX_JOINTS], uh[SM_HUMAN_JOINTS];
         SmoStepOut out;
@@ -1299,6 +1337,7 @@ void smo_step_batch_human(const SmScene* sc, int n, double* kin, double* ob, dou
         done[e] = (uint8_t)out.done;
         term[e] = out.term_reason;
         memcpy(info + (size_t)e * SM_INFO_STRIDE, out.info, sizeof(out.info));
+        if (hmargin) hmargin[e] = H.brake_margin;
         if (hinfo) { hinfo[4 * e] = H.braked; hinfo[4 * e + 1] = H.brake_poses; hinfo[4 * e + 2] = H.brake_collision; hinfo[4 * e + 3] = 0; }
     }
 }

@@ -57,6 +57,20 @@ class SmShape(C.Structure):
                 ("center", d * 3), ("radius", d)]
 
 
+class SmHumanBounds(C.Structure):
+    """Bounding volumes of the human's braking-trajectory check (include/smenv.h, smenv_debug_human_bounds)."""
+    f = C.c_float
+    _fields_ = [
+        ("n_gp", i32), ("gp_fa", i32 * 8), ("gp_fb", i32 * 8), ("gp_a0", i32 * 8), ("gp_na", i32 * 8), ("gp_b0", i32 * 8),
+        ("gp_nb", i32 * 8),
+        ("gp_ca", (f * 3) * 8), ("gp_ra", f * 8), ("gp_cb", (f * 3) * 8), ("gp_rb", f * 8),
+        ("gp_bmin", (f * 3) * 8), ("gp_bmax", (f * 3) * 8),
+        ("gp_sa", (f * 6) * 8), ("gp_sra", f * 8), ("gp_sb", (f * 6) * 8), ("gp_srb", f * 8),
+        ("hf_s0", i32 * 4), ("hf_sn", i32 * 4),
+        ("hf_seg", (f * 6) * 4), ("hf_rad", f * 4), ("hf_cover_rad", f * 4)]
+    del f
+
+
 class SmHuman(C.Structure):
     _fields_ = [
         ("enabled", i32), ("n_joints", i32),
@@ -176,7 +190,7 @@ EXPORTED_SYMBOLS = [
     "smenv_last_error", "smenv_abi_version", "smenv_sizeof_scene", "smenv_sizeof_shape", "smenv_create",
     "smenv_destroy", "smenv_pool_sizes", "smenv_fill_pools", "smenv_pool_ptrs", "smenv_copy_pools", "smenv_set_state", "smenv_reset",
     "smenv_step", "smenv_step_random", "smenv_step_host", "smenv_set_step_ranges", "smenv_safe_range", "smenv_distances", "smenv_observation",
-    "smenv_counters", "smenv_enable_counters", "smenv_launch_count", "smenv_debug_gjk", "smenv_debug_build_lut", "smenv_debug_lut_cell", "smenv_kernel_timing",
+    "smenv_counters", "smenv_enable_counters", "smenv_launch_count", "smenv_debug_gjk", "smenv_debug_build_lut", "smenv_debug_lut_cell", "smenv_debug_human_bounds", "smenv_kernel_timing",
     "smenv_kernel_times", "smenv_set_targets", "smenv_mlp_load", "smenv_mlp_forward", "smenv_risk_gate", "smenv_random_actions",
     "smenv_set_seed", "smenv_set_risk_gate", "smenv_set_human_actions_external", "smenv_set_human_state",
     "smenv_human_pool_sizes", "smenv_copy_human_pools", "smenv_measure_fma_peaks", "smenv_launch_config", "smenv_set_gate_exact", "smenv_mlp_forward_exact",

@@ -302,6 +302,143 @@ static int upload(T** dst, const std::vector<T>& src) {
     return SM_OK;
 }
 
+// link-group pairs of the human's braking-trajectory check and the capsules of the arm frames (human_brake_plan_kernel):
+// the pair list sorted by (frame of A, frame of B, A, B), per link-group pair the bounding volumes of both sides.  Host only,
+// shared by smenv_create and smenv_debug_human_bounds; hpairs receives the sorted pair list.
+static int human_brake_bounds(const SmScene* sc, DevHuman& u, std::vector<short>& hpairs) {
+    const SmHuman& h = sc->human;
+    std::vector<std::array<int, 4>> ps;
+    for (int i = 0; i < h.n_brake_pairs; ++i) {
+        const int a = h.brake_pairs[i][0], b = h.brake_pairs[i][1];
+        ps.push_back({sc->shapes[a].frame, sc->shapes[b].frame, a, b});
+    }
+    std::sort(ps.begin(), ps.end());
+    auto bound = [&](const std::vector<int>& ids, float* c, float* r, float* bmin, float* bmax) {
+        float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+        float mrg = 0.f;
+        for (int id : ids) {
+            const SmShape& sh = sc->shapes[id];
+            mrg = fmaxf(mrg, (float)sh.margin);
+            for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i)
+                for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], (float)sc->verts[3 * i + k]); hi[k] = fmaxf(hi[k], (float)sc->verts[3 * i + k]); }
+        }
+        float rad = 0.f;
+        for (int k = 0; k < 3; ++k) { c[k] = 0.5f * (lo[k] + hi[k]); bmin[k] = lo[k] - mrg - 1e-6f; bmax[k] = hi[k] + mrg + 1e-6f; }
+        for (int id : ids) {
+            const SmShape& sh = sc->shapes[id];
+            for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i) {
+                const float dx = (float)sc->verts[3 * i] - c[0], dy = (float)sc->verts[3 * i + 1] - c[1], dz = (float)sc->verts[3 * i + 2] - c[2];
+                rad = fmaxf(rad, sqrtf(dx * dx + dy * dy + dz * dz));
+            }
+        }
+        *r = rad * (1.0f + 1e-6f) + mrg + 1e-6f;
+    };
+    // capsule around a set of shapes: segment along the principal axis of the vertices, radius = largest distance of a
+    // vertex to the segment (+ margin)
+    auto capsule = [&](const std::vector<int>& ids, float* seg, float* r) {
+        std::vector<std::array<double, 3>> pts;
+        double mrg = 0.0;
+        for (int id : ids) {
+            const SmShape& sh = sc->shapes[id];
+            mrg = std::max(mrg, sh.margin);
+            for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i)
+                pts.push_back({sc->verts[3 * i], sc->verts[3 * i + 1], sc->verts[3 * i + 2]});
+        }
+        double m[3] = {0, 0, 0}, C[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
+        for (auto& q : pts) for (int k = 0; k < 3; ++k) m[k] += q[k] / (double)pts.size();
+        for (auto& q : pts)
+            for (int a = 0; a < 3; ++a) for (int b = 0; b < 3; ++b) C[a][b] += (q[a] - m[a]) * (q[b] - m[b]);
+        double u[3] = {1.0, 0.7, 0.3};
+        for (int it = 0; it < 64; ++it) {   // power iteration: dominant eigenvector of the covariance
+            double w[3];
+            for (int a = 0; a < 3; ++a) w[a] = C[a][0] * u[0] + C[a][1] * u[1] + C[a][2] * u[2];
+            const double nrm = sqrt(w[0] * w[0] + w[1] * w[1] + w[2] * w[2]);
+            if (nrm < 1e-30) break;
+            for (int a = 0; a < 3; ++a) u[a] = w[a] / nrm;
+        }
+        double tmin = 1e300, tmax = -1e300;
+        for (auto& q : pts) {
+            const double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
+            tmin = std::min(tmin, t); tmax = std::max(tmax, t);
+        }
+        // pull the end points in by the cross-section radius (a capsule's caps cover the ends)
+        double rad_line = 0.0;
+        for (auto& q : pts) {
+            const double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
+            double d2 = 0.0;
+            for (int a = 0; a < 3; ++a) { const double e = q[a] - m[a] - t * u[a]; d2 += e * e; }
+            rad_line = std::max(rad_line, sqrt(d2));
+        }
+        double t0 = tmin + rad_line, t1 = tmax - rad_line;
+        if (t0 > t1) t0 = t1 = 0.5 * (tmin + tmax);
+        double rad = 0.0;
+        for (auto& q : pts) {
+            double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
+            t = std::min(std::max(t, t0), t1);
+            double d2 = 0.0;
+            for (int a = 0; a < 3; ++a) { const double e = q[a] - m[a] - t * u[a]; d2 += e * e; }
+            rad = std::max(rad, sqrt(d2));
+        }
+        for (int a = 0; a < 3; ++a) { seg[a] = (float)(m[a] + t0 * u[a]); seg[3 + a] = (float)(m[a] + t1 * u[a]); }
+        *r = (float)(rad * (1.0 + 1e-5) + mrg + 1e-5);
+    };
+    int ngp = 0;
+    for (size_t i = 0; i < ps.size();) {
+        size_t e = i;
+        while (e < ps.size() && ps[e][0] == ps[i][0] && ps[e][1] == ps[i][1]) ++e;
+        if (ngp >= 8) return fail(SM_ERR_SCENE, "the human's braking-trajectory check has more than 8 link-group pairs");
+        std::vector<int> ia, ib;
+        for (size_t q = i; q < e; ++q) { ia.push_back(ps[q][2]); ib.push_back(ps[q][3]); }
+        u.gp_fa[ngp] = ps[i][0] - 100; u.gp_fb[ngp] = ps[i][1] >= 100 ? ps[i][1] - 100 : -1;   // -1: world frame
+        u.gp_off[ngp] = (int)i; u.gp_cnt[ngp] = (int)(e - i);
+        {   // the device code walks a group pair as two nested shape ranges
+            std::vector<int> ua(ia), ub(ib);
+            std::sort(ua.begin(), ua.end()); ua.erase(std::unique(ua.begin(), ua.end()), ua.end());
+            std::sort(ub.begin(), ub.end()); ub.erase(std::unique(ub.begin(), ub.end()), ub.end());
+            const bool dense = ua.size() * ub.size() == e - i && ua.back() - ua.front() + 1 == (int)ua.size() &&
+                               ub.back() - ub.front() + 1 == (int)ub.size();
+            if (!dense)
+                return fail(SM_ERR_SCENE, "the pairs of the human's braking check between two frames must be the cross "
+                                          "product of two contiguous shape ranges");
+            if (ub.size() > 32) return fail(SM_ERR_SCENE, "braking check: more than 32 shapes on side B of a link-group pair");
+            u.gp_a0[ngp] = ua.front(); u.gp_na[ngp] = (int)ua.size();
+            u.gp_b0[ngp] = ub.front(); u.gp_nb[ngp] = (int)ub.size();
+        }
+        float dmin[3], dmax[3];
+        bound(ia, u.gp_ca[ngp], &u.gp_ra[ngp], dmin, dmax);
+        bound(ib, u.gp_cb[ngp], &u.gp_rb[ngp], u.gp_bmin[ngp], u.gp_bmax[ngp]);
+        capsule(ia, u.gp_sa[ngp], &u.gp_sra[ngp]);
+        capsule(ib, u.gp_sb[ngp], &u.gp_srb[ngp]);
+        ++ngp;
+        i = e;
+    }
+    u.n_gp = ngp;
+    // arm frames 3, 4, 7, 8: shape range and capsule (side A of every group pair is one of them)
+    const int arm_frames[4] = {103, 104, 107, 108};
+    for (int fi = 0; fi < 4; ++fi) {
+        std::vector<int> ids;
+        for (int q = 0; q < h.n_arm_shapes; ++q)
+            if (sc->shapes[h.shape_off + q].frame == arm_frames[fi]) ids.push_back(h.shape_off + q);
+        u.hf_s0[fi] = ids.empty() ? h.shape_off : ids.front(); u.hf_sn[fi] = (int)ids.size();
+        if (!ids.empty() && ids.back() - ids.front() + 1 != (int)ids.size())
+            return fail(SM_ERR_SCENE, "the shapes of a human arm frame must be contiguous");
+        for (int k = 0; k < 6; ++k) u.hf_seg[fi][k] = 0.f;
+        u.hf_rad[fi] = 0.f;
+        if (!ids.empty()) capsule(ids, u.hf_seg[fi], &u.hf_rad[fi]);
+    }
+    for (int g = 0; g < ngp; ++g) {
+        const int fa = u.gp_fa[g], fb = u.gp_fb[g];
+        const bool arm_a = fa == 3 || fa == 4 || fa == 7 || fa == 8, arm_b = fb == 3 || fb == 4 || fb == 7 || fb == 8;
+        if (!arm_a || !(arm_b || fb == 0 || fb == -1))
+            return fail(SM_ERR_SCENE, "braking check: side A must be an arm frame, side B an arm frame, the trunk or the world");
+        if (h.n_arm_shapes > 32) return fail(SM_ERR_SCENE, "braking check: more than 32 arm shapes");
+        if (fb == 0 && (u.gp_b0[g] < h.shape_off + h.n_arm_shapes || h.n_shapes - h.n_arm_shapes > 32))
+            return fail(SM_ERR_SCENE, "braking check: trunk shapes must follow the arm shapes (at most 32)");
+    }
+    for (auto& q : ps) { hpairs.push_back((short)q[2]); hpairs.push_back((short)q[3]); }
+    return SM_OK;
+}
+
 extern "C" int smenv_destroy(SmEnv* env);
 // frees a half-built env on every early return of smenv_create
 struct CreateGuard {
@@ -635,137 +772,7 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
                 tmax = fmaxf(tmax, (float)h.contact_thresh[l][r]);
             }
         u.contact_thresh_max = tmax;
-        {   // pair list sorted by (frame of A, frame of B, A, B); link-group pairs with the bounding volumes of both sides
-            std::vector<std::array<int, 4>> ps;
-            for (int i = 0; i < h.n_brake_pairs; ++i) {
-                const int a = h.brake_pairs[i][0], b = h.brake_pairs[i][1];
-                ps.push_back({sc->shapes[a].frame, sc->shapes[b].frame, a, b});
-            }
-            std::sort(ps.begin(), ps.end());
-            auto bound = [&](const std::vector<int>& ids, float* c, float* r, float* bmin, float* bmax) {
-                float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
-                float mrg = 0.f;
-                for (int id : ids) {
-                    const SmShape& sh = sc->shapes[id];
-                    mrg = fmaxf(mrg, (float)sh.margin);
-                    for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i)
-                        for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], (float)sc->verts[3 * i + k]); hi[k] = fmaxf(hi[k], (float)sc->verts[3 * i + k]); }
-                }
-                float rad = 0.f;
-                for (int k = 0; k < 3; ++k) { c[k] = 0.5f * (lo[k] + hi[k]); bmin[k] = lo[k] - mrg - 1e-6f; bmax[k] = hi[k] + mrg + 1e-6f; }
-                for (int id : ids) {
-                    const SmShape& sh = sc->shapes[id];
-                    for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i) {
-                        const float dx = (float)sc->verts[3 * i] - c[0], dy = (float)sc->verts[3 * i + 1] - c[1], dz = (float)sc->verts[3 * i + 2] - c[2];
-                        rad = fmaxf(rad, sqrtf(dx * dx + dy * dy + dz * dz));
-                    }
-                }
-                *r = rad * (1.0f + 1e-6f) + mrg + 1e-6f;
-            };
-            // capsule around a set of shapes: segment along the principal axis of the vertices, radius = largest distance of a
-            // vertex to the segment (+ margin)
-            auto capsule = [&](const std::vector<int>& ids, float* seg, float* r) {
-                std::vector<std::array<double, 3>> pts;
-                double mrg = 0.0;
-                for (int id : ids) {
-                    const SmShape& sh = sc->shapes[id];
-                    mrg = std::max(mrg, sh.margin);
-                    for (int i = sh.vert_off; i < sh.vert_off + sh.vert_cnt; ++i)
-                        pts.push_back({sc->verts[3 * i], sc->verts[3 * i + 1], sc->verts[3 * i + 2]});
-                }
-                double m[3] = {0, 0, 0}, C[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
-                for (auto& q : pts) for (int k = 0; k < 3; ++k) m[k] += q[k] / (double)pts.size();
-                for (auto& q : pts)
-                    for (int a = 0; a < 3; ++a) for (int b = 0; b < 3; ++b) C[a][b] += (q[a] - m[a]) * (q[b] - m[b]);
-                double u[3] = {1.0, 0.7, 0.3};
-                for (int it = 0; it < 64; ++it) {   // power iteration: dominant eigenvector of the covariance
-                    double w[3];
-                    for (int a = 0; a < 3; ++a) w[a] = C[a][0] * u[0] + C[a][1] * u[1] + C[a][2] * u[2];
-                    const double nrm = sqrt(w[0] * w[0] + w[1] * w[1] + w[2] * w[2]);
-                    if (nrm < 1e-30) break;
-                    for (int a = 0; a < 3; ++a) u[a] = w[a] / nrm;
-                }
-                double tmin = 1e300, tmax = -1e300;
-                for (auto& q : pts) {
-                    const double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
-                    tmin = std::min(tmin, t); tmax = std::max(tmax, t);
-                }
-                // pull the end points in by the cross-section radius (a capsule's caps cover the ends)
-                double rad_line = 0.0;
-                for (auto& q : pts) {
-                    const double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
-                    double d2 = 0.0;
-                    for (int a = 0; a < 3; ++a) { const double e = q[a] - m[a] - t * u[a]; d2 += e * e; }
-                    rad_line = std::max(rad_line, sqrt(d2));
-                }
-                double t0 = tmin + rad_line, t1 = tmax - rad_line;
-                if (t0 > t1) t0 = t1 = 0.5 * (tmin + tmax);
-                double rad = 0.0;
-                for (auto& q : pts) {
-                    double t = (q[0] - m[0]) * u[0] + (q[1] - m[1]) * u[1] + (q[2] - m[2]) * u[2];
-                    t = std::min(std::max(t, t0), t1);
-                    double d2 = 0.0;
-                    for (int a = 0; a < 3; ++a) { const double e = q[a] - m[a] - t * u[a]; d2 += e * e; }
-                    rad = std::max(rad, sqrt(d2));
-                }
-                for (int a = 0; a < 3; ++a) { seg[a] = (float)(m[a] + t0 * u[a]); seg[3 + a] = (float)(m[a] + t1 * u[a]); }
-                *r = (float)(rad * (1.0 + 1e-5) + mrg + 1e-5);
-            };
-            int ngp = 0;
-            for (size_t i = 0; i < ps.size();) {
-                size_t e = i;
-                while (e < ps.size() && ps[e][0] == ps[i][0] && ps[e][1] == ps[i][1]) ++e;
-                if (ngp >= 8) return fail(SM_ERR_SCENE, "the human's braking-trajectory check has more than 8 link-group pairs");
-                std::vector<int> ia, ib;
-                for (size_t q = i; q < e; ++q) { ia.push_back(ps[q][2]); ib.push_back(ps[q][3]); }
-                u.gp_fa[ngp] = ps[i][0] - 100; u.gp_fb[ngp] = ps[i][1] >= 100 ? ps[i][1] - 100 : -1;   // -1: world frame
-                u.gp_off[ngp] = (int)i; u.gp_cnt[ngp] = (int)(e - i);
-                {   // the device code walks a group pair as two nested shape ranges
-                    std::vector<int> ua(ia), ub(ib);
-                    std::sort(ua.begin(), ua.end()); ua.erase(std::unique(ua.begin(), ua.end()), ua.end());
-                    std::sort(ub.begin(), ub.end()); ub.erase(std::unique(ub.begin(), ub.end()), ub.end());
-                    const bool dense = ua.size() * ub.size() == e - i && ua.back() - ua.front() + 1 == (int)ua.size() &&
-                                       ub.back() - ub.front() + 1 == (int)ub.size();
-                    if (!dense)
-                        return fail(SM_ERR_SCENE, "the pairs of the human's braking check between two frames must be the cross "
-                                                  "product of two contiguous shape ranges");
-                    if (ub.size() > 32) return fail(SM_ERR_SCENE, "braking check: more than 32 shapes on side B of a link-group pair");
-                    u.gp_a0[ngp] = ua.front(); u.gp_na[ngp] = (int)ua.size();
-                    u.gp_b0[ngp] = ub.front(); u.gp_nb[ngp] = (int)ub.size();
-                }
-                float dmin[3], dmax[3];
-                bound(ia, u.gp_ca[ngp], &u.gp_ra[ngp], dmin, dmax);
-                bound(ib, u.gp_cb[ngp], &u.gp_rb[ngp], u.gp_bmin[ngp], u.gp_bmax[ngp]);
-                capsule(ia, u.gp_sa[ngp], &u.gp_sra[ngp]);
-                capsule(ib, u.gp_sb[ngp], &u.gp_srb[ngp]);
-                ++ngp;
-                i = e;
-            }
-            u.n_gp = ngp;
-            // arm frames 3, 4, 7, 8: shape range and capsule (side A of every group pair is one of them)
-            const int arm_frames[4] = {103, 104, 107, 108};
-            for (int fi = 0; fi < 4; ++fi) {
-                std::vector<int> ids;
-                for (int q = 0; q < h.n_arm_shapes; ++q)
-                    if (sc->shapes[h.shape_off + q].frame == arm_frames[fi]) ids.push_back(h.shape_off + q);
-                u.hf_s0[fi] = ids.empty() ? h.shape_off : ids.front(); u.hf_sn[fi] = (int)ids.size();
-                if (!ids.empty() && ids.back() - ids.front() + 1 != (int)ids.size())
-                    return fail(SM_ERR_SCENE, "the shapes of a human arm frame must be contiguous");
-                for (int k = 0; k < 6; ++k) u.hf_seg[fi][k] = 0.f;
-                u.hf_rad[fi] = 0.f;
-                if (!ids.empty()) capsule(ids, u.hf_seg[fi], &u.hf_rad[fi]);
-            }
-            for (int g = 0; g < ngp; ++g) {
-                const int fa = u.gp_fa[g], fb = u.gp_fb[g];
-                const bool arm_a = fa == 3 || fa == 4 || fa == 7 || fa == 8, arm_b = fb == 3 || fb == 4 || fb == 7 || fb == 8;
-                if (!arm_a || !(arm_b || fb == 0 || fb == -1))
-                    return fail(SM_ERR_SCENE, "braking check: side A must be an arm frame, side B an arm frame, the trunk or the world");
-                if (h.n_arm_shapes > 32) return fail(SM_ERR_SCENE, "braking check: more than 32 arm shapes");
-                if (fb == 0 && (u.gp_b0[g] < h.shape_off + h.n_arm_shapes || h.n_shapes - h.n_arm_shapes > 32))
-                    return fail(SM_ERR_SCENE, "braking check: trunk shapes must follow the arm shapes (at most 32)");
-            }
-            for (auto& q : ps) { hpairs.push_back((short)q[2]); hpairs.push_back((short)q[3]); }
-        }
+        if (const int rc_b = human_brake_bounds(sc, u, hpairs)) return rc_b;
         // link groups: runs of consecutive human shapes in the same frame, with a bounding sphere in frame coordinates
         int ng = 0;
         for (int s = 0; s < h.n_shapes;) {
@@ -2196,6 +2203,35 @@ extern "C" int smenv_debug_build_lut(const float* xyz, int n, int res, uint32_t*
     return (int)t.size();
 }
 extern "C" int smenv_debug_lut_cell(float dx, float dy, float dz, int res) { return lut_cell_res(dx, dy, dz, res); }
+
+extern "C" int smenv_debug_human_bounds(const SmScene* sc, SmHumanBounds* out) {
+    if (!sc || !out) return fail(SM_ERR_ARG, "null argument");
+    if (!sc->human.enabled) return fail(SM_ERR_ARG, "smenv_debug_human_bounds: the scene has no human");
+    DevHuman u;
+    memset(&u, 0, sizeof(u));
+    std::vector<short> hpairs;
+    if (const int rc = human_brake_bounds(sc, u, hpairs)) return rc;
+    memset(out, 0, sizeof(*out));
+    out->n_gp = u.n_gp;
+    for (int g = 0; g < 8; ++g) {
+        out->gp_fa[g] = u.gp_fa[g]; out->gp_fb[g] = u.gp_fb[g];
+        out->gp_a0[g] = u.gp_a0[g]; out->gp_na[g] = u.gp_na[g]; out->gp_b0[g] = u.gp_b0[g]; out->gp_nb[g] = u.gp_nb[g];
+        out->gp_ra[g] = u.gp_ra[g]; out->gp_rb[g] = u.gp_rb[g]; out->gp_sra[g] = u.gp_sra[g]; out->gp_srb[g] = u.gp_srb[g];
+        for (int k = 0; k < 3; ++k) {
+            out->gp_ca[g][k] = u.gp_ca[g][k]; out->gp_cb[g][k] = u.gp_cb[g][k];
+            out->gp_bmin[g][k] = u.gp_bmin[g][k]; out->gp_bmax[g][k] = u.gp_bmax[g][k];
+        }
+        for (int k = 0; k < 6; ++k) { out->gp_sa[g][k] = u.gp_sa[g][k]; out->gp_sb[g][k] = u.gp_sb[g][k]; }
+    }
+    for (int fi = 0; fi < 4; ++fi) {
+        out->hf_s0[fi] = u.hf_s0[fi]; out->hf_sn[fi] = u.hf_sn[fi]; out->hf_rad[fi] = u.hf_rad[fi];
+        for (int k = 0; k < 6; ++k) out->hf_seg[fi][k] = u.hf_seg[fi][k];
+        const float* s = u.hf_seg[fi];
+        const float dx = s[3] - s[0], dy = s[4] - s[1], dz = s[5] - s[2];
+        out->hf_cover_rad[fi] = table_cover_radius(u.hf_rad[fi], sqrtf(dx * dx + dy * dy + dz * dz));
+    }
+    return SM_OK;
+}
 
 extern "C" int smenv_debug_gjk(SmEnv* env, const double* kin_host, const double* obst_host, int ia, int ib, float upper,
                                float* trace_host /* 32 x 8 */, float* result_host /* 4 + 12 * 9 */) {

@@ -236,6 +236,11 @@ __device__ __forceinline__ float segment_dist2(V3 p1, V3 q1, V3 p2, V3 q2) {
 static size_t human_plan_smem_bytes(int n_arm_shapes) {
     return (size_t)(n_arm_shapes + 8) * 3 * HBP_THREADS * sizeof(float) + HBP_MAX_TRUNK * sizeof(float4) + (64 + 32) * sizeof(float);
 }
+// radius of the two spheres at 1/4 and 3/4 of a capsule's segment (length len) that stand in for the capsule (radius ra)
+// in the test against the table's box: ra + len / 4, since a point of an end cap lies within ra of the segment's end and
+// that end within len / 4 of the nearer centre (sqrt(ra^2 + (len / 4)^2) covers the cylinder only: the capsule's segment
+// is pulled in by its radius, so vertices do lie in the caps).  Host and device: smenv_debug_human_bounds exports it.
+__host__ __device__ __forceinline__ float table_cover_radius(float ra, float len) { return ra + 0.25f * len; }
 __device__ __forceinline__ int hbp_frame_index(int f) { return f == 3 ? 0 : f == 4 ? 1 : f == 7 ? 2 : 3; }
 __device__ __forceinline__ void hbp_pick(int f, const Xf& F3, const Xf& F4, const Xf& F7, const Xf& F8, const Xf& B,
                                          const Xf& world, Xf& out) {
@@ -341,8 +346,7 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
             bool near_g;
             if (fb < 0) {    // the table's box against two spheres that cover the capsule of side A
                 const V3 dl = a1 - a0;
-                const float quarter = 0.25f * sqrtf(dot(dl, dl));
-                const float l = sqrtf(ra * ra + quarter * quarter) * (1.0f + 1e-5f) + safety + 1e-5f;
+                const float l = table_cover_radius(ra, sqrtf(dot(dl, dl))) * (1.0f + 1e-5f) + safety + 1e-5f;
                 near_g = box_dist2(a0 + 0.25f * dl, c_sc.hu.gp_bmin[g], c_sc.hu.gp_bmax[g]) <= l * l ||
                          box_dist2(a0 + 0.75f * dl, c_sc.hu.gp_bmin[g], c_sc.hu.gp_bmax[g]) <= l * l;
             } else {         // capsules of both sides: the arm groups are long and thin

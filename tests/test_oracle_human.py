@@ -161,3 +161,27 @@ def test_oracle_reproduces_human_golden_vectors(scene):
             assert np.array_equal(arr, g["out_" + key][s]), (key, s)
         assert np.array_equal(env.hstate, g["out_hstate"][s], equal_nan=True)
     assert (g["out_hinfo"][:, :, 0] != 0).any() and (g["out_done"] != 0).any()   # the vectors hold braking steps and terminations
+
+
+def test_brake_pair_distances_and_check_margin(scene):
+    """The pair-distance hook agrees with the collision predicate of the braking check, and the check's margin is the
+    distance of its deciding pose from the safety distance (a pose at rest: every visited pose is the start pose)."""
+    rng = np.random.default_rng(3)
+    h = scene.struct.human
+    seen = set()
+    for _ in range(300):
+        hq = rng.uniform(scene.human_pos_lo, scene.human_pos_hi)
+        d = oracle.human_brake_pair_distances(scene, hq)
+        assert d.shape == (h.n_brake_pairs,)
+        dmin = d.min()
+        assert (dmin < h.brake_safety) == oracle.human_pose_collides(scene, hq)
+        seen.add(bool(dmin < h.brake_safety))
+        z = np.zeros(8)
+        ex, _, poses, coll = oracle.human_check_braking(scene, hq, z, z, z)
+        margin = oracle.human_check_braking_margin(scene, hq, z, z, z)
+        assert ex == (dmin < h.brake_safety) and poses >= 1 and coll == (1 if ex else 0)
+        if abs(dmin - h.brake_safety) < 1e-3:
+            assert abs(margin - abs(dmin - h.brake_safety)) < 1e-12
+        else:
+            assert margin >= 1e-3 - 1e-12
+    assert seen == {True, False}

@@ -499,6 +499,29 @@ typedef struct SmHumanBounds {
  * smenv_create.  Returns SM_OK or a negative status (the scene is refused for the same reasons as by smenv_create). */
 int smenv_debug_human_bounds(const SmScene* scene, SmHumanBounds* out);
 
+/* Constants of the distance planning as distance_plan_kernel reads them, from the float32 vertices (frame coordinates).
+ * Per shape: the bounding sphere (center, radius), the box of the core vertices (bmin, bmax), the vertex mean (centroid)
+ * and the support-width table: the largest extent of the core about the centre in any direction of a cube-map cell
+ * (cell of a direction: smenv_debug_lut_cell with res 8).  Per pair of the pair table (static pairs, self pairs, then per
+ * obstacle, per mov_reward shape, per part): pair_tab = shape A | shape B << 12 | class << 24 | (B is in frame 0: box
+ * bound) << 31; pair_rm[0] = sum of the margins as the centroid upper bound subtracts it, pair_rm[1] = what the sphere or
+ * box lower bound subtracts.  self_query: self-collision pairs farther apart are pruned. */
+#define SM_PLAN_HWIDTH_CELLS 384   /* 6 cube-map faces x 8 x 8 cells */
+#define SM_PLAN_MAX_PAIRS 512
+typedef struct SmPlanBounds {
+    int32_t n_shapes, n_pairs_fixed, n_pairs;
+    double self_query;
+    float center[SM_MAX_SHAPES][3], radius[SM_MAX_SHAPES];
+    float bmin[SM_MAX_SHAPES][3], bmax[SM_MAX_SHAPES][3], centroid[SM_MAX_SHAPES][3];
+    uint32_t pair_tab[SM_PLAN_MAX_PAIRS];
+    float pair_rm[SM_PLAN_MAX_PAIRS][2];
+    float hwidth[SM_MAX_SHAPES][SM_PLAN_HWIDTH_CELLS];
+} SmPlanBounds;
+
+/* Host-only (no GPU needed): the constants above for a scene, built by the same code as smenv_create.  Returns SM_OK or a
+ * negative status (the scene is refused for the same reasons as by smenv_create). */
+int smenv_debug_plan_bounds(const SmScene* scene, SmPlanBounds* out);
+
 /* Debug: trace of one GJK call between shapes ia and ib for one env state given on the host (trace: 32 x 8 floats per
  * iteration = simplex size, |v|^2, v.w, support ids, v; result: distance, iterations, then the 9 robot frames). */
 int smenv_debug_gjk(SmEnv* env, const double* kin_host, const double* obst_host, int ia, int ib, float upper,

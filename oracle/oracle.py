@@ -100,6 +100,32 @@ def distances_h(scene, q, obst, hq):
     return ds.value, dse.value, dm.value
 
 
+def pair_classes(scene):
+    """(class, shape A, shape B) of every pair of the distance classes, in the order of pair_distances: [n_pairs, 3],
+    class 0 = static, 1 = self, 2 = moving."""
+    sc = scene.struct
+    rows = [(0, sc.static_pairs[i][0], sc.static_pairs[i][1]) for i in range(sc.n_static_pairs)]
+    rows += [(1, sc.self_pairs[i][0], sc.self_pairs[i][1]) for i in range(sc.n_self_pairs)]
+    rows += [(2, sc.mov_reward[r], sc.obst_shape_off[o] + k) for o in range(sc.n_obstacles)
+             for r in range(sc.n_mov_reward) for k in range(sc.obst_shape_cnt[o])]
+    return np.array(rows, dtype=np.int64).reshape(-1, 3)
+
+
+def pair_distances(scene, q, obst, hq=None):
+    """Distance of every pair of the distance classes (pair_classes order) for one env, margins subtracted, without
+    early stop: [n_pairs].  The class rules of distances() (cap and query filters, inactive ball, latched contact) are
+    not applied; hq: the human's joint angles in the Human scene."""
+    q = np.ascontiguousarray(q, dtype=np.float64)
+    ob = np.ascontiguousarray(obst, dtype=np.float64)
+    hq = None if hq is None else np.ascontiguousarray(hq, dtype=np.float64)
+    sc = scene.struct
+    out = np.zeros(sc.n_static_pairs + sc.n_self_pairs +
+                   sc.n_mov_reward * sum(sc.obst_shape_cnt[o] for o in range(sc.n_obstacles)))
+    lib().smo_plan_pair_distances(scene.pointer(), _p(q, C.c_double), _p(ob, C.c_double),
+                                  _p(hq, C.c_double) if hq is not None else None, _p(out, C.c_double))
+    return out
+
+
 def observation(scene, kin, obst):
     kin = np.ascontiguousarray(kin, dtype=np.float64)
     ob = np.ascontiguousarray(obst, dtype=np.float64)

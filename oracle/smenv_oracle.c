@@ -401,7 +401,11 @@ static int simplex_closest(double S[4][3], int* n, double* v) {
         sub3(b, a, ab); sub3(c, a, ac); cross3(ab, ac, n); sub3(d, a, ad);
         double sd = dot3(ad, n);   /* side of the opposite vertex */
         double so = -dot3(a, n);   /* side of the origin */
-        if (sd == 0.0) { outside_any = 1; } /* degenerate (flat) tetrahedron: treat every face as candidate */
+        /* degenerate (flat) tetrahedron: treat every face as candidate.  Flat to rounding counts as well: there the sign
+         * of sd is noise, and the origin far off the plane could pass every face test and be taken as enclosed (a
+         * converged search whose last support point closes a parallelogram with the simplex reported distance 0). */
+        if (fabs(sd) <= 1e-10 * sqrt(dot3(ab, ab) * dot3(ac, ac) * dot3(ad, ad))) sd = 0.0;
+        if (sd == 0.0) { outside_any = 1; }
         if (sd == 0.0 || so * sd < 0.0) {
             outside_any = 1;
             double p[3];
@@ -583,6 +587,26 @@ void smo_distances_h(const SmScene* sc, const double* q, const double* ob, const
             }
     }
     *d_moving = dm;
+}
+
+/* distance of every pair of the distance classes at robot pose q, margins subtracted, GJK without early stop (test
+ * hook: the tests find the pair that holds a class minimum and how far the other pairs are).  Pairs in the order of the
+ * device's pair table (smenv_create): static pairs, self pairs, then per obstacle, per mov_reward shape, per part.
+ * Obstacle poses as in smo_distances_h (hq: the human's joint angles, else NULL); the class rules of smo_distances_h
+ * (cap and query filters, inactive ball, latched contact) are not applied. */
+void smo_plan_pair_distances(const SmScene* sc, const double* q, const double* ob, const double* hq, double* out) {
+    Xf robot[1 + SM_MAX_JOINTS], obst[SM_MAX_OBST_FRAMES];
+    smo_fk(sc, q, robot);
+    obstacle_poses_h(sc, ob, hq, obst);
+    int k = 0;
+    for (int i = 0; i < sc->n_static_pairs; ++i)
+        out[k++] = pair_distance(sc, sc->static_pairs[i][0], sc->static_pairs[i][1], robot, obst, 0.0);
+    for (int i = 0; i < sc->n_self_pairs; ++i)
+        out[k++] = pair_distance(sc, sc->self_pairs[i][0], sc->self_pairs[i][1], robot, obst, 0.0);
+    for (int o = 0; o < sc->n_obstacles; ++o)
+        for (int r = 0; r < sc->n_mov_reward; ++r)
+            for (int s = 0; s < sc->obst_shape_cnt[o]; ++s)
+                out[k++] = pair_distance(sc, sc->mov_reward[r], sc->obst_shape_off[o] + s, robot, obst, 0.0);
 }
 
 /* contact in the simulation client: any manifold point between obstacle o and the robot, i.e. some convex pair

@@ -71,6 +71,22 @@ class SmHumanBounds(C.Structure):
     del f
 
 
+SM_PLAN_HWIDTH_CELLS = 384
+SM_PLAN_MAX_PAIRS = 512
+
+
+class SmPlanBounds(C.Structure):
+    """Constants of the distance planning (include/smenv.h, smenv_debug_plan_bounds)."""
+    f = C.c_float
+    _fields_ = [
+        ("n_shapes", i32), ("n_pairs_fixed", i32), ("n_pairs", i32), ("self_query", C.c_double),
+        ("center", (f * 3) * SM_MAX_SHAPES), ("radius", f * SM_MAX_SHAPES),
+        ("bmin", (f * 3) * SM_MAX_SHAPES), ("bmax", (f * 3) * SM_MAX_SHAPES), ("centroid", (f * 3) * SM_MAX_SHAPES),
+        ("pair_tab", C.c_uint32 * SM_PLAN_MAX_PAIRS), ("pair_rm", (f * 2) * SM_PLAN_MAX_PAIRS),
+        ("hwidth", (f * SM_PLAN_HWIDTH_CELLS) * SM_MAX_SHAPES)]
+    del f
+
+
 class SmHuman(C.Structure):
     _fields_ = [
         ("enabled", i32), ("n_joints", i32),
@@ -190,7 +206,7 @@ EXPORTED_SYMBOLS = [
     "smenv_last_error", "smenv_abi_version", "smenv_sizeof_scene", "smenv_sizeof_shape", "smenv_create",
     "smenv_destroy", "smenv_pool_sizes", "smenv_fill_pools", "smenv_pool_ptrs", "smenv_copy_pools", "smenv_set_state", "smenv_reset",
     "smenv_step", "smenv_step_random", "smenv_step_host", "smenv_set_step_ranges", "smenv_safe_range", "smenv_distances", "smenv_observation",
-    "smenv_counters", "smenv_enable_counters", "smenv_launch_count", "smenv_debug_gjk", "smenv_debug_build_lut", "smenv_debug_lut_cell", "smenv_debug_human_bounds", "smenv_kernel_timing",
+    "smenv_counters", "smenv_enable_counters", "smenv_launch_count", "smenv_debug_gjk", "smenv_debug_build_lut", "smenv_debug_lut_cell", "smenv_debug_human_bounds", "smenv_debug_plan_bounds", "smenv_kernel_timing",
     "smenv_kernel_times", "smenv_set_targets", "smenv_mlp_load", "smenv_mlp_forward", "smenv_risk_gate", "smenv_random_actions",
     "smenv_set_seed", "smenv_set_risk_gate", "smenv_set_human_actions_external", "smenv_set_human_state",
     "smenv_human_pool_sizes", "smenv_copy_human_pools", "smenv_measure_fma_peaks", "smenv_launch_config", "smenv_set_gate_exact", "smenv_mlp_forward_exact",

@@ -56,6 +56,7 @@ def load():
     lib.smenv_debug_build_lut.argtypes = [vp, i32, i32, vp, i32]
     lib.smenv_debug_lut_cell.argtypes = [C.c_float, C.c_float, C.c_float, i32]
     lib.smenv_debug_human_bounds.argtypes = [C.POINTER(abi.SmScene), C.POINTER(abi.SmHumanBounds)]
+    lib.smenv_debug_plan_bounds.argtypes = [C.POINTER(abi.SmScene), C.POINTER(abi.SmPlanBounds)]
     lib.smenv_set_risk_gate.argtypes = [vp, C.c_float]
     lib.smenv_random_actions.argtypes = [vp, C.POINTER(abi.SmBuffers), vp]
     lib.smenv_kernel_timing.argtypes = [vp, i32]

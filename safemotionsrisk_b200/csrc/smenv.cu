@@ -439,6 +439,62 @@ static int human_brake_bounds(const SmScene* sc, DevHuman& u, std::vector<short>
     return SM_OK;
 }
 
+// Constants of the distance planning (distance_plan_kernel), from the float32 vertices the kernels use: per shape the
+// bounding sphere, the box of the core vertices, the centroid and the support-width table (appended to hwidth); the pair
+// table with the margins and radii its bounds subtract; the self-collision query.  Fills d.shapes (all but .lut),
+// d.pair_tab, d.pair_rm, d.n_pairs_fixed, d.n_pairs and d.self_query.  Host only, shared by smenv_create and
+// smenv_debug_plan_bounds.
+static int plan_bounds(const SmScene* sc, const std::vector<float4>& verts, DevScene& d, std::vector<float>& hwidth) {
+    for (int s = 0; s < sc->n_shapes; ++s) {
+        const SmShape& h = sc->shapes[s];
+        DevShape& g = d.shapes[s];
+        g.frame = h.frame; g.off = h.vert_off; g.cnt = h.vert_cnt; g.link = h.link;
+        g.margin = (float)h.margin; g.cx = (float)h.center[0]; g.cy = (float)h.center[1]; g.cz = (float)h.center[2];
+        // bounding sphere recomputed on the float32 vertices so that it certainly contains them
+        float r = 0.f;
+        for (int k = 0; k < 3; ++k) { g.bmin[k] = FLT_MAX; g.bmax[k] = -FLT_MAX; }
+        for (int i = h.vert_off; i < h.vert_off + h.vert_cnt; ++i) {
+            float dx = verts[i].x - g.cx, dy = verts[i].y - g.cy, dz = verts[i].z - g.cz;
+            r = fmaxf(r, sqrtf(dx * dx + dy * dy + dz * dz));
+            g.bmin[0] = fminf(g.bmin[0], verts[i].x); g.bmax[0] = fmaxf(g.bmax[0], verts[i].x);
+            g.bmin[1] = fminf(g.bmin[1], verts[i].y); g.bmax[1] = fmaxf(g.bmax[1], verts[i].y);
+            g.bmin[2] = fminf(g.bmin[2], verts[i].z); g.bmax[2] = fmaxf(g.bmax[2], verts[i].z);
+        }
+        g.radius = r * (1.0f + 1e-6f) + 1e-7f;
+        double gs[3] = {0, 0, 0};
+        for (int i = h.vert_off; i < h.vert_off + h.vert_cnt; ++i) { gs[0] += verts[i].x; gs[1] += verts[i].y; gs[2] += verts[i].z; }
+        g.gx = (float)(gs[0] / h.vert_cnt); g.gy = (float)(gs[1] / h.vert_cnt); g.gz = (float)(gs[2] / h.vert_cnt);
+        g.hw = (int)hwidth.size();
+        {
+            const float cc[3] = {g.cx, g.cy, g.cz};
+            build_hwidth(verts.data() + h.vert_off, h.vert_cnt, cc, g.radius, hwidth);
+        }
+        g.lut = -1;
+    }
+    int np = 0;
+    auto push = [&](int a, int b, int cls) {
+        if (np < SM_MAX_PLAN_PAIRS) {
+            const DevShape& SA = d.shapes[a];
+            const DevShape& SB = d.shapes[b];
+            const bool box = SB.frame == 0;
+            d.pair_tab[np] = (uint32_t)a | ((uint32_t)b << 12) | ((uint32_t)cls << 24) | (box ? 0x80000000u : 0u);
+            const float m = SA.margin + SB.margin;
+            d.pair_rm[np] = make_float2(m * (1.0f - 1e-6f), (SA.radius + (box ? 0.f : SB.radius) + m) * (1.0f + 1e-6f));
+        }
+        ++np;
+    };
+    for (int i = 0; i < sc->n_static_pairs; ++i) push(sc->static_pairs[i][0], sc->static_pairs[i][1], 0);
+    for (int i = 0; i < sc->n_self_pairs; ++i) push(sc->self_pairs[i][0], sc->self_pairs[i][1], 1);
+    d.n_pairs_fixed = np;
+    for (int o = 0; o < sc->n_obstacles; ++o)
+        for (int r = 0; r < sc->n_mov_reward; ++r)
+            for (int k = 0; k < sc->obst_shape_cnt[o]; ++k) push(sc->mov_reward[r], sc->obst_shape_off[o] + k, 2);
+    d.n_pairs = np;
+    if (np > SM_MAX_PLAN_PAIRS) return fail(SM_ERR_SCENE, "too many convex pairs per env for the distance planning (max 512)");
+    d.self_query = std::min(sc->static_cap, std::max(sc->collision_dist, sc->w_self != 0.0 ? sc->d_self : 0.0));
+    return SM_OK;
+}
+
 extern "C" int smenv_destroy(SmEnv* env);
 // frees a half-built env on every early return of smenv_create
 struct CreateGuard {
@@ -501,32 +557,7 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
         verts[i] = make_float4((float)sc->verts[3 * i], (float)sc->verts[3 * i + 1], (float)sc->verts[3 * i + 2], 0.f);
     std::vector<uint32_t> lut;
     std::vector<float> hwidth;
-    for (int s = 0; s < sc->n_shapes; ++s) {
-        const SmShape& h = sc->shapes[s];
-        DevShape& g = d.shapes[s];
-        g.frame = h.frame; g.off = h.vert_off; g.cnt = h.vert_cnt; g.link = h.link;
-        g.margin = (float)h.margin; g.cx = (float)h.center[0]; g.cy = (float)h.center[1]; g.cz = (float)h.center[2];
-        // bounding sphere recomputed on the float32 vertices so that it certainly contains them
-        float r = 0.f;
-        for (int k = 0; k < 3; ++k) { g.bmin[k] = FLT_MAX; g.bmax[k] = -FLT_MAX; }
-        for (int i = h.vert_off; i < h.vert_off + h.vert_cnt; ++i) {
-            float dx = verts[i].x - g.cx, dy = verts[i].y - g.cy, dz = verts[i].z - g.cz;
-            r = fmaxf(r, sqrtf(dx * dx + dy * dy + dz * dz));
-            g.bmin[0] = fminf(g.bmin[0], verts[i].x); g.bmax[0] = fmaxf(g.bmax[0], verts[i].x);
-            g.bmin[1] = fminf(g.bmin[1], verts[i].y); g.bmax[1] = fmaxf(g.bmax[1], verts[i].y);
-            g.bmin[2] = fminf(g.bmin[2], verts[i].z); g.bmax[2] = fmaxf(g.bmax[2], verts[i].z);
-        }
-        g.radius = r * (1.0f + 1e-6f) + 1e-7f;
-        double gs[3] = {0, 0, 0};
-        for (int i = h.vert_off; i < h.vert_off + h.vert_cnt; ++i) { gs[0] += verts[i].x; gs[1] += verts[i].y; gs[2] += verts[i].z; }
-        g.gx = (float)(gs[0] / h.vert_cnt); g.gy = (float)(gs[1] / h.vert_cnt); g.gz = (float)(gs[2] / h.vert_cnt);
-        g.hw = (int)hwidth.size();
-        {
-            const float cc[3] = {g.cx, g.cy, g.cz};
-            build_hwidth(verts.data() + h.vert_off, h.vert_cnt, cc, g.radius, hwidth);
-        }
-        g.lut = -1;
-    }
+    if (const int rc = plan_bounds(sc, verts, d, hwidth)) return rc;
     // Support-direction tables.  The longest candidate list among the lanes of a GJK warp sets the trip count of its
     // support loop, so every hull that can have a table gets one as long as the kernel's shared-memory image (vertices +
     // tables + shapes) fits.  Candidates in order of quality, the first that fits the budget wins:
@@ -632,28 +663,6 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
             d.tp_rho[j] = rho;
         }
     }
-    {   // pair list of the distance planning
-        int np = 0;
-        auto push = [&](int a, int b, int cls) {
-            if (np < SM_MAX_PLAN_PAIRS) {
-                const DevShape& SA = d.shapes[a];
-                const DevShape& SB = d.shapes[b];
-                const bool box = SB.frame == 0;
-                d.pair_tab[np] = (uint32_t)a | ((uint32_t)b << 12) | ((uint32_t)cls << 24) | (box ? 0x80000000u : 0u);
-                const float m = SA.margin + SB.margin;
-                d.pair_rm[np] = make_float2(m * (1.0f - 1e-6f), (SA.radius + (box ? 0.f : SB.radius) + m) * (1.0f + 1e-6f));
-            }
-            ++np;
-        };
-        for (int i = 0; i < sc->n_static_pairs; ++i) push(sc->static_pairs[i][0], sc->static_pairs[i][1], 0);
-        for (int i = 0; i < sc->n_self_pairs; ++i) push(sc->self_pairs[i][0], sc->self_pairs[i][1], 1);
-        d.n_pairs_fixed = np;
-        for (int o = 0; o < sc->n_obstacles; ++o)
-            for (int r = 0; r < sc->n_mov_reward; ++r)
-                for (int k = 0; k < sc->obst_shape_cnt[o]; ++k) push(sc->mov_reward[r], sc->obst_shape_off[o] + k, 2);
-        d.n_pairs = np;
-        if (np > SM_MAX_PLAN_PAIRS) { return fail(SM_ERR_SCENE, "too many convex pairs per env for the distance planning (max 512)"); }
-    }
     // coarse contact phase: a change of joint j by dq moves the sphere centre of a contact slot in frame f by at most
     // dq * (sum of the fixed joint offsets between frame j+1 and f, plus the centre's own offset)
     for (int slot = 0; slot < sc->n_mov_contact; ++slot) {
@@ -685,7 +694,6 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
     for (int i = 0; i < 9; ++i) d.target_R[i] = (float)sc->target_R[i];
     d.ball_active_xy = sc->ball_active_xy;
     d.static_cap = sc->static_cap; d.moving_query = sc->moving_query; d.collision_dist = sc->collision_dist;
-    d.self_query = std::min(sc->static_cap, std::max(sc->collision_dist, sc->w_self != 0.0 ? sc->d_self : 0.0));
     d.w_self = sc->w_self; d.w_static = sc->w_static; d.w_moving = sc->w_moving;
     d.d_self = sc->d_self; d.d_static = sc->d_static; d.d_moving = sc->d_moving;
     d.w_low_acc = sc->w_low_acc; d.thr_low_acc = sc->thr_low_acc; d.w_low_vel = sc->w_low_vel; d.thr_low_vel = sc->thr_low_vel;
@@ -2203,6 +2211,33 @@ extern "C" int smenv_debug_build_lut(const float* xyz, int n, int res, uint32_t*
     return (int)t.size();
 }
 extern "C" int smenv_debug_lut_cell(float dx, float dy, float dz, int res) { return lut_cell_res(dx, dy, dz, res); }
+
+static_assert(SM_PLAN_HWIDTH_CELLS == 6 * SM_LUT_RES * SM_LUT_RES, "SmPlanBounds.hwidth holds one table per shape");
+static_assert(SM_PLAN_MAX_PAIRS == SM_MAX_PLAN_PAIRS, "SmPlanBounds.pair_tab holds the whole pair table");
+extern "C" int smenv_debug_plan_bounds(const SmScene* sc, SmPlanBounds* out) {
+    if (!sc || !out) return fail(SM_ERR_ARG, "null argument");
+    if (sc->n_shapes > SM_MAX_SHAPES || sc->n_verts <= 0) return fail(SM_ERR_SCENE, "bad shape table");
+    std::vector<float4> verts(sc->n_verts);
+    for (int i = 0; i < sc->n_verts; ++i)
+        verts[i] = make_float4((float)sc->verts[3 * i], (float)sc->verts[3 * i + 1], (float)sc->verts[3 * i + 2], 0.f);
+    std::vector<DevScene> dv(1);
+    DevScene& d = dv[0];
+    memset(&d, 0, sizeof(d));
+    std::vector<float> hwidth;
+    if (const int rc = plan_bounds(sc, verts, d, hwidth)) return rc;
+    memset(out, 0, sizeof(*out));
+    out->n_shapes = sc->n_shapes; out->n_pairs_fixed = d.n_pairs_fixed; out->n_pairs = d.n_pairs;
+    out->self_query = d.self_query;
+    for (int s = 0; s < sc->n_shapes; ++s) {
+        const DevShape& g = d.shapes[s];
+        out->center[s][0] = g.cx; out->center[s][1] = g.cy; out->center[s][2] = g.cz; out->radius[s] = g.radius;
+        out->centroid[s][0] = g.gx; out->centroid[s][1] = g.gy; out->centroid[s][2] = g.gz;
+        for (int k = 0; k < 3; ++k) { out->bmin[s][k] = g.bmin[k]; out->bmax[s][k] = g.bmax[k]; }
+        memcpy(out->hwidth[s], hwidth.data() + g.hw, sizeof(out->hwidth[s]));
+    }
+    for (int p = 0; p < d.n_pairs; ++p) { out->pair_tab[p] = d.pair_tab[p]; out->pair_rm[p][0] = d.pair_rm[p].x; out->pair_rm[p][1] = d.pair_rm[p].y; }
+    return SM_OK;
+}
 
 extern "C" int smenv_debug_human_bounds(const SmScene* sc, SmHumanBounds* out) {
     if (!sc || !out) return fail(SM_ERR_ARG, "null argument");

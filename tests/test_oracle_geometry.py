@@ -1,8 +1,15 @@
 """Oracle FK and GJK against independent computations (closed forms, brute-force QP)."""
 import numpy as np
+import pytest
 from scipy.optimize import minimize
 
 from oracle import oracle
+from safemotionsrisk_b200.config import ball_backup_config, space_backup_config, space_task_config
+from safemotionsrisk_b200.scene import Scene
+
+SCENES = {"space": space_backup_config, "space_bm": lambda: space_backup_config(ball_machine_mode=True),
+          "ball": ball_backup_config, "ball_bm": lambda: ball_backup_config(ball_machine_mode=True),
+          "space_task_bm": lambda: space_task_config(ball_machine_mode=True)}
 
 IDENT = np.array([1, 0, 0, 0, 1, 0, 0, 0, 1, 0, 0, 0], dtype=np.float64)
 
@@ -140,3 +147,59 @@ def test_table_box_core_is_shrunk_by_the_margin(space_scene):
     table = [s for s in space_scene.shapes if s["frame"] == 0 and s["cnt"] == 8][-1]
     v = table["verts"]
     assert np.allclose(v.max(0), [0.6 - 0.001, 0.8 - 0.001, -0.001]) and np.allclose(v.min(0), [-0.599, -0.799, -0.199])
+
+
+@pytest.mark.parametrize("name", ["space", "space_bm", "ball", "ball_bm", "space_task_bm"])
+def test_pair_distances_rebuild_the_class_distances(name):
+    """oracle.pair_distances lists every pair of the three distance classes (oracle.pair_classes order, the order of the
+    device's pair table); with the class rules of oracle.distances applied to it (cap and query filters, inactive ball,
+    latched contact) its class minima are the oracle's distances, exactly."""
+    scene = Scene(SCENES[name]())
+    sc = scene.struct
+    cls = oracle.pair_classes(scene)
+    assert [int((cls[:, 0] == c).sum()) for c in range(3)] == [
+        sc.n_static_pairs, sc.n_self_pairs, sc.n_mov_reward * sum(sc.obst_shape_cnt[o] for o in range(sc.n_obstacles))]
+    cap, query = sc.static_cap, sc.moving_query
+    rng = np.random.default_rng(11)
+    hits = np.zeros(3, dtype=int)
+    for _ in range(300):
+        q = rng.uniform(scene.pos_lo, scene.pos_hi)
+        ob = np.zeros(16)
+        if name.startswith("ball"):
+            ob[2:5] = rng.uniform([-0.8, -0.8, 0.1], [0.6, 0.8, 1.3])
+            ob[8:11] = rng.uniform(-1, 1, 3)
+            ob[12] = rng.uniform(0, 0.05)
+            ob[5:8] = rng.uniform(-1, 1, 3)
+            ob[13] = rng.random() < 0.8
+        else:
+            ob[0] = rng.integers(0, sc.planet_steps)
+        ob[1] = rng.random() < 0.1
+        d = oracle.pair_distances(scene, q, ob)
+        assert d.shape == (len(cls),)
+        ref = oracle.distances(scene, q, ob)
+        ds = min([cap] + [x for x in d[cls[:, 0] == 0] if x <= cap])
+        dse = min([cap] + [x for x in d[cls[:, 0] == 1] if x <= cap])
+        inactive = name.startswith("ball") and ob[13] == 0    # an inactive ball is not in the list of obstacles
+        dm = min([query + 0.002] + [x for x in d[cls[:, 0] == 2] if x <= query and not inactive])
+        if ob[1] != 0 or dm <= 0.0:                           # latched contact, or touching
+            dm = 0.0
+        assert (ds, dse, dm) == ref
+        hits += [ds < cap, dse < cap, 0.0 < dm < query]
+    # every class reports pair distances below its cap (the 1 mm moving query of space_task_bm aside)
+    assert hits[0] > 5 and (hits[1] > 5 or sc.n_self_pairs == 0) and (hits[2] > 5 or query < 0.01), hits
+
+
+def test_gjk_does_not_take_a_flat_simplex_for_an_enclosure(space_bm_scene):
+    """At this space_bm pose the GJK search between the ball machine (shape 9, frame 7) and shape 6 (frame 5) converges
+    at 0.0796 m, and its last support point closes a parallelogram with the simplex.  The tetrahedron is flat to
+    rounding, the side tests of its faces see noise, and the oracle used to report the pair as touching (distance 0).
+    The same hulls transformed to world coordinates first give the right distance."""
+    q = [1.9779949815397064, -1.6819379156182812, -2.2868158860081147, -0.9867392662235596, -1.956367020523305,
+         -0.3821141234131943, -2.2938491379058235]
+    fr = oracle.fk(space_bm_scene, q)
+    a, b = space_bm_scene.shapes[9], space_bm_scene.shapes[6]
+    assert (a["frame"], b["frame"]) == (7, 5)
+    d = oracle.gjk(a["verts"], fr[7], b["verts"], fr[5])
+    world = lambda s, f: s["verts"] @ fr[f][:9].reshape(3, 3).T + fr[f][9:]
+    ref = oracle.gjk(world(a, 7), IDENT, world(b, 5), IDENT)
+    assert abs(ref - 0.0796) < 1e-4 and abs(d - ref) < 1e-12, (d, ref)

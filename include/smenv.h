@@ -454,6 +454,19 @@ int smenv_risk_gate(SmEnv* env, const SmBuffers* buf, float threshold, float* ri
  * computed from it, safe_motions_base.py:1066); info slots SM_INFO_RISKY_ACTION / RISK / FIRST_RISKY_STEP report the
  * gate.  Needs both networks (smenv_mlp_load).  threshold < 0 switches the gate off (default). */
 int smenv_set_risk_gate(SmEnv* env, float threshold);
+/* How the gate inside the step decides (risk_state_config 4, RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_TRAJECTORY,
+ * safe_motions_base.py:1520-1592).  backup_steps = 0: by the risk network (default).  backup_steps = K > 0: by look-ahead:
+ * per env range, before the real step, the range's state is copied into shadow buffers owned by the library, the shadow
+ * episode clock is set to 0, and K + 1 steps without auto reset run on the copy: the proposed buf->actions, then K times
+ * the backup policy's action (tensor cores, tanh mean head) for the shadow observation.  Sub-step i uses step counter
+ * s + i (s = the real step's; the Human scene draws its policy noise from it, so that sub-step 0 equals the real step when
+ * the action is kept).  An env is risky exactly when some sub-step ends its episode for a reason other than
+ * SM_TERM_TRAJECTORY_LENGTH; the risk network is not consulted, so the threshold does not change the decision.  Risky envs
+ * execute the backup policy's action for the real observation as with the network gate (float32 with smenv_set_gate_exact);
+ * SM_INFO_RISK reports 0 or 1.  Applies only while the gate is on (smenv_set_risk_gate).  In the measurement mode the
+ * sub-steps run untimed before the timed real step; smenv_counters includes their work.  The shadow buffers are allocated
+ * by the first call with K > 0 and freed by smenv_destroy.  SM_ERR_STATE if the backup policy is not loaded. */
+int smenv_set_risk_lookahead(SmEnv* env, int backup_steps);
 /* Exact gate (default on): the tensor-core risk (fp16 operands) of the rows within `band` of the threshold is re-computed
  * in float32 on the CUDA cores before the decision, and the backup policy's action of the risky rows is computed in
  * float32 too, so that decisions and executed actions are those of a float32 evaluation of the shipped networks

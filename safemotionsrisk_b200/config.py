@@ -105,7 +105,10 @@ _UNSUPPORTED_UNLESS = dict(
     risk_state_deterministic_backup_trajectory=False, risk_store_ground_truth=False,
     risk_ignore_estimation_probability=0.0, risk_config=None,
 )
-_ALSO_ACCEPTED = dict(action_preprocessing_function=("tanh",))   # equivalent to the default (SURVEY Appendix A, Q1)
+# values besides the default that are implemented: "tanh" is equivalent to the default (SURVEY Appendix A, Q1);
+# risk_state_config 4 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_TRAJECTORY) is the backup-trajectory look-ahead
+# inside the step (smenv_set_risk_lookahead)
+_ALSO_ACCEPTED = dict(action_preprocessing_function=("tanh",), risk_state_config=(4,))
 
 
 class EnvConfig(dict):
@@ -126,6 +129,9 @@ class EnvConfig(dict):
                                               key, self[key], default))
         if (self["risk_config_dir"] is None) != (self["risk_threshold"] is None) and self["risk_config_dir"] is not None:
             raise ValueError("risk_config_dir needs risk_threshold (safe_motions_base.py:527-579, README.md:223-235)")
+        if self["risk_state_config"] == 4 and self["risk_config_dir"] is None:
+            raise ValueError("risk_state_config=4 (the backup-trajectory look-ahead) needs risk_config_dir, which supplies "
+                             "the backup policy, and risk_threshold")
         if self["robot_scene"] != 0:
             raise NotImplementedError("only robot_scene=0 (one iiwa7) is implemented; the reference itself defines "
                                       "only robot_scene 0 and 9 (robot_scene_base.py:169-183)")

@@ -211,6 +211,9 @@ struct SmEnv {
     int* d_gate_list = nullptr;    // [0..15] counters (two per env range), then [n] near-threshold rows, [n] risky rows
     int gate_exact = 1;            // re-rate near-threshold rows and compute the backup actions in float32 (smenv_set_gate_exact)
     float gate_band = 0.01f;       // |risk - threshold| below which the tensor-core risk is re-rated
+    int lookahead_steps = 0;       // > 0: the gate decides by a look-ahead of that many backup steps (smenv_set_risk_lookahead)
+    SmBuffers la_buf = {};         // [n] shadow copy of every record the step writes, and a stats vector nobody reads
+    std::vector<void*> la_allocs;
     // Human scene (smenv_human.cuh)
     bool human = false;
     int human_external = 0;        // the human's actions come from buf->hactions (parity protocol)
@@ -1076,6 +1079,7 @@ extern "C" int smenv_destroy(SmEnv* env) {
     if (env->h_step) cudaFreeHost(env->h_step);
     cudaFree(env->d_step);
     for (void* q : env->net_allocs) cudaFree(q);
+    for (void* q : env->la_allocs) cudaFree(q);
     cudaFree(env->d_risk); cudaFree(env->d_backup); cudaFree(env->d_exec); cudaFree(env->d_risky); cudaFree(env->d_gate_list);
     cudaFree(env->d_hpairs); cudaFree(env->d_hthresh); cudaFree(env->d_hrange); cudaFree(env->d_hbacc); cudaFree(env->d_hposes);
     cudaFree(env->d_hbinfo); cudaFree(env->d_hunits); cudaFree(env->d_hscratch); cudaFree(env->d_hpolicy); cudaFree(env->d_hstart_pool); cudaFree(env->d_hpool_brake); cudaFree(env->d_hpool_bcount); cudaFree(env->d_htarget_pool);
@@ -1442,17 +1446,26 @@ static int mlp_exact_launch(SmEnv* env, int which, MlpSeg s0, MlpSeg s1, MlpSeg 
 // (risk observation, proposed action) on the tensor cores; in exact mode the rows within gate_band of the threshold are
 // re-rated in float32 and the backup policy's action of the risky rows is computed in float32 on that subset; else the
 // backup policy runs on the tensor cores for every row.  Executed actions go to `exec` (== bv.actions: in place).
-static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, float threshold, float* risk, uint8_t* risky,
-                       float* backup, float* exec, cudaStream_t stream) {
+// the risk observation is the observation without the target-point entries (observations.py:419-431): joint position /
+// velocity / acceleration, then the obstacle entries
+static void risk_observation(const SmEnv* env, const float* obs, MlpSeg& kinem, MlpSeg& rest) {
     const DevScene& hs = env->host_scene;
     const int nj = hs.n_joints, ow = hs.obs_size;
-    // the risk observation is the observation without the target-point entries (observations.py:419-431): joint
-    // position / velocity / acceleration, then the obstacle entries
     const int n_tp = hs.use_target_points ? 3 * hs.obs_add_tp_pos + 3 * hs.obs_add_tp_rel : 0;
-    const MlpSeg kinem{bv.obs, ow, 3 * nj}, rest{bv.obs + 3 * nj + n_tp, ow, ow - 3 * nj - n_tp};
-    const MlpSeg act{bv.actions, nj, nj}, none{nullptr, 0, 0};
+    kinem = MlpSeg{obs, ow, 3 * nj};
+    rest = MlpSeg{obs + 3 * nj + n_tp, ow, ow - 3 * nj - n_tp};
+}
+
+// The gate's decision on a given risk over the envs of `bv`: risk >= threshold executes the backup policy's action for
+// bv.obs, on the tensor cores for every row, or in exact mode in float32 for the risky rows only (the caller has cleared
+// the counts of slot `chunk`).  Executed actions go to `exec` (== bv.actions: in place).
+static int gate_decide(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, float threshold, const float* risk,
+                       uint8_t* risky, float* backup, float* exec, cudaStream_t stream) {
+    const int nj = env->host_scene.n_joints;
+    MlpSeg kinem, rest;
+    risk_observation(env, bv.obs, kinem, rest);
+    const MlpSeg none{nullptr, 0, 0};
     int rc;
-    if ((rc = mlp_launch(env, SM_NET_RISK, kinem, rest, act, risk, 1, m, stream))) return rc;
     if (!env->gate_exact) {
         if ((rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, none, backup, MLP_MAX_OUT, m, stream))) return rc;
         risk_gate_kernel<<<(m + 255) / 256, 256, 0, stream>>>(bv.actions, exec, risk, backup, MLP_MAX_OUT, nj, m, threshold, risky);
@@ -1461,17 +1474,31 @@ static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk
         return SM_OK;
     }
     int* counts = env->d_gate_list + 2 * chunk;
-    int* near_list = env->d_gate_list + 32 + e0;
     int* risky_list = env->d_gate_list + 32 + env->n + e0;
-    CU(cudaMemsetAsync(counts, 0, 2 * sizeof(int), stream));
-    gate_band_kernel<<<(m + 255) / 256, 256, 0, stream>>>(risk, m, threshold, env->gate_band, near_list, counts);
-    env->launches++;
-    if ((rc = mlp_exact_launch(env, SM_NET_RISK, kinem, rest, act, near_list, counts, m, risk, 1, 1, stream))) return rc;
     risk_decide_kernel<<<(m + 255) / 256, 256, 0, stream>>>(bv.actions, exec, risk, nj, m, threshold, risky, risky_list, counts + 1);
     env->launches++;
     if ((rc = mlp_exact_launch(env, SM_NET_BACKUP, kinem, rest, none, risky_list, counts + 1, m, exec, nj, nj, stream))) return rc;
     CU(cudaGetLastError());
     return SM_OK;
+}
+
+static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, float threshold, float* risk, uint8_t* risky,
+                       float* backup, float* exec, cudaStream_t stream) {
+    const int nj = env->host_scene.n_joints;
+    MlpSeg kinem, rest;
+    risk_observation(env, bv.obs, kinem, rest);
+    const MlpSeg act{bv.actions, nj, nj};
+    int rc;
+    if ((rc = mlp_launch(env, SM_NET_RISK, kinem, rest, act, risk, 1, m, stream))) return rc;
+    if (env->gate_exact) {
+        int* counts = env->d_gate_list + 2 * chunk;
+        int* near_list = env->d_gate_list + 32 + e0;
+        CU(cudaMemsetAsync(counts, 0, 2 * sizeof(int), stream));
+        gate_band_kernel<<<(m + 255) / 256, 256, 0, stream>>>(risk, m, threshold, env->gate_band, near_list, counts);
+        env->launches++;
+        if ((rc = mlp_exact_launch(env, SM_NET_RISK, kinem, rest, act, near_list, counts, m, risk, 1, 1, stream))) return rc;
+    }
+    return gate_decide(env, bv, e0, m, chunk, threshold, risk, risky, backup, exec, stream);
 }
 
 static void launch_gjk(SmEnv* env, const GjkArgs& G, cudaStream_t stream) {
@@ -1493,13 +1520,15 @@ static void launch_gjk(SmEnv* env, const GjkArgs& G, cudaStream_t stream) {
     }
 }
 
-// The kernels of one env step over the envs [e0, e0 + m) on `stream`, with the work lists of slot `chunk`: every list
-// of the whole env ([0] = count, [1..k n] = entries) holds the sub-lists of the ranges back to back, the range's
-// sub-list starting at entry k * e0 + chunk (its own count first).  Ranges in flight at once need distinct slots.
-static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chunk, int auto_reset, int random_actions,
-                      uint32_t step_counter, bool tk, cudaStream_t stream, const uint32_t* step_ptr = nullptr) {
-    const SmBuffers buf_v = buffers_at(*full, e0, env->host_scene.n_joints, env->host_scene.obs_size);
-    const SmBuffers* buf = &buf_v;
+// The kernels of one env step over the m envs of the view `bv` (envs [e0, e0 + m) of the whole env) on `stream`, with the
+// work lists of slot `chunk`: every list of the whole env ([0] = count, [1..k n] = entries) holds the sub-lists of the
+// ranges back to back, the range's sub-list starting at entry k * e0 + chunk (its own count first).  Ranges in flight at
+// once need distinct slots.  exec: the actions to execute (NULL: bv.actions); risk / risky: the gate's outcome for the info
+// record (NULL: gate off).  The Philox step counter is step_counter + sub (step_ptr: read from device memory, plus sub).
+static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, int auto_reset, int random_actions,
+                      const float* exec, const float* risk, const uint8_t* risky, uint32_t step_counter, uint32_t sub,
+                      bool tk, cudaStream_t stream, const uint32_t* step_ptr) {
+    const SmBuffers* buf = &bv;
     const int per_env_items = env->item_capacity / env->n;
     int* worklist = env->d_worklist + 2 * chunk;
     float* scratch = env->d_scratch + (size_t)e0 * SM_SCRATCH_FLOATS;
@@ -1512,7 +1541,7 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     JointArgs JA;
     JA.buf = *buf; JA.n = m; JA.random_actions = random_actions;
     JA.k0 = (uint32_t)env->seed; JA.k1 = (uint32_t)(env->seed >> 32);
-    JA.step_counter = step_counter;
+    JA.step_counter = step_counter + sub;
     JA.env_base = e0;
     JA.scratch = scratch;
     JA.worklist = worklist;  // clears the item counter and the overflow count
@@ -1521,29 +1550,12 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     JA.tasks = tasks;
     JA.hpar = env->d_hpar + (size_t)e0 * 8 * SM_HPAR;
     JA.counters = env->count ? env->d_counters : nullptr;
-    JA.exec = nullptr;
+    JA.exec = exec;
     JA.set = 0; JA.nj = env->host_scene.n_joints; JA.defer = 0; JA.range_out = nullptr;
     JA.track_vel = env->host_scene.track_vel; JA.store_qset = env->host_scene.use_target_points;
     JA.keep_overflow = env->human ? 1 : 0;
     JA.clear_extra = nullptr;
     if (env->human) JA.worklist = nullptr;   // the nested env's kernels clear the counters (its braking check emits items first)
-    const bool gate = env->gate_threshold >= 0.0f;
-    if (gate) {   // actions.py:303-340: rate the proposed action, execute the backup policy's where it is risky
-        if (!buf->obs) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the observation buffer");
-        if (random_actions) {
-            if (!buf->actions) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the action buffer");
-            random_actions_kernel<<<(m * env->host_scene.n_joints + 255) / 256, 256, 0, stream>>>(
-                const_cast<float*>(buf->actions), env->host_scene.n_joints, m, e0, step_counter, (uint32_t)env->seed,
-                (uint32_t)(env->seed >> 32));
-            env->launches++;
-            JA.random_actions = 0;
-        }
-        float* exec = env->d_exec + (size_t)e0 * env->host_scene.n_joints;
-        int rc = gate_launch(env, buf_v, e0, m, chunk, env->gate_threshold, env->d_risk + e0, env->d_risky + e0,
-                             env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
-        if (rc) return rc;
-        JA.exec = exec;
-    }
     static const bool dbg_sync = getenv("SMENV_DEBUG_SYNC") != nullptr;  // locate a faulting kernel: sync after each
 #define SM_MARK(i)                                                                                           \
     do {                                                                                                     \
@@ -1583,7 +1595,8 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
         if (!buf->hkin || !buf->hstate || !buf->hbrake || !buf->hobs || !buf->hactions)
             return fail(SM_ERR_ARG, "smenv_step: the Human scene needs the hkin / hstate / hbrake / hobs / hactions buffers");
         HA.buf = *buf; HA.n = m; HA.env_base = e0;
-        HA.k0 = (uint32_t)env->seed; HA.k1 = (uint32_t)(env->seed >> 32); HA.step_counter = step_counter;
+        HA.k0 = (uint32_t)env->seed; HA.k1 = (uint32_t)(env->seed >> 32); HA.step_counter = step_counter + sub;
+        HA.step_offset = sub;
         HA.step_ptr = step_ptr;   // host-buffer step: the counter lives in device memory (graph replays)
         HA.policy_out = env->d_hpolicy + (size_t)e0 * 16;
         HA.range = env->d_hrange + (size_t)e0 * 32;
@@ -1686,8 +1699,8 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     A.target_pool = env->pools_filled ? env->d_target_pool : nullptr;
     A.target_pool_n = env->pools_filled ? env->target_pool_n : 0;
     A.counters = env->d_counters;
-    A.risk = gate ? env->d_risk + e0 : nullptr;
-    A.risky = gate ? env->d_risky + e0 : nullptr;
+    A.risk = risk;
+    A.risky = risky;
     const int T = SM_WARPS_PER_BLOCK * 32;
     const int blocks = (m + SM_WARPS_PER_BLOCK - 1) / SM_WARPS_PER_BLOCK;
     const int grid_p = blocks < env->grid_broad ? blocks : env->grid_broad;
@@ -1739,6 +1752,83 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     env->launches += contacts ? 5 : 3;
     CU(cudaGetLastError());
     return SM_OK;
+}
+
+// The gate's look-ahead (smenv_set_risk_lookahead) over the envs of `bv` (m envs from env e0): the range's records are
+// copied into the shadow buffers, whose episode clock restarts at 0 (switch_to_backup_client, safe_motions_base.py:
+// 1818-1822); K + 1 steps without auto reset run on the copy, the proposed action first, then the backup policy's; the risk
+// latches to 1 where one of them ends the episode for a reason other than the trajectory length; the gate decides on it.
+static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
+                            cudaStream_t stream, const uint32_t* step_ptr) {
+    const int nj = env->host_scene.n_joints, ow = env->host_scene.obs_size;
+    SmBuffers sv = buffers_at(env->la_buf, e0, nj, ow);
+    float* shadow_actions = const_cast<float*>(sv.actions);
+    const size_t n = (size_t)m;
+    const struct { void* dst; const void* src; size_t bytes; } recs[] = {
+        {sv.kin, bv.kin, n * SM_KIN_STRIDE * sizeof(double)}, {sv.obst, bv.obst, n * SM_OBST_STRIDE * sizeof(double)},
+        {sv.episode, bv.episode, n * 4 * sizeof(int32_t)}, {sv.ep_return, bv.ep_return, n * sizeof(double)},
+        {sv.target, bv.target, n * SM_TP_STRIDE * sizeof(double)}, {sv.obs, bv.obs, n * ow * sizeof(float)},
+        {sv.reward, bv.reward, n * sizeof(float)}, {sv.done, bv.done, n}, {sv.term_reason, bv.term_reason, n * sizeof(int32_t)},
+        {sv.info, bv.info, n * SM_INFO_STRIDE * sizeof(float)}, {sv.epacc, bv.epacc, n * SM_EP_STRIDE * sizeof(float)},
+        {sv.epinfo, bv.epinfo, n * SM_EP_STRIDE * sizeof(float)}, {shadow_actions, bv.actions, n * nj * sizeof(float)},
+        {sv.hkin, bv.hkin, n * SM_KIN_STRIDE * sizeof(double)}, {sv.hstate, bv.hstate, n * SM_HSTATE_STRIDE * sizeof(double)},
+        {sv.hbrake, bv.hbrake, n * SM_HBRAKE_STEPS * SM_HUMAN_JOINTS * sizeof(double)},
+        {sv.hobs, bv.hobs, n * SM_HOBS_STRIDE * sizeof(float)}, {sv.hactions, bv.hactions, n * SM_HUMAN_JOINTS * sizeof(float)}};
+    for (const auto& r : recs)
+        if (r.dst && r.src) CU(cudaMemcpyAsync(r.dst, r.src, r.bytes, cudaMemcpyDeviceToDevice, stream));
+    // records the caller does not keep stay absent in the copy
+    if (!bv.target) sv.target = nullptr;
+    if (!bv.epacc) { sv.epacc = nullptr; sv.epinfo = nullptr; }
+    CU(cudaMemset2DAsync(sv.episode, 4 * sizeof(int32_t), 0, sizeof(int32_t), n, stream));   // episode_length = 0
+    float* risk = env->d_risk + e0;
+    CU(cudaMemsetAsync(risk, 0, n * sizeof(float), stream));
+    MlpSeg kinem, rest;
+    risk_observation(env, sv.obs, kinem, rest);
+    int rc;
+    for (int i = 0; i <= env->lookahead_steps; ++i) {
+        if (i > 0 && (rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0}, shadow_actions, nj, m, stream)))
+            return rc;
+        if ((rc = step_chain(env, sv, e0, m, chunk, 0, 0, nullptr, nullptr, nullptr, step_counter, (uint32_t)i, false, stream,
+                             step_ptr)))
+            return rc;
+        lookahead_latch_kernel<<<(m + 255) / 256, 256, 0, stream>>>(risk, sv.done, sv.term_reason, m);
+        env->launches++;
+    }
+    CU(cudaGetLastError());
+    if (env->gate_exact) CU(cudaMemsetAsync(env->d_gate_list + 2 * chunk, 0, 2 * sizeof(int), stream));
+    // risk is 0 or 1: 0.5 separates them whatever the gate's threshold
+    return gate_decide(env, bv, e0, m, chunk, 0.5f, risk, env->d_risky + e0, env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec,
+                       stream);
+}
+
+// One env step over the envs [e0, e0 + m) on `stream` with the work lists of slot `chunk` (step_chain): with the gate on
+// (actions.py:303-340) the proposed actions are rated first -- by the risk network, or by the look-ahead -- and the backup
+// policy's action is executed where they are risky.
+static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chunk, int auto_reset, int random_actions,
+                      uint32_t step_counter, bool tk, cudaStream_t stream, const uint32_t* step_ptr = nullptr) {
+    const SmBuffers buf_v = buffers_at(*full, e0, env->host_scene.n_joints, env->host_scene.obs_size);
+    const SmBuffers* buf = &buf_v;
+    const bool gate = env->gate_threshold >= 0.0f;
+    float* exec = nullptr;
+    if (gate) {
+        if (!buf->obs) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the observation buffer");
+        if (random_actions) {
+            if (!buf->actions) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the action buffer");
+            random_actions_kernel<<<(m * env->host_scene.n_joints + 255) / 256, 256, 0, stream>>>(
+                const_cast<float*>(buf->actions), env->host_scene.n_joints, m, e0, step_counter, (uint32_t)env->seed,
+                (uint32_t)(env->seed >> 32));
+            env->launches++;
+            random_actions = 0;
+        }
+        exec = env->d_exec + (size_t)e0 * env->host_scene.n_joints;
+        const int rc = env->lookahead_steps > 0
+                           ? lookahead_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr)
+                           : gate_launch(env, buf_v, e0, m, chunk, env->gate_threshold, env->d_risk + e0, env->d_risky + e0,
+                                         env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
+        if (rc) return rc;
+    }
+    return step_chain(env, buf_v, e0, m, chunk, auto_reset, random_actions, exec, gate ? env->d_risk + e0 : nullptr,
+                      gate ? env->d_risky + e0 : nullptr, step_counter, 0, tk, stream, step_ptr);
 }
 
 // The count of the deferred-joint list is cleared by the finish kernel of the previous step; when the number of ranges
@@ -1834,7 +1924,7 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
 struct HostStepKey {
     SmBuffers buf;
     const void* h[4];
-    int auto_reset, chunks, count, pools, human_external, gate_exact;
+    int auto_reset, chunks, count, pools, human_external, gate_exact, lookahead;
     float gate, gate_band;
 };
 
@@ -1909,6 +1999,7 @@ extern "C" int smenv_step_host(SmEnv* env, const SmBuffers* buf, const float* h_
     key.h[0] = h_actions; key.h[1] = h_obs; key.h[2] = h_reward; key.h[3] = h_done;
     key.auto_reset = auto_reset; key.chunks = chunks; key.count = env->count ? 1 : 0; key.pools = env->pools_filled ? 1 : 0; key.gate = env->gate_threshold;
     key.human_external = env->human_external ? 1 : 0; key.gate_exact = env->gate_exact ? 1 : 0; key.gate_band = env->gate_band;
+    key.lookahead = env->lookahead_steps;
     if (!env->host_graph || memcmp(&key, env->host_graph_key, sizeof(key)) != 0) {
         if (env->host_graph) { cudaGraphExecDestroy(env->host_graph); env->host_graph = nullptr; }
         const unsigned long long launches0 = env->launches;
@@ -2122,6 +2213,49 @@ extern "C" int smenv_set_risk_gate(SmEnv* env, float threshold) {
     if (threshold >= 0.0f && (!env->net_loaded[0] || !env->net_loaded[1]))
         return fail(SM_ERR_STATE, "smenv_set_risk_gate: load the risk network and the backup policy first (smenv_mlp_load)");
     env->gate_threshold = threshold >= 0.0f ? threshold : -1.0f;
+    return SM_OK;
+}
+
+extern "C" int smenv_set_risk_lookahead(SmEnv* env, int backup_steps) {
+    if (!env) return fail(SM_ERR_ARG, "smenv_set_risk_lookahead: null env");
+    if (backup_steps < 0) return fail(SM_ERR_ARG, "smenv_set_risk_lookahead: backup_steps must be >= 0");
+    if (backup_steps > 0 && !env->net_loaded[SM_NET_BACKUP])
+        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: load the backup policy first (smenv_mlp_load)");
+    if (backup_steps > 0 && env->la_allocs.empty()) {
+        CU(cudaSetDevice(env->device));
+        const size_t n = (size_t)env->n;
+        const DevScene& hs = env->host_scene;
+        SmBuffers& b = env->la_buf;
+        float* actions = nullptr;
+        const struct { void** p; size_t bytes; bool used; } recs[] = {
+            {(void**)&b.kin, n * SM_KIN_STRIDE * sizeof(double), true}, {(void**)&b.obst, n * SM_OBST_STRIDE * sizeof(double), true},
+            {(void**)&b.episode, n * 4 * sizeof(int32_t), true}, {(void**)&b.ep_return, n * sizeof(double), true},
+            {(void**)&b.target, n * SM_TP_STRIDE * sizeof(double), hs.use_target_points != 0},
+            {(void**)&b.obs, n * hs.obs_size * sizeof(float), true}, {(void**)&b.reward, n * sizeof(float), true},
+            {(void**)&b.done, n, true}, {(void**)&b.term_reason, n * sizeof(int32_t), true},
+            {(void**)&b.info, n * SM_INFO_STRIDE * sizeof(float), true},
+            {(void**)&b.epacc, n * SM_EP_STRIDE * sizeof(float), true}, {(void**)&b.epinfo, n * SM_EP_STRIDE * sizeof(float), true},
+            {(void**)&actions, n * hs.n_joints * sizeof(float), true},
+            {(void**)&b.hkin, n * SM_KIN_STRIDE * sizeof(double), env->human},
+            {(void**)&b.hstate, n * SM_HSTATE_STRIDE * sizeof(double), env->human},
+            {(void**)&b.hbrake, n * SM_HBRAKE_STEPS * SM_HUMAN_JOINTS * sizeof(double), env->human},
+            {(void**)&b.hobs, n * SM_HOBS_STRIDE * sizeof(float), env->human},
+            {(void**)&b.hactions, n * SM_HUMAN_JOINTS * sizeof(float), env->human},
+            {(void**)&b.stats, 32 * sizeof(double), true}};   // the shadow steps' episode statistics: nobody reads them
+        for (const auto& r : recs) {
+            if (!r.used) continue;
+            const cudaError_t e = cudaMalloc(r.p, r.bytes);
+            if (e != cudaSuccess) {
+                for (void* q : env->la_allocs) cudaFree(q);
+                env->la_allocs.clear();
+                b = SmBuffers{};
+                return fail(SM_ERR_CUDA, std::string("smenv_set_risk_lookahead: cudaMalloc: ") + cudaGetErrorString(e));
+            }
+            env->la_allocs.push_back(*r.p);
+        }
+        b.actions = actions;
+    }
+    env->lookahead_steps = backup_steps;
     return SM_OK;
 }
 

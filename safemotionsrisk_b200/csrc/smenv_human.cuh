@@ -25,6 +25,7 @@ struct HumanArgs {
     SmBuffers buf;
     int n, env_base;
     uint32_t k0, k1, step_counter;
+    uint32_t step_offset;      // added to *step_ptr: sub-step i of the look-ahead (smenv_set_risk_lookahead) draws with s + i
     const uint32_t* step_ptr;  // if set, the step counter is read from device memory instead (graph replays of the host step)
     const float* policy_out;   // [n][16] outputs of the human's policy (tanh), NULL: buf.hactions come from the caller
     double* range;             // [n][8][4] lo, hi, mapped acceleration of every human joint (joint kernels, deferred)
@@ -60,7 +61,7 @@ __global__ void human_action_kernel(HumanArgs A) {
     const float* o = A.policy_out + (size_t)env * 16;
     const float mean = o[j];
     const float log_std = (float)c_sc.hu.log_std_lo + 0.5f * (o[8 + j] + 1.0f) * (float)(c_sc.hu.log_std_hi - c_sc.hu.log_std_lo);
-    const uint32_t step = A.step_ptr ? __ldg(A.step_ptr) : A.step_counter;
+    const uint32_t step = A.step_ptr ? __ldg(A.step_ptr) + A.step_offset : A.step_counter;
     const uint4 r = philox((uint32_t)(env + A.env_base), step, (uint32_t)j, 0x4057u, A.k0, A.k1);
     const float u1 = fmaxf(u01f(r.x), 5.9604645e-8f), u2 = u01f(r.y);
     const float eps = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);   // Box-Muller

@@ -479,6 +479,13 @@ __global__ void __launch_bounds__(256) mlp_exact_kernel(MlpExactArgs A) {
     }
 }
 
+// the look-ahead's risk (smenv_set_risk_lookahead): 1 once a sub-step of the env's shadow copy ended its episode for a
+// reason other than the trajectory length (risk_ground_truth's labelling rule, safe_motions_base.py:1520-1592)
+__global__ void lookahead_latch_kernel(float* risk, const uint8_t* done, const int32_t* term_reason, int n) {
+    const int env = blockIdx.x * blockDim.x + threadIdx.x;
+    if (env < n && done[env] && term_reason[env] != SM_TERM_TRAJECTORY_LENGTH) risk[env] = 1.0f;
+}
+
 // rows whose tensor-core risk lies within `band` of the threshold -> list (re-rated exactly before the gate decides)
 __global__ void gate_band_kernel(const float* risk, int n, float threshold, float band, int* list, int* count) {
     const int env = blockIdx.x * blockDim.x + threadIdx.x;

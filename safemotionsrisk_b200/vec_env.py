@@ -135,6 +135,8 @@ class SafeMotionsVecEnv:
         if self.config.risk_config_dir is not None:
             self.load_networks(self._resolve_risk_config_dir(self.config.risk_config_dir))
             self.set_risk_gate(self.config.risk_threshold)
+            if self.config.risk_state_config == 4:
+                self.set_risk_lookahead(self.config.risk_state_backup_trajectory_steps or 20)
             if self.config.risk_check_initial_backup_trajectory and not fill_pools:
                 raise ValueError("risk_check_initial_backup_trajectory needs the start pools (fill_pools=True)")
 
@@ -194,6 +196,15 @@ class SafeMotionsVecEnv:
         thr = -1.0 if threshold is None else float(threshold)
         cabi.check(self._lib.smenv_set_risk_gate(self._handle, thr), "smenv_set_risk_gate")
         self._gate_threshold = None if threshold is None else float(threshold)
+
+    def set_risk_lookahead(self, backup_steps):
+        """risk_state_config 4 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_TRAJECTORY, safe_motions_base.py:
+        1520-1592) inside the step: while the risk gate is on, an env's action is risky exactly when a copy of the env
+        that executes it and then follows the backup policy for `backup_steps` steps (no auto reset, the episode clock
+        from 0) ends its episode for a reason other than the trajectory length -- the labelling rule of
+        risk_ground_truth.  The risk network is not consulted, so the threshold does not change the decision.  0 or None
+        switches back to the network gate (smenv_set_risk_lookahead).  Needs the backup policy (load_networks)."""
+        cabi.check(self._lib.smenv_set_risk_lookahead(self._handle, int(backup_steps or 0)), "smenv_set_risk_lookahead")
 
     def close(self):
         if self._handle:

@@ -445,14 +445,18 @@ int smenv_mlp_load(SmEnv* env, int which, int n_tc, const int32_t* dims, int hid
 int smenv_mlp_forward(SmEnv* env, int which, const float* in0, int in0_w, const float* in1, int in1_w, float* out,
                       int out_stride, int n, SmStream stream);
 /* Risk gate on buf->actions in place: risk(obs, action) >= threshold replaces the env's action by the backup policy's
- * (obs = buf->obs, the observation the action was computed from).  risk_out [N] / risky_out [N] may be NULL. */
+ * (obs = buf->obs, the observation the action was computed from).  risk_out [N] / risky_out [N] may be NULL.
+ * SM_ERR_STATE if the loaded risk network is a state network (see smenv_set_risk_next_state). */
 int smenv_risk_gate(SmEnv* env, const SmBuffers* buf, float threshold, float* risk_out, uint8_t* risky_out,
                     SmStream stream);
 /* Risk gate inside the step (actions.py:303-340): with threshold >= 0 every smenv_step / smenv_step_random /
  * smenv_step_host first rates buf->actions with the risk network on buf->obs and executes the backup policy's action
  * in the envs rated >= threshold.  buf->actions keeps the proposed action (the action punishment of the reward is
  * computed from it, safe_motions_base.py:1066); info slots SM_INFO_RISKY_ACTION / RISK / FIRST_RISKY_STEP report the
- * gate.  Needs both networks (smenv_mlp_load).  threshold < 0 switches the gate off (default). */
+ * gate.  Needs both networks (smenv_mlp_load).  threshold < 0 switches the gate off (default).  The risk network's input
+ * width, recorded by smenv_mlp_load, tells its kind: the risk observation followed by the action (a state-action network,
+ * which the network gate needs) or the risk observation alone (a state network, which smenv_set_risk_next_state needs);
+ * switching the gate on with the other kind returns SM_ERR_STATE (the look-ahead does not consult the network). */
 int smenv_set_risk_gate(SmEnv* env, float threshold);
 /* How the gate inside the step decides (risk_state_config 4, RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_TRAJECTORY,
  * safe_motions_base.py:1520-1592).  backup_steps = 0: by the risk network (default).  backup_steps = K > 0: by look-ahead:
@@ -465,8 +469,22 @@ int smenv_set_risk_gate(SmEnv* env, float threshold);
  * execute the backup policy's action for the real observation as with the network gate (float32 with smenv_set_gate_exact);
  * SM_INFO_RISK reports 0 or 1.  Applies only while the gate is on (smenv_set_risk_gate).  In the measurement mode the
  * sub-steps run untimed before the timed real step; smenv_counters includes their work.  The shadow buffers are allocated
- * by the first call with K > 0 and freed by smenv_destroy.  SM_ERR_STATE if the backup policy is not loaded. */
+ * by the first call with K > 0 (or smenv_set_risk_next_state) and freed by smenv_destroy.  SM_ERR_STATE if the backup
+ * policy is not loaded or the next-state check is on. */
 int smenv_set_risk_lookahead(SmEnv* env, int backup_steps);
+/* The gate rates the simulated next state (risk_state_config 3, RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP) with a state
+ * risk network, whose input is the risk observation alone.  enable = 1: per env range, before the real step, the range's
+ * state is copied into the shadow buffers (those of the look-ahead) with its episode clock as it is, and one step without
+ * auto reset runs the proposed buf->actions on the copy with the real step's counter (in the Human scene the human's policy
+ * noise is that of the real step).  The risk is the state network's rating of the shadow's risk observation (tensor cores;
+ * with smenv_set_gate_exact the rows within the band of the threshold re-rated in float32), set to 1 where the simulated
+ * step ended its episode for a reason other than SM_TERM_TRAJECTORY_LENGTH (a kept action never ends its own step in a
+ * collision).  risk >= threshold executes the backup policy's action for the real observation as with the network gate;
+ * SM_INFO_RISK reports the risk.  Applies only while the gate is on (smenv_set_risk_gate).  In the measurement mode the
+ * simulated step runs untimed before the timed real step; smenv_counters includes its work.  SM_ERR_STATE if the backup
+ * policy is not loaded, the loaded risk network is not a state network or the look-ahead is on; enable = 0 with the gate
+ * on and a state network loaded returns SM_ERR_STATE as well (the network gate cannot use that network). */
+int smenv_set_risk_next_state(SmEnv* env, int enable);
 /* Exact gate (default on): the tensor-core risk (fp16 operands) of the rows within `band` of the threshold is re-computed
  * in float32 on the CUDA cores before the decision, and the backup policy's action of the risky rows is computed in
  * float32 too, so that decisions and executed actions are those of a float32 evaluation of the shipped networks

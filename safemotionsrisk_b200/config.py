@@ -106,9 +106,17 @@ _UNSUPPORTED_UNLESS = dict(
     risk_ignore_estimation_probability=0.0, risk_config=None,
 )
 # values besides the default that are implemented: "tanh" is equivalent to the default (SURVEY Appendix A, Q1);
-# risk_state_config 4 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_TRAJECTORY) is the backup-trajectory look-ahead
-# inside the step (smenv_set_risk_lookahead)
-_ALSO_ACCEPTED = dict(action_preprocessing_function=("tanh",), risk_state_config=(4,))
+# risk_state_config 3 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP) rates the simulated next state with a state risk network
+# inside the step (smenv_set_risk_next_state); risk_state_config 4 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP_AND_BACKUP_
+# TRAJECTORY) is the backup-trajectory look-ahead inside the step (smenv_set_risk_lookahead)
+_ALSO_ACCEPTED = dict(action_preprocessing_function=("tanh",), risk_state_config=(3, 4))
+
+
+def _names_state_action_network(path):
+    """True if a component of `path` is state_action (the shipped networks, risk_networks/state_action/<scene>) or
+    state_action_risk (the state-action outputs of risk_train)."""
+    parts = str(path).replace("\\", "/").split("/")
+    return any(p in ("state_action", "state_action_risk") for p in parts)
 
 
 class EnvConfig(dict):
@@ -132,6 +140,14 @@ class EnvConfig(dict):
         if self["risk_state_config"] == 4 and self["risk_config_dir"] is None:
             raise ValueError("risk_state_config=4 (the backup-trajectory look-ahead) needs risk_config_dir, which supplies "
                              "the backup policy, and risk_threshold")
+        if self["risk_state_config"] == 3:
+            if self["risk_config_dir"] is None or self["risk_threshold"] is None:
+                raise ValueError("risk_state_config=3 (rate the simulated next state) needs risk_config_dir, which supplies "
+                                 "the state risk network, and risk_threshold")
+            if _names_state_action_network(self["risk_config_dir"]):
+                raise NotImplementedError("risk_state_config=3 rates the simulated next state with a state risk network "
+                                          "(risk_train on state_risk data); rating it with the state-action network of "
+                                          "{!r} is not implemented".format(self["risk_config_dir"]))
         if self["robot_scene"] != 0:
             raise NotImplementedError("only robot_scene=0 (one iiwa7) is implemented; the reference itself defines "
                                       "only robot_scene 0 and 9 (robot_scene_base.py:169-183)")

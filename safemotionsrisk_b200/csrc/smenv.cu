@@ -212,6 +212,7 @@ struct SmEnv {
     int gate_exact = 1;            // re-rate near-threshold rows and compute the backup actions in float32 (smenv_set_gate_exact)
     float gate_band = 0.01f;       // |risk - threshold| below which the tensor-core risk is re-rated
     int lookahead_steps = 0;       // > 0: the gate decides by a look-ahead of that many backup steps (smenv_set_risk_lookahead)
+    int next_state = 0;            // the gate rates the simulated next state with a state risk network (smenv_set_risk_next_state)
     SmBuffers la_buf = {};         // [n] shadow copy of every record the step writes, and a stats vector nobody reads
     std::vector<void*> la_allocs;
     // Human scene (smenv_human.cuh)
@@ -1448,10 +1449,12 @@ static int mlp_exact_launch(SmEnv* env, int which, MlpSeg s0, MlpSeg s1, MlpSeg 
 // backup policy runs on the tensor cores for every row.  Executed actions go to `exec` (== bv.actions: in place).
 // the risk observation is the observation without the target-point entries (observations.py:419-431): joint position /
 // velocity / acceleration, then the obstacle entries
-static void risk_observation(const SmEnv* env, const float* obs, MlpSeg& kinem, MlpSeg& rest) {
+static int risk_obs_width(const SmEnv* env) {
     const DevScene& hs = env->host_scene;
-    const int nj = hs.n_joints, ow = hs.obs_size;
-    const int n_tp = hs.use_target_points ? 3 * hs.obs_add_tp_pos + 3 * hs.obs_add_tp_rel : 0;
+    return hs.obs_size - (hs.use_target_points ? 3 * hs.obs_add_tp_pos + 3 * hs.obs_add_tp_rel : 0);
+}
+static void risk_observation(const SmEnv* env, const float* obs, MlpSeg& kinem, MlpSeg& rest) {
+    const int nj = env->host_scene.n_joints, ow = env->host_scene.obs_size, n_tp = ow - risk_obs_width(env);
     kinem = MlpSeg{obs, ow, 3 * nj};
     rest = MlpSeg{obs + 3 * nj + n_tp, ow, ow - 3 * nj - n_tp};
 }
@@ -1482,12 +1485,10 @@ static int gate_decide(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk
     return SM_OK;
 }
 
-static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, float threshold, float* risk, uint8_t* risky,
-                       float* backup, float* exec, cudaStream_t stream) {
-    const int nj = env->host_scene.n_joints;
-    MlpSeg kinem, rest;
-    risk_observation(env, bv.obs, kinem, rest);
-    const MlpSeg act{bv.actions, nj, nj};
+// The risk network on the m rows (kinem, rest, act) -- act is empty for a state network -- on the tensor cores; in exact
+// mode the rows within gate_band of the threshold are re-rated in float32 (the counts of slot `chunk` are cleared here).
+static int risk_rate(SmEnv* env, MlpSeg kinem, MlpSeg rest, MlpSeg act, int e0, int m, int chunk, float threshold, float* risk,
+                     cudaStream_t stream) {
     int rc;
     if ((rc = mlp_launch(env, SM_NET_RISK, kinem, rest, act, risk, 1, m, stream))) return rc;
     if (env->gate_exact) {
@@ -1498,7 +1499,24 @@ static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk
         env->launches++;
         if ((rc = mlp_exact_launch(env, SM_NET_RISK, kinem, rest, act, near_list, counts, m, risk, 1, 1, stream))) return rc;
     }
+    return SM_OK;
+}
+
+static int gate_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, float threshold, float* risk, uint8_t* risky,
+                       float* backup, float* exec, cudaStream_t stream) {
+    const int nj = env->host_scene.n_joints;
+    MlpSeg kinem, rest;
+    risk_observation(env, bv.obs, kinem, rest);
+    const MlpSeg act{bv.actions, nj, nj};
+    int rc;
+    if ((rc = risk_rate(env, kinem, rest, act, e0, m, chunk, threshold, risk, stream))) return rc;
     return gate_decide(env, bv, e0, m, chunk, threshold, risk, risky, backup, exec, stream);
+}
+
+// Whether the loaded risk network takes the risk observation alone -- a state network, by the input width smenv_mlp_load
+// recorded -- rather than followed by the action (a state-action network).
+static bool risk_net_is_state(const SmEnv* env) {
+    return env->net_loaded[SM_NET_RISK] && env->nets[SM_NET_RISK].n_in == risk_obs_width(env);
 }
 
 static void launch_gjk(SmEnv* env, const GjkArgs& G, cudaStream_t stream) {
@@ -1754,15 +1772,12 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
     return SM_OK;
 }
 
-// The gate's look-ahead (smenv_set_risk_lookahead) over the envs of `bv` (m envs from env e0): the range's records are
-// copied into the shadow buffers, whose episode clock restarts at 0 (switch_to_backup_client, safe_motions_base.py:
-// 1818-1822); K + 1 steps without auto reset run on the copy, the proposed action first, then the backup policy's; the risk
-// latches to 1 where one of them ends the episode for a reason other than the trajectory length; the gate decides on it.
-static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
-                            cudaStream_t stream, const uint32_t* step_ptr) {
+// Copies the records of the envs of `bv` (m envs from env e0) into the shadow buffers (smenv_set_risk_lookahead /
+// smenv_set_risk_next_state) and sets `sv` to the shadow view of the range; records the caller does not keep stay absent
+// in the copy.
+static int shadow_copy(SmEnv* env, const SmBuffers& bv, int e0, int m, SmBuffers& sv, cudaStream_t stream) {
     const int nj = env->host_scene.n_joints, ow = env->host_scene.obs_size;
-    SmBuffers sv = buffers_at(env->la_buf, e0, nj, ow);
-    float* shadow_actions = const_cast<float*>(sv.actions);
+    sv = buffers_at(env->la_buf, e0, nj, ow);
     const size_t n = (size_t)m;
     const struct { void* dst; const void* src; size_t bytes; } recs[] = {
         {sv.kin, bv.kin, n * SM_KIN_STRIDE * sizeof(double)}, {sv.obst, bv.obst, n * SM_OBST_STRIDE * sizeof(double)},
@@ -1770,21 +1785,34 @@ static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int 
         {sv.target, bv.target, n * SM_TP_STRIDE * sizeof(double)}, {sv.obs, bv.obs, n * ow * sizeof(float)},
         {sv.reward, bv.reward, n * sizeof(float)}, {sv.done, bv.done, n}, {sv.term_reason, bv.term_reason, n * sizeof(int32_t)},
         {sv.info, bv.info, n * SM_INFO_STRIDE * sizeof(float)}, {sv.epacc, bv.epacc, n * SM_EP_STRIDE * sizeof(float)},
-        {sv.epinfo, bv.epinfo, n * SM_EP_STRIDE * sizeof(float)}, {shadow_actions, bv.actions, n * nj * sizeof(float)},
+        {sv.epinfo, bv.epinfo, n * SM_EP_STRIDE * sizeof(float)}, {const_cast<float*>(sv.actions), bv.actions, n * nj * sizeof(float)},
         {sv.hkin, bv.hkin, n * SM_KIN_STRIDE * sizeof(double)}, {sv.hstate, bv.hstate, n * SM_HSTATE_STRIDE * sizeof(double)},
         {sv.hbrake, bv.hbrake, n * SM_HBRAKE_STEPS * SM_HUMAN_JOINTS * sizeof(double)},
         {sv.hobs, bv.hobs, n * SM_HOBS_STRIDE * sizeof(float)}, {sv.hactions, bv.hactions, n * SM_HUMAN_JOINTS * sizeof(float)}};
     for (const auto& r : recs)
         if (r.dst && r.src) CU(cudaMemcpyAsync(r.dst, r.src, r.bytes, cudaMemcpyDeviceToDevice, stream));
-    // records the caller does not keep stay absent in the copy
     if (!bv.target) sv.target = nullptr;
     if (!bv.epacc) { sv.epacc = nullptr; sv.epinfo = nullptr; }
+    return SM_OK;
+}
+
+// The gate's look-ahead (smenv_set_risk_lookahead) over the envs of `bv` (m envs from env e0): the range's records are
+// copied into the shadow buffers, whose episode clock restarts at 0 (switch_to_backup_client, safe_motions_base.py:
+// 1818-1822); K + 1 steps without auto reset run on the copy, the proposed action first, then the backup policy's; the risk
+// latches to 1 where one of them ends the episode for a reason other than the trajectory length; the gate decides on it.
+static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
+                            cudaStream_t stream, const uint32_t* step_ptr) {
+    const int nj = env->host_scene.n_joints;
+    SmBuffers sv;
+    int rc;
+    if ((rc = shadow_copy(env, bv, e0, m, sv, stream))) return rc;
+    float* shadow_actions = const_cast<float*>(sv.actions);
+    const size_t n = (size_t)m;
     CU(cudaMemset2DAsync(sv.episode, 4 * sizeof(int32_t), 0, sizeof(int32_t), n, stream));   // episode_length = 0
     float* risk = env->d_risk + e0;
     CU(cudaMemsetAsync(risk, 0, n * sizeof(float), stream));
     MlpSeg kinem, rest;
     risk_observation(env, sv.obs, kinem, rest);
-    int rc;
     for (int i = 0; i <= env->lookahead_steps; ++i) {
         if (i > 0 && (rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0}, shadow_actions, nj, m, stream)))
             return rc;
@@ -1801,9 +1829,45 @@ static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int 
                        stream);
 }
 
+// The gate's next-state check (smenv_set_risk_next_state) over the envs of `bv` (m envs from env e0): the range's records
+// are copied into the shadow buffers with their episode clock as it is -- the simulated step is the real next step --; one
+// step without auto reset runs the proposed actions on the copy with the real step counter; the state risk network rates
+// the shadow's risk observation (float32 near the threshold in exact mode); the risk is set to 1 where the simulated step
+// ended its episode for a reason other than the trajectory length; the gate decides on it at its threshold.
+static int next_state_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
+                             cudaStream_t stream, const uint32_t* step_ptr) {
+    SmBuffers sv;
+    int rc;
+    if ((rc = shadow_copy(env, bv, e0, m, sv, stream))) return rc;
+    if ((rc = step_chain(env, sv, e0, m, chunk, 0, 0, nullptr, nullptr, nullptr, step_counter, 0, false, stream, step_ptr)))
+        return rc;
+    float* risk = env->d_risk + e0;
+    MlpSeg kinem, rest;
+    risk_observation(env, sv.obs, kinem, rest);
+    if ((rc = risk_rate(env, kinem, rest, MlpSeg{nullptr, 0, 0}, e0, m, chunk, env->gate_threshold, risk, stream))) return rc;
+    lookahead_latch_kernel<<<(m + 255) / 256, 256, 0, stream>>>(risk, sv.done, sv.term_reason, m);
+    env->launches++;
+    CU(cudaGetLastError());
+    return gate_decide(env, bv, e0, m, chunk, env->gate_threshold, risk, env->d_risky + e0,
+                       env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
+}
+
+// The gate's mode against the loaded risk network: the network gate needs a state-action network, the next-state check a
+// state network; the look-ahead does not consult it.
+static int gate_mode_check(const SmEnv* env, const char* who) {
+    if (env->lookahead_steps > 0) return SM_OK;
+    if (env->next_state && !risk_net_is_state(env))
+        return fail(SM_ERR_STATE, std::string(who) + ": the next-state check needs a state risk network (input: the risk "
+                                                     "observation)");
+    if (!env->next_state && risk_net_is_state(env))
+        return fail(SM_ERR_STATE, std::string(who) + ": the loaded risk network is a state network (input: the risk "
+                                                     "observation); the network gate needs a state-action network");
+    return SM_OK;
+}
+
 // One env step over the envs [e0, e0 + m) on `stream` with the work lists of slot `chunk` (step_chain): with the gate on
-// (actions.py:303-340) the proposed actions are rated first -- by the risk network, or by the look-ahead -- and the backup
-// policy's action is executed where they are risky.
+// (actions.py:303-340) the proposed actions are rated first -- by the risk network, by the look-ahead, or by the state risk
+// network on the simulated next state -- and the backup policy's action is executed where they are risky.
 static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chunk, int auto_reset, int random_actions,
                       uint32_t step_counter, bool tk, cudaStream_t stream, const uint32_t* step_ptr = nullptr) {
     const SmBuffers buf_v = buffers_at(*full, e0, env->host_scene.n_joints, env->host_scene.obs_size);
@@ -1812,6 +1876,7 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     float* exec = nullptr;
     if (gate) {
         if (!buf->obs) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the observation buffer");
+        if (int rc = gate_mode_check(env, "smenv_step")) return rc;
         if (random_actions) {
             if (!buf->actions) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the action buffer");
             random_actions_kernel<<<(m * env->host_scene.n_joints + 255) / 256, 256, 0, stream>>>(
@@ -1823,6 +1888,8 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
         exec = env->d_exec + (size_t)e0 * env->host_scene.n_joints;
         const int rc = env->lookahead_steps > 0
                            ? lookahead_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr)
+                       : env->next_state
+                           ? next_state_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr)
                            : gate_launch(env, buf_v, e0, m, chunk, env->gate_threshold, env->d_risk + e0, env->d_risky + e0,
                                          env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
         if (rc) return rc;
@@ -1924,7 +1991,7 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
 struct HostStepKey {
     SmBuffers buf;
     const void* h[4];
-    int auto_reset, chunks, count, pools, human_external, gate_exact, lookahead;
+    int auto_reset, chunks, count, pools, human_external, gate_exact, lookahead, next_state;
     float gate, gate_band;
 };
 
@@ -1999,7 +2066,7 @@ extern "C" int smenv_step_host(SmEnv* env, const SmBuffers* buf, const float* h_
     key.h[0] = h_actions; key.h[1] = h_obs; key.h[2] = h_reward; key.h[3] = h_done;
     key.auto_reset = auto_reset; key.chunks = chunks; key.count = env->count ? 1 : 0; key.pools = env->pools_filled ? 1 : 0; key.gate = env->gate_threshold;
     key.human_external = env->human_external ? 1 : 0; key.gate_exact = env->gate_exact ? 1 : 0; key.gate_band = env->gate_band;
-    key.lookahead = env->lookahead_steps;
+    key.lookahead = env->lookahead_steps; key.next_state = env->next_state;
     if (!env->host_graph || memcmp(&key, env->host_graph_key, sizeof(key)) != 0) {
         if (env->host_graph) { cudaGraphExecDestroy(env->host_graph); env->host_graph = nullptr; }
         const unsigned long long launches0 = env->launches;
@@ -2201,6 +2268,9 @@ extern "C" int smenv_risk_gate(SmEnv* env, const SmBuffers* buf, float threshold
                                SmStream s) {
     if (!env || !buf || !buf->actions || !buf->obs) return fail(SM_ERR_ARG, "smenv_risk_gate: null argument");
     if (!env->net_loaded[0] || !env->net_loaded[1]) return fail(SM_ERR_STATE, "smenv_risk_gate: load both networks first");
+    if (risk_net_is_state(env))
+        return fail(SM_ERR_STATE, "smenv_risk_gate: the loaded risk network is a state network; this call rates (state, "
+                                  "action) pairs");
     cudaStream_t stream = (cudaStream_t)s;
     DevLock dev_lock_(env); int rc = activate(env, stream);
     if (rc) return rc;
@@ -2212,7 +2282,50 @@ extern "C" int smenv_set_risk_gate(SmEnv* env, float threshold) {
     if (!env) return fail(SM_ERR_ARG, "smenv_set_risk_gate: null env");
     if (threshold >= 0.0f && (!env->net_loaded[0] || !env->net_loaded[1]))
         return fail(SM_ERR_STATE, "smenv_set_risk_gate: load the risk network and the backup policy first (smenv_mlp_load)");
+    if (threshold >= 0.0f) {
+        const int rc = gate_mode_check(env, "smenv_set_risk_gate");
+        if (rc) return rc;
+    }
     env->gate_threshold = threshold >= 0.0f ? threshold : -1.0f;
+    return SM_OK;
+}
+
+// The shadow buffers of the look-ahead and of the next-state check, allocated on the first enable of either and freed by
+// smenv_destroy: every record the step writes, and a stats vector nobody reads.
+static int shadow_alloc(SmEnv* env, const char* who) {
+    if (!env->la_allocs.empty()) return SM_OK;
+    CU(cudaSetDevice(env->device));
+    const size_t n = (size_t)env->n;
+    const DevScene& hs = env->host_scene;
+    SmBuffers& b = env->la_buf;
+    float* actions = nullptr;
+    const struct { void** p; size_t bytes; bool used; } recs[] = {
+        {(void**)&b.kin, n * SM_KIN_STRIDE * sizeof(double), true}, {(void**)&b.obst, n * SM_OBST_STRIDE * sizeof(double), true},
+        {(void**)&b.episode, n * 4 * sizeof(int32_t), true}, {(void**)&b.ep_return, n * sizeof(double), true},
+        {(void**)&b.target, n * SM_TP_STRIDE * sizeof(double), hs.use_target_points != 0},
+        {(void**)&b.obs, n * hs.obs_size * sizeof(float), true}, {(void**)&b.reward, n * sizeof(float), true},
+        {(void**)&b.done, n, true}, {(void**)&b.term_reason, n * sizeof(int32_t), true},
+        {(void**)&b.info, n * SM_INFO_STRIDE * sizeof(float), true},
+        {(void**)&b.epacc, n * SM_EP_STRIDE * sizeof(float), true}, {(void**)&b.epinfo, n * SM_EP_STRIDE * sizeof(float), true},
+        {(void**)&actions, n * hs.n_joints * sizeof(float), true},
+        {(void**)&b.hkin, n * SM_KIN_STRIDE * sizeof(double), env->human},
+        {(void**)&b.hstate, n * SM_HSTATE_STRIDE * sizeof(double), env->human},
+        {(void**)&b.hbrake, n * SM_HBRAKE_STEPS * SM_HUMAN_JOINTS * sizeof(double), env->human},
+        {(void**)&b.hobs, n * SM_HOBS_STRIDE * sizeof(float), env->human},
+        {(void**)&b.hactions, n * SM_HUMAN_JOINTS * sizeof(float), env->human},
+        {(void**)&b.stats, 32 * sizeof(double), true}};   // the shadow steps' episode statistics: nobody reads them
+    for (const auto& r : recs) {
+        if (!r.used) continue;
+        const cudaError_t e = cudaMalloc(r.p, r.bytes);
+        if (e != cudaSuccess) {
+            for (void* q : env->la_allocs) cudaFree(q);
+            env->la_allocs.clear();
+            b = SmBuffers{};
+            return fail(SM_ERR_CUDA, std::string(who) + ": cudaMalloc: " + cudaGetErrorString(e));
+        }
+        env->la_allocs.push_back(*r.p);
+    }
+    b.actions = actions;
     return SM_OK;
 }
 
@@ -2221,41 +2334,36 @@ extern "C" int smenv_set_risk_lookahead(SmEnv* env, int backup_steps) {
     if (backup_steps < 0) return fail(SM_ERR_ARG, "smenv_set_risk_lookahead: backup_steps must be >= 0");
     if (backup_steps > 0 && !env->net_loaded[SM_NET_BACKUP])
         return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: load the backup policy first (smenv_mlp_load)");
-    if (backup_steps > 0 && env->la_allocs.empty()) {
-        CU(cudaSetDevice(env->device));
-        const size_t n = (size_t)env->n;
-        const DevScene& hs = env->host_scene;
-        SmBuffers& b = env->la_buf;
-        float* actions = nullptr;
-        const struct { void** p; size_t bytes; bool used; } recs[] = {
-            {(void**)&b.kin, n * SM_KIN_STRIDE * sizeof(double), true}, {(void**)&b.obst, n * SM_OBST_STRIDE * sizeof(double), true},
-            {(void**)&b.episode, n * 4 * sizeof(int32_t), true}, {(void**)&b.ep_return, n * sizeof(double), true},
-            {(void**)&b.target, n * SM_TP_STRIDE * sizeof(double), hs.use_target_points != 0},
-            {(void**)&b.obs, n * hs.obs_size * sizeof(float), true}, {(void**)&b.reward, n * sizeof(float), true},
-            {(void**)&b.done, n, true}, {(void**)&b.term_reason, n * sizeof(int32_t), true},
-            {(void**)&b.info, n * SM_INFO_STRIDE * sizeof(float), true},
-            {(void**)&b.epacc, n * SM_EP_STRIDE * sizeof(float), true}, {(void**)&b.epinfo, n * SM_EP_STRIDE * sizeof(float), true},
-            {(void**)&actions, n * hs.n_joints * sizeof(float), true},
-            {(void**)&b.hkin, n * SM_KIN_STRIDE * sizeof(double), env->human},
-            {(void**)&b.hstate, n * SM_HSTATE_STRIDE * sizeof(double), env->human},
-            {(void**)&b.hbrake, n * SM_HBRAKE_STEPS * SM_HUMAN_JOINTS * sizeof(double), env->human},
-            {(void**)&b.hobs, n * SM_HOBS_STRIDE * sizeof(float), env->human},
-            {(void**)&b.hactions, n * SM_HUMAN_JOINTS * sizeof(float), env->human},
-            {(void**)&b.stats, 32 * sizeof(double), true}};   // the shadow steps' episode statistics: nobody reads them
-        for (const auto& r : recs) {
-            if (!r.used) continue;
-            const cudaError_t e = cudaMalloc(r.p, r.bytes);
-            if (e != cudaSuccess) {
-                for (void* q : env->la_allocs) cudaFree(q);
-                env->la_allocs.clear();
-                b = SmBuffers{};
-                return fail(SM_ERR_CUDA, std::string("smenv_set_risk_lookahead: cudaMalloc: ") + cudaGetErrorString(e));
-            }
-            env->la_allocs.push_back(*r.p);
-        }
-        b.actions = actions;
+    if (backup_steps > 0 && env->next_state)
+        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: the next-state check is on (smenv_set_risk_next_state)");
+    if (backup_steps > 0) {
+        const int rc = shadow_alloc(env, "smenv_set_risk_lookahead");
+        if (rc) return rc;
+    } else if (env->gate_threshold >= 0.0f && !env->next_state && risk_net_is_state(env)) {
+        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: the gate is on with a state risk network; switch it off first "
+                                  "(smenv_set_risk_gate)");
     }
     env->lookahead_steps = backup_steps;
+    return SM_OK;
+}
+
+extern "C" int smenv_set_risk_next_state(SmEnv* env, int enable) {
+    if (!env) return fail(SM_ERR_ARG, "smenv_set_risk_next_state: null env");
+    if (enable) {
+        if (!env->net_loaded[SM_NET_BACKUP])
+            return fail(SM_ERR_STATE, "smenv_set_risk_next_state: load the backup policy first (smenv_mlp_load)");
+        if (!risk_net_is_state(env))
+            return fail(SM_ERR_STATE, "smenv_set_risk_next_state: load a state risk network first (smenv_mlp_load, input: "
+                                      "the risk observation)");
+        if (env->lookahead_steps > 0)
+            return fail(SM_ERR_STATE, "smenv_set_risk_next_state: the look-ahead is on (smenv_set_risk_lookahead)");
+        const int rc = shadow_alloc(env, "smenv_set_risk_next_state");
+        if (rc) return rc;
+    } else if (env->gate_threshold >= 0.0f && env->lookahead_steps == 0 && risk_net_is_state(env)) {
+        return fail(SM_ERR_STATE, "smenv_set_risk_next_state: the gate is on with a state risk network; switch it off first "
+                                  "(smenv_set_risk_gate)");
+    }
+    env->next_state = enable != 0;
     return SM_OK;
 }
 

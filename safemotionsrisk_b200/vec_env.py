@@ -134,9 +134,11 @@ class SafeMotionsVecEnv:
         # the risk network (its backup policy comes with it), risk_threshold switches the gate on inside step()
         if self.config.risk_config_dir is not None:
             self.load_networks(self._resolve_risk_config_dir(self.config.risk_config_dir))
-            self.set_risk_gate(self.config.risk_threshold)
-            if self.config.risk_state_config == 4:
+            if self.config.risk_state_config == 3:
+                self.set_risk_next_state(True)
+            elif self.config.risk_state_config == 4:
                 self.set_risk_lookahead(self.config.risk_state_backup_trajectory_steps or 20)
+            self.set_risk_gate(self.config.risk_threshold)
             if self.config.risk_check_initial_backup_trajectory and not fill_pools:
                 raise ValueError("risk_check_initial_backup_trajectory needs the start pools (fill_pools=True)")
 
@@ -205,6 +207,16 @@ class SafeMotionsVecEnv:
         risk_ground_truth.  The risk network is not consulted, so the threshold does not change the decision.  0 or None
         switches back to the network gate (smenv_set_risk_lookahead).  Needs the backup policy (load_networks)."""
         cabi.check(self._lib.smenv_set_risk_lookahead(self._handle, int(backup_steps or 0)), "smenv_set_risk_lookahead")
+
+    def set_risk_next_state(self, enable):
+        """risk_state_config 3 (RISK_CHECK_NEXT_STATE_SIMULATE_NEXT_STEP) inside the step: while the risk gate is on, a
+        copy of every env executes the proposed action for one step (no auto reset, the episode clock as it is, the real
+        step's random stream), and the action is risky when the state risk network rates the state it leads to >= the
+        threshold, or when that step ends the episode for a reason other than the trajectory length
+        (smenv_set_risk_next_state).  Needs a state risk network (input: the risk observation alone; risk_train on
+        state_risk data) and the backup policy (load_networks).  False switches back; with the gate on and a state network
+        loaded, switch the gate off first."""
+        cabi.check(self._lib.smenv_set_risk_next_state(self._handle, int(bool(enable))), "smenv_set_risk_next_state")
 
     def close(self):
         if self._handle:
@@ -611,9 +623,20 @@ class SafeMotionsVecEnv:
         pol = [(wp["backup/{}/kernel".format(n)], wp["backup/{}/bias".format(n)]) for n in ("fc_1", "fc_2", "fc_out")]
         pol[-1] = (pol[-1][0][:, :nj], pol[-1][1][:nj])  # deterministic action = the mean head
         risk_obs = self.scene.obs_size - self.scene.obs_target_size   # without the target-point entries
-        if risk[0][0].shape[0] != risk_obs + nj or pol[0][0].shape[0] != risk_obs:
+        if risk[0][0].shape[0] not in (risk_obs, risk_obs + nj) or pol[0][0].shape[0] != risk_obs:
             raise ValueError("networks expect a risk observation of size {}, the env produces {}".format(
                 pol[0][0].shape[0], risk_obs))
+        # the risk network's kind by its input width: the risk observation alone (a state network, risk_train on
+        # state_risk data) or followed by the action (a state-action network, the shipped ones)
+        kind = "state" if risk[0][0].shape[0] == risk_obs else "state_action"
+        if kind == "state" and self.config.risk_state_config not in (3, 4):
+            raise ValueError("{}: a state risk network (input: the risk observation, {} values) rates states, not "
+                             "actions; the network gate of risk_state_config={} needs a state-action network (input {}); "
+                             "risk_state_config=3 rates the simulated next state with it".format(
+                                 source, risk_obs, self.config.risk_state_config, risk_obs + nj))
+        if kind == "state_action" and self.config.risk_state_config == 3:
+            raise NotImplementedError("{}: risk_state_config=3 rates the simulated next state with a state risk network; "
+                                      "rating it with a state-action network is not implemented".format(source))
         risk_hidden = 0
         if "risk/hidden_layer_activation" in w.files:   # written by risk_train.export_weights
             act, last = str(w["risk/hidden_layer_activation"]), str(w["risk/last_layer_activation"])
@@ -631,6 +654,7 @@ class SafeMotionsVecEnv:
         self.risky = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
         self._networks = True
         self._network_source = source
+        self.risk_network_kind = kind
 
     def mlp_forward(self, which, in0, in1=None, n_out=1):
         """Parity hook: the loaded network `which` (0 risk, 1 backup policy) on caller-supplied rows."""
@@ -742,6 +766,16 @@ class SafeMotionsVecEnv:
             self.auto_reset = auto
             self.set_risk_gate(gate)
         return state, act, risky.float()
+
+    def state_risk_ground_truth(self, backup_steps=20):
+        """Ground truth of the state risk (the labels a state risk network learns, risk_state_config 3): from a copy of
+        the current state the backup policy acts for `backup_steps` steps with the episode clock at 0 and no auto reset;
+        a state is risky (1.0) if its episode ends in that window for any reason other than the trajectory length --
+        initial_backup_trajectory_unsafe's rule.  The env state is restored afterwards.  Returns (risk_observation [N, D],
+        risk [N]) as device tensors: rows for risk_data.write_risk_csv(directory, state, risk) (state_risk files)."""
+        state = self.risk_observation().clone()
+        risk = self.initial_backup_trajectory_unsafe(int(backup_steps)).float()
+        return state, risk
 
     KERNELS = ("human_policy", "human_joint_kernels", "human_brake_traj_kernel", "human_brake_plan_kernel",
                "human_brake_gjk", "human_advance_outcome", "joint_kernel", "joint_heavy_kernel", "contact_plan_kernel",

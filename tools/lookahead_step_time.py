@@ -1,21 +1,30 @@
 #!/usr/bin/env python
 """Step time of the risk check inside the step, 65 536 envs by default: no gate, the network gate (risk network +
-backup policy) and the backup-trajectory look-ahead (risk_state_config 4, K backup steps, smenv_set_risk_lookahead), on
-space_task_bm (the env of BASELINE.json configs[3]) and human.  Random-action rollout with auto reset; every variant is
-warmed up, then `--steps` steps are timed one by one with CUDA events, the L2 flushed (256 MiB write) between them as
-bench.py does.  Prints one JSON line: ms per step and env-steps/s per variant, the ratio look-ahead / ungated, and the
-GPU's name and power limit read in the same run."""
+backup policy), the next-state check (risk_state_config 3: one simulated step and a state risk network,
+smenv_set_risk_next_state) and the backup-trajectory look-ahead (risk_state_config 4, K backup steps,
+smenv_set_risk_lookahead), on space_task_bm (the env of BASELINE.json configs[3]) and human.  The next-state check uses
+the state network of `--state-risk-net` (an .npz written by risk_train) or, without it, a seeded random one with the
+shipped risk network's hidden widths (512 / 256 / 128, selu, sigmoid), its threshold at the median of its risk over the
+reset states unless `--state-risk-threshold` is given; `risky_fraction` matters there, because in exact mode the float32
+backup work grows with it.  Random-action rollout with auto reset; every variant is warmed up, then `--steps` steps are
+timed one by one with CUDA events, the L2 flushed (256 MiB write) between them as bench.py does.  Prints one JSON line:
+ms per step and env-steps/s per variant, the ratios to the ungated step, and the GPU's name and power limit read in the
+same run."""
 import argparse
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch  # noqa: E402
 
 from bench import scene_config  # noqa: E402
-from safemotionsrisk_b200 import abi  # noqa: E402
+from safemotionsrisk_b200 import abi, risk_train  # noqa: E402
+from safemotionsrisk_b200.config import EnvConfig  # noqa: E402
+from safemotionsrisk_b200.scene import Scene  # noqa: E402
 from safemotionsrisk_b200.vec_env import SafeMotionsVecEnv  # noqa: E402
 
 THRESHOLD = {"space_task_bm": 0.065, "human": 0.06}   # README.md:223-235, as bench.py --risk-gate
@@ -49,6 +58,30 @@ def time_variant(env, steps, warmup, flush):
             "risky_fraction": float(risky.item()) / (env.num_envs * steps)}
 
 
+def random_state_net(scene, path, seed=0):
+    """A seeded random state risk network for `scene` (risk observation -> 512 -> 256 -> 128 -> 1) written to `path`."""
+    sc = Scene(scene_config(scene))
+    torch.manual_seed(seed)
+    model = risk_train.build_model(sc.obs_size - sc.obs_target_size, [512, 256, 128], "selu")
+    risk_train.export_weights(model, path, "selu", "sigmoid")
+    return path
+
+
+def time_next_state(scene, args, flush, tmp):
+    net = args.state_risk_net or random_state_net(scene, os.path.join(tmp, "state_net_{}.npz".format(scene)))
+    cfg = EnvConfig(**dict(scene_config(scene), risk_config_dir=net, risk_threshold=0.5, risk_state_config=3))
+    env = SafeMotionsVecEnv(num_envs=args.envs, config=cfg, seed=1)
+    env.reset()
+    thr = args.state_risk_threshold
+    if thr is None:
+        thr = float(torch.quantile(env.mlp_forward(0, env.risk_observation())[:, 0], 0.5).item())
+    env.set_risk_gate(thr)
+    r = time_variant(env, args.steps, args.warmup, flush)
+    r.update(threshold=thr, state_risk_net=args.state_risk_net or "random (seed 0, 512/256/128)")
+    env.close()
+    return r
+
+
 def main():
     p = argparse.ArgumentParser(description=__doc__)
     p.add_argument("--envs", type=int, default=65536)
@@ -56,6 +89,8 @@ def main():
     p.add_argument("--warmup", type=int, default=10)
     p.add_argument("--backup-steps", type=int, default=20)
     p.add_argument("--scenes", default="space_task_bm,human")
+    p.add_argument("--state-risk-net", default=None, help="state risk network (.npz) of the next-state variant")
+    p.add_argument("--state-risk-threshold", type=float, default=None)
     args = p.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("lookahead_step_time.py needs a CUDA device")
@@ -64,6 +99,7 @@ def main():
     result = {"tool": "lookahead_step_time", "gpu": torch.cuda.get_device_name(dev), "power_limit_w": power_limit_w(dev),
               "envs": args.envs, "steps": args.steps, "warmup": args.warmup, "backup_steps": args.backup_steps,
               "l2": "flushed between timed steps (256 MiB write)", "scenes": {}}
+    tmp = tempfile.mkdtemp(prefix="lookahead_step_time_")
     for scene in args.scenes.split(","):
         env = SafeMotionsVecEnv(num_envs=args.envs, config=scene_config(scene), seed=1)
         env.load_networks()
@@ -76,9 +112,12 @@ def main():
         env.set_risk_lookahead(args.backup_steps)
         r["lookahead"] = time_variant(env, args.steps, args.warmup, flush)
         r["lookahead_over_ungated"] = r["lookahead"]["ms_per_step"] / r["ungated"]["ms_per_step"]
-        result["scenes"][scene] = r
         env.close()
         del env
+        r["next_state"] = time_next_state(scene, args, flush, tmp)
+        r["next_state_over_ungated"] = r["next_state"]["ms_per_step"] / r["ungated"]["ms_per_step"]
+        result["scenes"][scene] = r
+    shutil.rmtree(tmp, ignore_errors=True)
     print(json.dumps(result))
 
 

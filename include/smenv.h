@@ -485,6 +485,25 @@ int smenv_set_risk_lookahead(SmEnv* env, int backup_steps);
  * policy is not loaded, the loaded risk network is not a state network or the look-ahead is on; enable = 0 with the gate
  * on and a state network loaded returns SM_ERR_STATE as well (the network gate cannot use that network). */
 int smenv_set_risk_next_state(SmEnv* env, int enable);
+/* Initial-backup-trajectory check of the start pool (risk_check_initial_backup_trajectory, observations.py:155-185).
+ * A reset copies a start-pool entry into the env verbatim (robot and obstacle records; in the Human scene the paired human
+ * start state and its stored braking trajectory), so the check is a property of the entry and runs once per entry when
+ * the pool is filled.  backup_steps = K > 0: every entry is reset into the shadow buffers of smenv_set_risk_lookahead
+ * (allocated here if needed) and the backup policy acts for K steps with the episode clock from 0, no auto reset and the
+ * gate off; the entry fails when one of those steps ends its episode for a reason other than SM_TERM_TRAJECTORY_LENGTH.
+ * The pool is checked in batches of at most num_envs entries; env i of a batch draws from the Philox streams of its pool
+ * entry, with step counters of its own (the Human and Ball scenes are stochastic: a verdict is one sample).  The pool is
+ * then partitioned stably -- passing entries first in their original order, failing entries after them -- and every reset
+ * (smenv_reset, the auto reset of the step, the human's reset with it) draws from the passing entries only: rejection
+ * sampling from the pool, with no per-step cost.  The real env's buffers, statistics and step counter are not touched.
+ * The call checks the current pools if they are filled and every later smenv_fill_pools does the same; it synchronises
+ * `stream` once per check.  SM_ERR_STATE without a loaded backup policy, or when no entry passes (the pool then stays in
+ * its original order and resets draw from all of it).  backup_steps = 0 switches the check off: resets draw from the whole
+ * pool again; the checked order stays until the next smenv_fill_pools, which restores the unchecked pool exactly. */
+int smenv_set_initial_backup_check(SmEnv* env, int backup_steps, SmStream stream);
+/* checked: the start-pool entries the check rated for the current pools (0 while the check is off or the pools are not
+ * filled); passed: the leading entries resets draw from (the passing entries; the whole pool while the check is off). */
+int smenv_initial_backup_check_counts(SmEnv* env, int* checked, int* passed);
 /* Exact gate (default on): the tensor-core risk (fp16 operands) of the rows within `band` of the threshold is re-computed
  * in float32 on the CUDA cores before the decision, and the backup policy's action of the risky rows is computed in
  * float32 too, so that decisions and executed actions are those of a float32 evaluation of the shipped networks

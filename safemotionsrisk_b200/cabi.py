@@ -60,6 +60,8 @@ def load():
     lib.smenv_set_risk_gate.argtypes = [vp, C.c_float]
     lib.smenv_set_risk_lookahead.argtypes = [vp, i32]
     lib.smenv_set_risk_next_state.argtypes = [vp, i32]
+    lib.smenv_set_initial_backup_check.argtypes = [vp, i32, vp]
+    lib.smenv_initial_backup_check_counts.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
     lib.smenv_random_actions.argtypes = [vp, C.POINTER(abi.SmBuffers), vp]
     lib.smenv_kernel_timing.argtypes = [vp, i32]
     lib.smenv_kernel_times.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32), i32]

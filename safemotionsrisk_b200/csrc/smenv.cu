@@ -186,6 +186,14 @@ struct SmEnv {
     double* d_target_pool = nullptr;   // [target_pool_n][4] target points of the reaching task
     int target_pool_n = 0;
     int start_pool_n = 0, ball_pool_n = 0;
+    int start_draw_n = 0;        // leading start-pool entries resets draw from: start_pool_n, or the passing entries of the
+                                 // initial-backup-trajectory check (smenv_set_initial_backup_check)
+    int init_check_steps = 0;    // > 0: every pool fill checks the start pool with that many backup-policy steps
+    int init_checked = 0;        // entries the check rated for the current pools
+    float* d_pool_verdict = nullptr;   // [start_pool_n] 1: the entry's backup trajectory ends in a collision
+    int* d_pool_entry = nullptr;       // [start_pool_n] 0, 1, 2 ...: the pool entry of every env of a check batch
+    int* d_pool_dest = nullptr;        // [start_pool_n + 1] new position of every entry, then the passing count
+    double* d_pool_scratch = nullptr;  // scatter target of the compaction (the largest pool array)
     bool pools_filled = false;
     unsigned long long* d_counters = nullptr;
     float* d_scratch = nullptr;  // per-env hand-over between the phase kernels of a step
@@ -215,6 +223,7 @@ struct SmEnv {
     int next_state = 0;            // the gate rates the simulated next state with a state risk network (smenv_set_risk_next_state)
     SmBuffers la_buf = {};         // [n] shadow copy of every record the step writes, and a stats vector nobody reads
     std::vector<void*> la_allocs;
+    std::vector<size_t> la_bytes;
     // Human scene (smenv_human.cuh)
     bool human = false;
     int human_external = 0;        // the human's actions come from buf->hactions (parity protocol)
@@ -904,6 +913,7 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
     }
     // pools: one start state per env is plenty of variety up to 65536; balls are consumed faster
     env->start_pool_n = num_envs < 65536 ? (num_envs < 1024 ? 1024 : num_envs) : 65536;
+    env->start_draw_n = env->start_pool_n;
     env->ball_pool_n = (sc->n_obstacles > 0 && sc->obst_kind[0] == SM_OBST_BALL) ? 4 * env->start_pool_n : 0;
     CU(cudaMalloc((void**)&env->d_start_pool, (size_t)env->start_pool_n * SM_POOL_STRIDE * sizeof(double)));
     CU(cudaMemset(env->d_start_pool, 0, (size_t)env->start_pool_n * SM_POOL_STRIDE * sizeof(double)));
@@ -1081,6 +1091,7 @@ extern "C" int smenv_destroy(SmEnv* env) {
     cudaFree(env->d_step);
     for (void* q : env->net_allocs) cudaFree(q);
     for (void* q : env->la_allocs) cudaFree(q);
+    cudaFree(env->d_pool_verdict); cudaFree(env->d_pool_entry); cudaFree(env->d_pool_dest); cudaFree(env->d_pool_scratch);
     cudaFree(env->d_risk); cudaFree(env->d_backup); cudaFree(env->d_exec); cudaFree(env->d_risky); cudaFree(env->d_gate_list);
     cudaFree(env->d_hpairs); cudaFree(env->d_hthresh); cudaFree(env->d_hrange); cudaFree(env->d_hbacc); cudaFree(env->d_hposes);
     cudaFree(env->d_hbinfo); cudaFree(env->d_hunits); cudaFree(env->d_hscratch); cudaFree(env->d_hpolicy); cudaFree(env->d_hstart_pool); cudaFree(env->d_hpool_brake); cudaFree(env->d_hpool_bcount); cudaFree(env->d_htarget_pool);
@@ -1136,6 +1147,8 @@ extern "C" int smenv_copy_pools(SmEnv* env, double* host_start, double* host_bal
     return SM_OK;
 }
 
+static int pool_check_launch(SmEnv* env, cudaStream_t stream);
+
 extern "C" int smenv_fill_pools(SmEnv* env, uint64_t seed, SmStream s) {
     if (!env) return fail(SM_ERR_ARG, "null env");
     cudaStream_t stream = (cudaStream_t)s;
@@ -1165,6 +1178,9 @@ extern "C" int smenv_fill_pools(SmEnv* env, uint64_t seed, SmStream s) {
     }
     CU(cudaGetLastError());
     env->pools_filled = true;
+    env->start_draw_n = env->start_pool_n;
+    env->init_checked = 0;
+    if (env->init_check_steps > 0) return pool_check_launch(env, stream);
     return SM_OK;
 }
 
@@ -1293,8 +1309,8 @@ extern "C" int smenv_reset(SmEnv* env, const SmBuffers* buf, const uint8_t* mask
     cudaStream_t stream = (cudaStream_t)s;
     DevLock dev_lock_(env); int rc = activate(env, stream);
     if (rc) return rc;
-    ResetArgs A{*buf, env->n, mask, env->d_start_pool, env->start_pool_n, env->d_target_pool, env->target_pool_n,
-                (uint32_t)env->seed, (uint32_t)(env->seed >> 32)};
+    ResetArgs A{*buf, env->n, mask, env->d_start_pool, env->start_draw_n, env->d_target_pool, env->target_pool_n,
+                (uint32_t)env->seed, (uint32_t)(env->seed >> 32), nullptr};
     reset_kernel<<<(env->n * 32 + 255) / 256, 256, 0, stream>>>(A);
     env->launches++;
     if (env->human) {
@@ -1303,7 +1319,7 @@ extern "C" int smenv_reset(SmEnv* env, const SmBuffers* buf, const uint8_t* mask
         HumanArgs H;
         memset(&H, 0, sizeof(H));
         H.buf = *buf; H.n = env->n; H.env_base = 0; H.k0 = (uint32_t)env->seed; H.k1 = (uint32_t)(env->seed >> 32);
-        H.mask = mask; H.start_pool = env->d_hstart_pool; H.start_pool_n = env->start_pool_n;
+        H.mask = mask; H.start_pool = env->d_hstart_pool; H.start_pool_n = env->start_draw_n;
         H.pool_brake = env->d_hpool_brake; H.pool_bcount = env->d_hpool_bcount;
         H.target_pool = env->d_htarget_pool; H.target_pool_n = env->htarget_pool_n;
         human_reset_kernel<<<(env->n * 8 + 255) / 256, 256, 0, stream>>>(H, 0);
@@ -1543,9 +1559,12 @@ static void launch_gjk(SmEnv* env, const GjkArgs& G, cudaStream_t stream) {
 // ranges back to back, the range's sub-list starting at entry k * e0 + chunk (its own count first).  Ranges in flight at
 // once need distinct slots.  exec: the actions to execute (NULL: bv.actions); risk / risky: the gate's outcome for the info
 // record (NULL: gate off).  The Philox step counter is step_counter + sub (step_ptr: read from device memory, plus sub).
+// stream_e0: the Philox stream index of env 0 of the view (-1: e0; the pool check runs its batches in the view of envs
+// [0, m) with the streams of their pool entries).
 static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, int auto_reset, int random_actions,
                       const float* exec, const float* risk, const uint8_t* risky, uint32_t step_counter, uint32_t sub,
-                      bool tk, cudaStream_t stream, const uint32_t* step_ptr) {
+                      bool tk, cudaStream_t stream, const uint32_t* step_ptr, int stream_e0 = -1) {
+    if (stream_e0 < 0) stream_e0 = e0;
     const SmBuffers* buf = &bv;
     const int per_env_items = env->item_capacity / env->n;
     int* worklist = env->d_worklist + 2 * chunk;
@@ -1560,7 +1579,7 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
     JA.buf = *buf; JA.n = m; JA.random_actions = random_actions;
     JA.k0 = (uint32_t)env->seed; JA.k1 = (uint32_t)(env->seed >> 32);
     JA.step_counter = step_counter + sub;
-    JA.env_base = e0;
+    JA.env_base = stream_e0;
     JA.scratch = scratch;
     JA.worklist = worklist;  // clears the item counter and the overflow count
     JA.heavy = heavy;
@@ -1612,7 +1631,7 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
         // ---------------- the nested env of the human up to its setpoints (Human.step, ctlp.py:4818-4840)
         if (!buf->hkin || !buf->hstate || !buf->hbrake || !buf->hobs || !buf->hactions)
             return fail(SM_ERR_ARG, "smenv_step: the Human scene needs the hkin / hstate / hbrake / hobs / hactions buffers");
-        HA.buf = *buf; HA.n = m; HA.env_base = e0;
+        HA.buf = *buf; HA.n = m; HA.env_base = stream_e0;
         HA.k0 = (uint32_t)env->seed; HA.k1 = (uint32_t)(env->seed >> 32); HA.step_counter = step_counter + sub;
         HA.step_offset = sub;
         HA.step_ptr = step_ptr;   // host-buffer step: the counter lives in device memory (graph replays)
@@ -1630,7 +1649,7 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
         HA.target_pool_n = env->pools_filled ? env->htarget_pool_n : 0;
         HA.start_pool = env->pools_filled ? env->d_hstart_pool : nullptr;
         HA.pool_brake = env->pools_filled ? env->d_hpool_brake : nullptr; HA.pool_bcount = env->d_hpool_bcount;
-        HA.start_pool_n = env->pools_filled ? env->start_pool_n : 0;
+        HA.start_pool_n = env->pools_filled ? env->start_draw_n : 0;
         HA.cwork = cwork;
         HA.counters = env->count ? env->d_counters : nullptr;
         SM_MARK(SM_K_HUMAN_POLICY);
@@ -1704,14 +1723,14 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
     StepArgs A;
     A.buf = *buf; A.n = m; A.auto_reset = auto_reset;
     A.k0 = (uint32_t)env->seed; A.k1 = (uint32_t)(env->seed >> 32);
-    A.env_base = e0;
+    A.env_base = stream_e0;
     A.scratch = scratch;
     A.res = res;
     A.heavy = heavy;
     A.overflow = worklist + 1;
     A.host_flag = env->d_flag;
     A.start_pool = env->pools_filled ? env->d_start_pool : nullptr;
-    A.start_pool_n = env->pools_filled ? env->start_pool_n : 0;
+    A.start_pool_n = env->pools_filled ? env->start_draw_n : 0;
     A.ball_pool = env->pools_filled ? env->d_ball_pool : nullptr;
     A.ball_pool_n = env->pools_filled ? env->ball_pool_n : 0;
     A.target_pool = env->pools_filled ? env->d_target_pool : nullptr;
@@ -1991,7 +2010,7 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
 struct HostStepKey {
     SmBuffers buf;
     const void* h[4];
-    int auto_reset, chunks, count, pools, human_external, gate_exact, lookahead, next_state;
+    int auto_reset, chunks, count, pools, start_draw_n, human_external, gate_exact, lookahead, next_state;
     float gate, gate_band;
 };
 
@@ -2066,7 +2085,7 @@ extern "C" int smenv_step_host(SmEnv* env, const SmBuffers* buf, const float* h_
     key.h[0] = h_actions; key.h[1] = h_obs; key.h[2] = h_reward; key.h[3] = h_done;
     key.auto_reset = auto_reset; key.chunks = chunks; key.count = env->count ? 1 : 0; key.pools = env->pools_filled ? 1 : 0; key.gate = env->gate_threshold;
     key.human_external = env->human_external ? 1 : 0; key.gate_exact = env->gate_exact ? 1 : 0; key.gate_band = env->gate_band;
-    key.lookahead = env->lookahead_steps; key.next_state = env->next_state;
+    key.lookahead = env->lookahead_steps; key.next_state = env->next_state; key.start_draw_n = env->start_draw_n;
     if (!env->host_graph || memcmp(&key, env->host_graph_key, sizeof(key)) != 0) {
         if (env->host_graph) { cudaGraphExecDestroy(env->host_graph); env->host_graph = nullptr; }
         const unsigned long long launches0 = env->launches;
@@ -2320,10 +2339,12 @@ static int shadow_alloc(SmEnv* env, const char* who) {
         if (e != cudaSuccess) {
             for (void* q : env->la_allocs) cudaFree(q);
             env->la_allocs.clear();
+            env->la_bytes.clear();
             b = SmBuffers{};
             return fail(SM_ERR_CUDA, std::string(who) + ": cudaMalloc: " + cudaGetErrorString(e));
         }
         env->la_allocs.push_back(*r.p);
+        env->la_bytes.push_back(r.bytes);
     }
     b.actions = actions;
     return SM_OK;
@@ -2364,6 +2385,132 @@ extern "C" int smenv_set_risk_next_state(SmEnv* env, int enable) {
                                   "(smenv_set_risk_gate)");
     }
     env->next_state = enable != 0;
+    return SM_OK;
+}
+
+// The initial-backup-trajectory check of the start pool (smenv_set_initial_backup_check; observations.py:155-185): every
+// entry is reset into the shadow buffers -- robot record, obstacle record and, in the Human scene, its paired human start
+// state and stored braking trajectory, as a reset copies them into an env -- and the backup policy acts for K steps
+// without auto reset and with the gate off; the entry fails when one of them ends its episode for a reason other than the
+// trajectory length (the rule of initial_backup_trajectory_unsafe).  The shadow buffers hold n envs, so the pool is
+// checked in batches of at most n entries.  Env i of the batch from entry `offset` draws from the Philox streams of entry
+// offset + i with the step counters SM_POOL_CHECK_STEP0 + sub-step (a range the real step counter does not reach in
+// practice): entries of different batches share no human-noise, human-target or ball-draw stream, and a verdict depends
+// on the seed and the entry's position alone, not on n.  The pool is then partitioned stably by verdict -- passing entries
+// first, every array indexed by the entry moved together -- and resets draw from the passing ones.  The real env's
+// buffers, statistics and step counter are not touched.
+#define SM_POOL_CHECK_STEP0 0x80000000u
+
+template <typename T>
+static int pool_compact(SmEnv* env, T* arr, int stride, cudaStream_t stream) {
+    T* tmp = reinterpret_cast<T*>(env->d_pool_scratch);
+    const size_t total = (size_t)env->start_pool_n * stride;
+    pool_scatter_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(arr, tmp, env->d_pool_dest, env->start_pool_n,
+                                                                               stride);
+    env->launches++;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(arr, tmp, total * sizeof(T), cudaMemcpyDeviceToDevice, stream));
+    return SM_OK;
+}
+
+static int pool_check_launch(SmEnv* env, cudaStream_t stream) {
+    const int P = env->start_pool_n, K = env->init_check_steps, nj = env->host_scene.n_joints;
+    const uint32_t k0 = (uint32_t)env->seed, k1 = (uint32_t)(env->seed >> 32);
+    int rc = set_list_layout(env, 1, stream);   // the batches use the work lists of slot 0 over up to n envs
+    if (rc) return rc;
+    CU(cudaMemsetAsync(env->d_pool_verdict, 0, (size_t)P * sizeof(float), stream));
+    const SmBuffers& sv = env->la_buf;
+    float* shadow_actions = const_cast<float*>(sv.actions);
+    MlpSeg kinem, rest;
+    risk_observation(env, sv.obs, kinem, rest);
+    for (int offset = 0; offset < P; offset += env->n) {
+        const int B = std::min(env->n, P - offset);
+        for (size_t i = 0; i < env->la_allocs.size(); ++i)   // fresh records: reset and draw counters from 0
+            CU(cudaMemsetAsync(env->la_allocs[i], 0, env->la_bytes[i], stream));
+        const int* entry = env->d_pool_entry + offset;
+        ResetArgs RA{sv, B, nullptr, env->d_start_pool, P, env->d_target_pool, env->target_pool_n, k0, k1, entry};
+        reset_kernel<<<(B * 32 + 255) / 256, 256, 0, stream>>>(RA);
+        env->launches++;
+        if (env->human) {
+            HumanArgs H;
+            memset(&H, 0, sizeof(H));
+            H.buf = sv; H.n = B; H.env_base = offset; H.k0 = k0; H.k1 = k1;
+            H.start_pool = env->d_hstart_pool; H.start_pool_n = P; H.entry = entry;
+            H.pool_brake = env->d_hpool_brake; H.pool_bcount = env->d_hpool_bcount;
+            H.target_pool = env->d_htarget_pool; H.target_pool_n = env->htarget_pool_n;
+            human_reset_kernel<<<(B * 8 + 255) / 256, 256, 0, stream>>>(H, 0);
+            env->launches++;
+        }
+        CU(cudaGetLastError());
+        for (int i = 0; i < K; ++i) {
+            if ((rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0}, shadow_actions, nj, B, stream)))
+                return rc;
+            if ((rc = step_chain(env, sv, 0, B, 0, 0, 0, nullptr, nullptr, nullptr, SM_POOL_CHECK_STEP0, (uint32_t)i, false,
+                                 stream, nullptr, offset)))
+                return rc;
+            lookahead_latch_kernel<<<(B + 255) / 256, 256, 0, stream>>>(env->d_pool_verdict + offset, sv.done, sv.term_reason, B);
+            env->launches++;
+        }
+        CU(cudaGetLastError());
+    }
+    pool_partition_kernel<<<1, SM_PARTITION_THREADS, 0, stream>>>(env->d_pool_verdict, P, env->d_pool_dest, env->d_pool_dest + P);
+    env->launches++;
+    CU(cudaGetLastError());
+    if ((rc = pool_compact(env, env->d_start_pool, SM_POOL_STRIDE, stream))) return rc;
+    if (env->human) {   // entry e of the human's pools pairs with entry e of the robot's
+        if ((rc = pool_compact(env, env->d_hstart_pool, SM_HPOOL_STRIDE, stream))) return rc;
+        if ((rc = pool_compact(env, env->d_hpool_brake, SM_HBRAKE_STEPS * 8, stream))) return rc;
+        if ((rc = pool_compact(env, env->d_hpool_bcount, 1, stream))) return rc;
+    }
+    int passed = 0;
+    CU(cudaMemcpyAsync(&passed, env->d_pool_dest + P, sizeof(int), cudaMemcpyDeviceToHost, stream));
+    CU(cudaStreamSynchronize(stream));
+    env->init_checked = P;
+    if (passed == 0)
+        return fail(SM_ERR_STATE, "initial-backup-trajectory check: no entry of the start pool (" + std::to_string(P) +
+                                      " entries) keeps its backup trajectory of " + std::to_string(K) +
+                                      " steps free of collisions; resets draw from the whole pool");
+    env->start_draw_n = passed;
+    return SM_OK;
+}
+
+extern "C" int smenv_set_initial_backup_check(SmEnv* env, int backup_steps, SmStream s) {
+    if (!env) return fail(SM_ERR_ARG, "smenv_set_initial_backup_check: null env");
+    if (backup_steps < 0) return fail(SM_ERR_ARG, "smenv_set_initial_backup_check: backup_steps must be >= 0");
+    if (backup_steps == 0) {
+        env->init_check_steps = 0;
+        env->init_checked = 0;
+        env->start_draw_n = env->start_pool_n;
+        return SM_OK;
+    }
+    if (!env->net_loaded[SM_NET_BACKUP])
+        return fail(SM_ERR_STATE, "smenv_set_initial_backup_check: load the backup policy first (smenv_mlp_load)");
+    cudaStream_t stream = (cudaStream_t)s;
+    DevLock dev_lock_(env); int rc = activate(env, stream);
+    if (rc) return rc;
+    if ((rc = shadow_alloc(env, "smenv_set_initial_backup_check"))) return rc;
+    if (!env->d_pool_verdict) {
+        const size_t P = (size_t)env->start_pool_n;
+        const size_t widest = env->human ? SM_HBRAKE_STEPS * 8 : SM_POOL_STRIDE;
+        CU(cudaMalloc((void**)&env->d_pool_verdict, P * sizeof(float)));
+        CU(cudaMalloc((void**)&env->d_pool_entry, P * sizeof(int)));
+        CU(cudaMalloc((void**)&env->d_pool_dest, (P + 1) * sizeof(int)));
+        CU(cudaMalloc((void**)&env->d_pool_scratch, P * widest * sizeof(double)));
+        pool_entry_kernel<<<(unsigned)((P + 255) / 256), 256, 0, stream>>>(env->d_pool_entry, (int)P);
+        env->launches++;
+        CU(cudaGetLastError());
+    }
+    env->init_check_steps = backup_steps;
+    env->start_draw_n = env->start_pool_n;
+    env->init_checked = 0;
+    if (!env->pools_filled) return SM_OK;
+    return pool_check_launch(env, stream);
+}
+
+extern "C" int smenv_initial_backup_check_counts(SmEnv* env, int* checked, int* passed) {
+    if (!env) return fail(SM_ERR_ARG, "smenv_initial_backup_check_counts: null env");
+    if (checked) *checked = env->init_checked;
+    if (passed) *passed = env->start_draw_n;
     return SM_OK;
 }
 

@@ -49,6 +49,7 @@ struct HumanArgs {
     int* cwork;                // contact planning: [0] = count, [1..] = env * 8 + span
     const uint8_t* mask;       // reset: envs to reset (NULL = by done flag / all)
     unsigned long long* counters;
+    const int* entry;          // reset: [n] pool entry of env i (the pool check, smenv_set_initial_backup_check), NULL: drawn
 };
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -905,7 +906,8 @@ __global__ void __launch_bounds__(256) human_reset_kernel(HumanArgs A, int by_do
     if (active) active = by_done ? A.buf.done[env] != 0 : !(A.mask && !A.mask[env]);
     const int4 ep = *reinterpret_cast<const int4*>(A.buf.episode + 4 * env);
     const uint4 r = philox((uint32_t)(env + A.env_base), (uint32_t)(ep.y - 1), 0x5E7u, 1u, A.k0, A.k1);   // the robot's draw
-    const double* e = A.start_pool + (size_t)(r.x % (uint32_t)(A.start_pool_n > 0 ? A.start_pool_n : 1)) * SM_HPOOL_STRIDE;
+    const uint32_t pick = A.entry ? (uint32_t)A.entry[env] : r.x % (uint32_t)(A.start_pool_n > 0 ? A.start_pool_n : 1);
+    const double* e = A.start_pool + (size_t)pick * SM_HPOOL_STRIDE;
     {
         const unsigned gmask = 0xffu << (lane & 24);
         const uint4 r2 = philox((uint32_t)(env + A.env_base), (uint32_t)(ep.y - 1), 0x5E8u, 4u, A.k0, A.k1);
@@ -925,7 +927,7 @@ __global__ void __launch_bounds__(256) human_reset_kernel(HumanArgs A, int by_do
     __syncwarp();
     if (A.pool_brake) {   // the braking trajectory of a pool entry does not depend on the env: stored with the pool
         if (active) {
-            const size_t entry = (size_t)(r.x % (uint32_t)A.start_pool_n);
+            const size_t entry = pick;
             const int k = c_sc.hu.check_braking && c_sc.hu.initial_braking_trajectory ? A.pool_bcount[entry] : 0;
             const double* src = A.pool_brake + entry * SM_HBRAKE_STEPS * 8;
             double* hb = A.buf.hbrake + env * SM_HBRAKE_STEPS * 8;

@@ -346,6 +346,7 @@ struct ResetArgs {
     const double* target_pool;
     int target_pool_n;
     uint32_t k0, k1;
+    const int* entry;   // [n] pool entry of env i (the pool check, smenv_set_initial_backup_check), NULL: drawn
 };
 
 // injected first target points (parity protocol) or, with first_target == NULL, draws from the pool
@@ -387,7 +388,8 @@ __global__ void __launch_bounds__(256) reset_kernel(ResetArgs A) {
     if (A.mask && !A.mask[env]) return;
     int4 ep = *reinterpret_cast<const int4*>(A.buf.episode + 4 * (size_t)env);
     uint4 r = philox((uint32_t)env, (uint32_t)ep.y, 0x5E7u, 1u, A.k0, A.k1);
-    const double* e = A.start_pool + (size_t)(r.x % (uint32_t)A.start_pool_n) * SM_POOL_STRIDE;
+    const uint32_t pick = A.entry ? (uint32_t)A.entry[env] : r.x % (uint32_t)A.start_pool_n;
+    const double* e = A.start_pool + (size_t)pick * SM_POOL_STRIDE;
     A.buf.kin[(size_t)env * SM_KIN_STRIDE + lane] = e[lane];
     if (lane < SM_OBST_STRIDE) A.buf.obst[(size_t)env * SM_OBST_STRIDE + lane] = e[SM_KIN_STRIDE + lane];
     if (lane == 0) {
@@ -402,6 +404,51 @@ __global__ void __launch_bounds__(256) reset_kernel(ResetArgs A) {
     }
     write_observation(A.buf.obs + (size_t)env * c_sc.obs_size, e, e + SM_KIN_STRIDE, tp, lane, 32,
                       A.buf.hobs ? A.buf.hobs + (size_t)env * SM_HOBS_STRIDE : nullptr);
+}
+
+// ---------------- the initial-backup-trajectory check of the start pool (smenv_set_initial_backup_check)
+__global__ void pool_entry_kernel(int* entry, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) entry[i] = i;
+}
+
+// Stable partition of the pool by verdict: dest[e] is the new position of entry e, the passing entries (verdict 0) first
+// and the failing ones after them, each in their original order; *passed is the number of passing entries.  One CTA:
+// every thread counts a contiguous run of entries, a scan over the runs gives each run its first positions.
+#define SM_PARTITION_THREADS 1024
+__global__ void __launch_bounds__(SM_PARTITION_THREADS) pool_partition_kernel(const float* verdict, int n, int* dest,
+                                                                              int* passed) {
+    __shared__ int s_scan[SM_PARTITION_THREADS];
+    const int t = threadIdx.x;
+    const int per = (n + SM_PARTITION_THREADS - 1) / SM_PARTITION_THREADS;
+    const int e0 = min(n, t * per), e1 = min(n, e0 + per);
+    int cnt = 0;
+#pragma unroll 1
+    for (int e = e0; e < e1; ++e) cnt += verdict[e] == 0.0f;
+    s_scan[t] = cnt;
+    __syncthreads();
+#pragma unroll 1
+    for (int off = 1; off < SM_PARTITION_THREADS; off <<= 1) {   // inclusive scan of the run counts
+        const int v = t >= off ? s_scan[t - off] : 0;
+        __syncthreads();
+        s_scan[t] += v;
+        __syncthreads();
+    }
+    const int total = s_scan[SM_PARTITION_THREADS - 1];
+    int before = s_scan[t] - cnt;   // passing entries before entry e
+#pragma unroll 1
+    for (int e = e0; e < e1; ++e) dest[e] = verdict[e] == 0.0f ? before++ : total + (e - before);
+    if (t == 0) *passed = total;
+}
+
+// dst[dest[e]] = src[e] for the n records of `stride` elements of a pool array
+template <typename T>
+__global__ void pool_scatter_kernel(const T* __restrict__ src, T* __restrict__ dst, const int* __restrict__ dest, int n,
+                                    int stride) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * stride) return;
+    const size_t e = i / stride, k = i % stride;
+    dst[(size_t)dest[e] * stride + k] = src[i];
 }
 
 // observation only (after smenv_set_state)

@@ -218,6 +218,30 @@ class SafeMotionsVecEnv:
         loaded, switch the gate off first."""
         cabi.check(self._lib.smenv_set_risk_next_state(self._handle, int(bool(enable))), "smenv_set_risk_next_state")
 
+    def _initial_backup_steps(self):
+        return int(self.config.risk_state_initial_backup_trajectory_steps or
+                   self.config.risk_state_backup_trajectory_steps or 20)
+
+    def set_initial_backup_check(self, steps):
+        """risk_check_initial_backup_trajectory (observations.py:155-185) as a property of the start pool: every pool
+        entry is checked once, when the pool is filled -- the backup policy acts for `steps` steps from the entry (episode
+        clock at 0, no auto reset, gate off), and the entry fails if its episode ends in that window for a reason other
+        than the trajectory length (initial_backup_trajectory_unsafe's rule) -- and every reset, reset() and the device
+        auto reset of step() / step_random() / step_host() alike, draws from the passing entries only.  The current
+        pools are checked at once, and every later fill (set_seed) again.  0 or None switches the check off: resets draw
+        from the whole pool again (smenv_set_initial_backup_check).  Needs the backup policy (load_networks); raises if no
+        entry passes."""
+        cabi.check(self._lib.smenv_set_initial_backup_check(self._handle, int(steps or 0), self._stream()),
+                   "smenv_set_initial_backup_check")
+
+    def initial_backup_check_counts(self):
+        """(checked, passed): the start-pool entries the initial-backup-trajectory check rated for the current pools (0
+        while it is off), and the entries resets draw from (the passing ones; the whole pool while the check is off)."""
+        checked, passed = C.c_int(), C.c_int()
+        cabi.check(self._lib.smenv_initial_backup_check_counts(self._handle, C.byref(checked), C.byref(passed)),
+                   "smenv_initial_backup_check_counts")
+        return checked.value, passed.value
+
     def close(self):
         if self._handle:
             self._lib.smenv_destroy(self._handle)
@@ -302,8 +326,6 @@ class SafeMotionsVecEnv:
         cabi.check(self._lib.smenv_reset(self._handle, C.byref(self._buf), C.c_void_p(m.data_ptr()) if m is not None
                                          else None, self._stream()), "smenv_reset")
         self.episode_counter += self.num_envs if m is None else int(m.sum().item())
-        if self.config.risk_check_initial_backup_trajectory and self._networks:
-            self._recheck_initial_states(m)
         if self._squeeze:
             return self.obs[0].cpu().numpy()
         return self.obs
@@ -313,8 +335,7 @@ class SafeMotionsVecEnv:
         policy acts for `steps` steps (default: the episode length of the backup policy's training env, 20); an env is
         unsafe if its episode ends in that window for a reason other than the trajectory length.  The state is
         restored.  Returns a bool tensor [N]."""
-        steps = int(steps or self.config.risk_state_initial_backup_trajectory_steps or
-                    self.config.risk_state_backup_trajectory_steps or 20)
+        steps = int(steps or self._initial_backup_steps())
         snap = self.snapshot()
         auto, gate = self.auto_reset, self._gate_threshold
         self.auto_reset = False
@@ -330,18 +351,6 @@ class SafeMotionsVecEnv:
             self.auto_reset = auto
             self.set_risk_gate(gate)
         return unsafe
-
-    def _recheck_initial_states(self, mask, max_rounds=8):
-        """Re-resets the (masked) envs whose start state has no valid backup trajectory (observations.py:181-183)."""
-        for _ in range(max_rounds):
-            unsafe = self.initial_backup_trajectory_unsafe()
-            if mask is not None:
-                unsafe &= mask.bool()
-            if not bool(unsafe.any().item()):
-                return
-            um = unsafe.to(torch.uint8).contiguous()
-            cabi.check(self._lib.smenv_reset(self._handle, C.byref(self._buf), C.c_void_p(um.data_ptr()),
-                                             self._stream()), "smenv_reset")
 
     def set_state(self, q, v, a, obst=None, mask=None, first_target=None):
         """Injects start states (parity protocol, SURVEY 8c): q, v, a [N, n_joints] float64, obst [N, 16] or None;
@@ -370,24 +379,13 @@ class SafeMotionsVecEnv:
         else:
             arr = np.asarray(actions, dtype=np.float32).reshape(self.num_envs, -1)
             self.actions.copy_(torch.from_numpy(arr), non_blocking=False)
-        cabi.check(self._lib.smenv_step(self._handle, C.byref(self._buf), int(self._device_auto_reset()),
-                                        self._stream()), "smenv_step")
-
-    def _device_auto_reset(self):
-        # with risk_check_initial_backup_trajectory every new start state has to pass the backup-trajectory check, so
-        # finished envs are re-initialised by reset(mask) after the step instead of inside the finish kernel
-        return self.auto_reset and not (self.config.risk_check_initial_backup_trajectory and self._networks)
+        cabi.check(self._lib.smenv_step(self._handle, C.byref(self._buf), int(self.auto_reset), self._stream()),
+                   "smenv_step")
 
     def _after_step(self):
-        self._auto_reset_done = self.done if self._device_auto_reset() else None
-        if self.auto_reset and not self._device_auto_reset():
-            done = self.done.clone()
-            if bool(done.any().item()):
-                out = (self.reward.clone(), self.term_reason.clone(), self.info.clone())
-                self.reset(done)
-                self.done.copy_(done)
-                self.reward.copy_(out[0]); self.term_reason.copy_(out[1]); self.info.copy_(out[2])
-                self._auto_reset_done = done
+        # finished envs were re-initialised inside the step (with risk_check_initial_backup_trajectory from the checked
+        # start pool, set_initial_backup_check)
+        self._auto_reset_done = self.done if self.auto_reset else None
 
     def step(self, actions):
         """One env step for all envs.  actions: [N, n_joints] in [-1, 1] (torch on the env's device, or array-like).
@@ -401,8 +399,8 @@ class SafeMotionsVecEnv:
 
     def step_random(self):
         """Step with device-generated U(-1, 1) actions (``random_agent``, safe_motions_base.py:1047-1048)."""
-        cabi.check(self._lib.smenv_step_random(self._handle, C.byref(self._buf), int(self._device_auto_reset()),
-                                               self._stream()), "smenv_step_random")
+        cabi.check(self._lib.smenv_step_random(self._handle, C.byref(self._buf), int(self.auto_reset), self._stream()),
+                   "smenv_step_random")
         self._after_step()
         return self._outputs()
 
@@ -424,12 +422,12 @@ class SafeMotionsVecEnv:
         try:   # the gate runs inside the env ranges of the host step (same CUDA graph as the ungated step)
             cabi.check(self._lib.smenv_step_host(self._handle, C.byref(self._buf), self._h_actions.data_ptr(),
                                                  self._h_obs.data_ptr(), self._h_reward.data_ptr(),
-                                                 self._h_done.data_ptr(), int(self._device_auto_reset()), int(chunks),
+                                                 self._h_done.data_ptr(), int(self.auto_reset), int(chunks),
                                                  self._stream()), "smenv_step_host")
         finally:
             if gate_threshold is not None and gate_threshold != prev:
                 self.set_risk_gate(prev)
-        self._auto_reset_done = self.done if self._device_auto_reset() else None
+        self._auto_reset_done = self.done if self.auto_reset else None
         return self._h_obs.numpy(), self._h_reward.numpy(), self._h_done.numpy()
 
     def _outputs(self):
@@ -655,6 +653,8 @@ class SafeMotionsVecEnv:
         self._networks = True
         self._network_source = source
         self.risk_network_kind = kind
+        if self.config.risk_check_initial_backup_trajectory:
+            self.set_initial_backup_check(self._initial_backup_steps())
 
     def mlp_forward(self, which, in0, in1=None, n_out=1):
         """Parity hook: the loaded network `which` (0 risk, 1 backup policy) on caller-supplied rows."""

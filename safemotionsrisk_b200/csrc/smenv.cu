@@ -170,6 +170,10 @@ static void build_hwidth(const float4* v, int n, const float* c, float radius, s
     }
 }
 
+// What the risk gate rates a proposed action by: the risk network (state-action), the state risk network on the
+// simulated next state (smenv_set_risk_next_state), or a look-ahead of the backup policy (smenv_set_risk_lookahead).
+enum RiskCheck { RISK_NETWORK, RISK_NEXT_STATE, RISK_LOOKAHEAD };
+
 struct SmEnv {
     int n = 0, device = 0;
     uint64_t seed = 0;
@@ -219,8 +223,8 @@ struct SmEnv {
     int* d_gate_list = nullptr;    // [0..15] counters (two per env range), then [n] near-threshold rows, [n] risky rows
     int gate_exact = 1;            // re-rate near-threshold rows and compute the backup actions in float32 (smenv_set_gate_exact)
     float gate_band = 0.01f;       // |risk - threshold| below which the tensor-core risk is re-rated
-    int lookahead_steps = 0;       // > 0: the gate decides by a look-ahead of that many backup steps (smenv_set_risk_lookahead)
-    int next_state = 0;            // the gate rates the simulated next state with a state risk network (smenv_set_risk_next_state)
+    RiskCheck risk_check = RISK_NETWORK;
+    int lookahead_k = 0;           // backup steps of the look-ahead; 0 outside RISK_LOOKAHEAD
     SmBuffers la_buf = {};         // [n] shadow copy of every record the step writes, and a stats vector nobody reads
     std::vector<void*> la_allocs;
     std::vector<size_t> la_bytes;
@@ -1302,31 +1306,39 @@ extern "C" int smenv_observation(SmEnv* env, const SmBuffers* buf, SmStream s) {
     return SM_OK;
 }
 
-extern "C" int smenv_reset(SmEnv* env, const SmBuffers* buf, const uint8_t* mask, SmStream s) {
-    if (!env || !buf) return fail(SM_ERR_ARG, "smenv_reset: null argument");
-    if (!env->pools_filled) return fail(SM_ERR_STATE, "smenv_reset: call smenv_fill_pools first");
-    if (mask && !is_device_ptr(mask)) return fail(SM_ERR_ARG, "smenv_reset: mask must be a device pointer");
-    cudaStream_t stream = (cudaStream_t)s;
-    DevLock dev_lock_(env); int rc = activate(env, stream);
-    if (rc) return rc;
-    ResetArgs A{*buf, env->n, mask, env->d_start_pool, env->start_draw_n, env->d_target_pool, env->target_pool_n,
-                (uint32_t)env->seed, (uint32_t)(env->seed >> 32), nullptr};
-    reset_kernel<<<(env->n * 32 + 255) / 256, 256, 0, stream>>>(A);
+// Starts a new episode in the m envs of `bv` where mask is set (NULL: all): reset_kernel and, in the Human scene,
+// human_reset_kernel.  Env i starts from pool entry entry[i] (NULL: drawn from the first draw_n entries); env_base is the
+// Philox stream index of env 0 of the view for the human's draws.
+static int reset_launch(SmEnv* env, const SmBuffers& bv, int m, const uint8_t* mask, const int* entry, int env_base,
+                        int draw_n, cudaStream_t stream) {
+    const uint32_t k0 = (uint32_t)env->seed, k1 = (uint32_t)(env->seed >> 32);
+    ResetArgs A{bv, m, mask, env->d_start_pool, draw_n, env->d_target_pool, env->target_pool_n, k0, k1, entry};
+    reset_kernel<<<(m * 32 + 255) / 256, 256, 0, stream>>>(A);
     env->launches++;
     if (env->human) {
-        if (!buf->hkin || !buf->hstate || !buf->hbrake || !buf->hobs)
-            return fail(SM_ERR_ARG, "smenv_reset: the Human scene needs the hkin / hstate / hbrake / hobs buffers");
         HumanArgs H;
         memset(&H, 0, sizeof(H));
-        H.buf = *buf; H.n = env->n; H.env_base = 0; H.k0 = (uint32_t)env->seed; H.k1 = (uint32_t)(env->seed >> 32);
-        H.mask = mask; H.start_pool = env->d_hstart_pool; H.start_pool_n = env->start_draw_n;
+        H.buf = bv; H.n = m; H.env_base = env_base; H.k0 = k0; H.k1 = k1;
+        H.mask = mask; H.start_pool = env->d_hstart_pool; H.start_pool_n = draw_n; H.entry = entry;
         H.pool_brake = env->d_hpool_brake; H.pool_bcount = env->d_hpool_bcount;
         H.target_pool = env->d_htarget_pool; H.target_pool_n = env->htarget_pool_n;
-        human_reset_kernel<<<(env->n * 8 + 255) / 256, 256, 0, stream>>>(H, 0);
+        human_reset_kernel<<<(m * 8 + 255) / 256, 256, 0, stream>>>(H, 0);
         env->launches++;
     }
     CU(cudaGetLastError());
     return SM_OK;
+}
+
+extern "C" int smenv_reset(SmEnv* env, const SmBuffers* buf, const uint8_t* mask, SmStream s) {
+    if (!env || !buf) return fail(SM_ERR_ARG, "smenv_reset: null argument");
+    if (!env->pools_filled) return fail(SM_ERR_STATE, "smenv_reset: call smenv_fill_pools first");
+    if (mask && !is_device_ptr(mask)) return fail(SM_ERR_ARG, "smenv_reset: mask must be a device pointer");
+    if (env->human && (!buf->hkin || !buf->hstate || !buf->hbrake || !buf->hobs))
+        return fail(SM_ERR_ARG, "smenv_reset: the Human scene needs the hkin / hstate / hbrake / hobs buffers");
+    cudaStream_t stream = (cudaStream_t)s;
+    DevLock dev_lock_(env); int rc = activate(env, stream);
+    if (rc) return rc;
+    return reset_launch(env, *buf, env->n, mask, nullptr, 0, env->start_draw_n, stream);
 }
 
 extern "C" int smenv_set_human_actions_external(SmEnv* env, int external) {
@@ -1559,12 +1571,11 @@ static void launch_gjk(SmEnv* env, const GjkArgs& G, cudaStream_t stream) {
 // ranges back to back, the range's sub-list starting at entry k * e0 + chunk (its own count first).  Ranges in flight at
 // once need distinct slots.  exec: the actions to execute (NULL: bv.actions); risk / risky: the gate's outcome for the info
 // record (NULL: gate off).  The Philox step counter is step_counter + sub (step_ptr: read from device memory, plus sub).
-// stream_e0: the Philox stream index of env 0 of the view (-1: e0; the pool check runs its batches in the view of envs
+// stream_e0: the Philox stream index of env 0 of the view (e0, but the pool check runs its batches in the view of envs
 // [0, m) with the streams of their pool entries).
 static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, int auto_reset, int random_actions,
                       const float* exec, const float* risk, const uint8_t* risky, uint32_t step_counter, uint32_t sub,
-                      bool tk, cudaStream_t stream, const uint32_t* step_ptr, int stream_e0 = -1) {
-    if (stream_e0 < 0) stream_e0 = e0;
+                      bool tk, cudaStream_t stream, const uint32_t* step_ptr, int stream_e0) {
     const SmBuffers* buf = &bv;
     const int per_env_items = env->item_capacity / env->n;
     int* worklist = env->d_worklist + 2 * chunk;
@@ -1815,33 +1826,50 @@ static int shadow_copy(SmEnv* env, const SmBuffers& bv, int e0, int m, SmBuffers
     return SM_OK;
 }
 
+// One step of the shadow view `sv` (m envs from env e0, work lists of slot `chunk`): no auto reset, no random actions, no
+// gate, untimed; Philox step counter step_counter + sub (step_ptr: read from device memory, plus sub), stream index of env
+// 0 of the view `stream_e0`.
+static int shadow_step(SmEnv* env, const SmBuffers& sv, int e0, int m, int chunk, uint32_t step_counter, uint32_t sub,
+                       const uint32_t* step_ptr, int stream_e0, cudaStream_t stream) {
+    return step_chain(env, sv, e0, m, chunk, 0, 0, nullptr, nullptr, nullptr, step_counter, sub, false, stream, step_ptr,
+                      stream_e0);
+}
+
+// `steps` shadow steps of `sv` (shadow_step's arguments), the backup policy's action before each -- before the first only
+// when `proposed` is false: the proposed actions in sv.actions go first --; after each, `verdict` latches to 1 where the
+// step ended its episode for a reason other than the trajectory length.
+static int shadow_rollout(SmEnv* env, const SmBuffers& sv, int e0, int m, int chunk, int steps, bool proposed,
+                          uint32_t step_counter, const uint32_t* step_ptr, int stream_e0, float* verdict,
+                          cudaStream_t stream) {
+    MlpSeg kinem, rest;
+    risk_observation(env, sv.obs, kinem, rest);
+    int rc;
+    for (int i = 0; i < steps; ++i) {
+        if ((i > 0 || !proposed) && (rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0},
+                                                     const_cast<float*>(sv.actions), env->host_scene.n_joints, m, stream)))
+            return rc;
+        if ((rc = shadow_step(env, sv, e0, m, chunk, step_counter, (uint32_t)i, step_ptr, stream_e0, stream))) return rc;
+        lookahead_latch_kernel<<<(m + 255) / 256, 256, 0, stream>>>(verdict, sv.done, sv.term_reason, m);
+        env->launches++;
+    }
+    CU(cudaGetLastError());
+    return SM_OK;
+}
+
 // The gate's look-ahead (smenv_set_risk_lookahead) over the envs of `bv` (m envs from env e0): the range's records are
 // copied into the shadow buffers, whose episode clock restarts at 0 (switch_to_backup_client, safe_motions_base.py:
 // 1818-1822); K + 1 steps without auto reset run on the copy, the proposed action first, then the backup policy's; the risk
 // latches to 1 where one of them ends the episode for a reason other than the trajectory length; the gate decides on it.
 static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
                             cudaStream_t stream, const uint32_t* step_ptr) {
-    const int nj = env->host_scene.n_joints;
     SmBuffers sv;
     int rc;
     if ((rc = shadow_copy(env, bv, e0, m, sv, stream))) return rc;
-    float* shadow_actions = const_cast<float*>(sv.actions);
-    const size_t n = (size_t)m;
-    CU(cudaMemset2DAsync(sv.episode, 4 * sizeof(int32_t), 0, sizeof(int32_t), n, stream));   // episode_length = 0
+    CU(cudaMemset2DAsync(sv.episode, 4 * sizeof(int32_t), 0, sizeof(int32_t), (size_t)m, stream));   // episode_length = 0
     float* risk = env->d_risk + e0;
-    CU(cudaMemsetAsync(risk, 0, n * sizeof(float), stream));
-    MlpSeg kinem, rest;
-    risk_observation(env, sv.obs, kinem, rest);
-    for (int i = 0; i <= env->lookahead_steps; ++i) {
-        if (i > 0 && (rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0}, shadow_actions, nj, m, stream)))
-            return rc;
-        if ((rc = step_chain(env, sv, e0, m, chunk, 0, 0, nullptr, nullptr, nullptr, step_counter, (uint32_t)i, false, stream,
-                             step_ptr)))
-            return rc;
-        lookahead_latch_kernel<<<(m + 255) / 256, 256, 0, stream>>>(risk, sv.done, sv.term_reason, m);
-        env->launches++;
-    }
-    CU(cudaGetLastError());
+    CU(cudaMemsetAsync(risk, 0, (size_t)m * sizeof(float), stream));
+    if ((rc = shadow_rollout(env, sv, e0, m, chunk, env->lookahead_k + 1, true, step_counter, step_ptr, e0, risk, stream)))
+        return rc;
     if (env->gate_exact) CU(cudaMemsetAsync(env->d_gate_list + 2 * chunk, 0, 2 * sizeof(int), stream));
     // risk is 0 or 1: 0.5 separates them whatever the gate's threshold
     return gate_decide(env, bv, e0, m, chunk, 0.5f, risk, env->d_risky + e0, env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec,
@@ -1852,14 +1880,14 @@ static int lookahead_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int 
 // are copied into the shadow buffers with their episode clock as it is -- the simulated step is the real next step --; one
 // step without auto reset runs the proposed actions on the copy with the real step counter; the state risk network rates
 // the shadow's risk observation (float32 near the threshold in exact mode); the risk is set to 1 where the simulated step
-// ended its episode for a reason other than the trajectory length; the gate decides on it at its threshold.
+// ended its episode for a reason other than the trajectory length (after the rating, unlike shadow_rollout); the gate
+// decides on it at its threshold.
 static int next_state_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk, uint32_t step_counter, float* exec,
                              cudaStream_t stream, const uint32_t* step_ptr) {
     SmBuffers sv;
     int rc;
     if ((rc = shadow_copy(env, bv, e0, m, sv, stream))) return rc;
-    if ((rc = step_chain(env, sv, e0, m, chunk, 0, 0, nullptr, nullptr, nullptr, step_counter, 0, false, stream, step_ptr)))
-        return rc;
+    if ((rc = shadow_step(env, sv, e0, m, chunk, step_counter, 0, step_ptr, e0, stream))) return rc;
     float* risk = env->d_risk + e0;
     MlpSeg kinem, rest;
     risk_observation(env, sv.obs, kinem, rest);
@@ -1871,17 +1899,13 @@ static int next_state_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, int
                        env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
 }
 
-// The gate's mode against the loaded risk network: the network gate needs a state-action network, the next-state check a
-// state network; the look-ahead does not consult it.
-static int gate_mode_check(const SmEnv* env, const char* who) {
-    if (env->lookahead_steps > 0) return SM_OK;
-    if (env->next_state && !risk_net_is_state(env))
-        return fail(SM_ERR_STATE, std::string(who) + ": the next-state check needs a state risk network (input: the risk "
-                                                     "observation)");
-    if (!env->next_state && risk_net_is_state(env))
-        return fail(SM_ERR_STATE, std::string(who) + ": the loaded risk network is a state network (input: the risk "
-                                                     "observation); the network gate needs a state-action network");
-    return SM_OK;
+// Whether the gate may run in `mode` with the loaded risk network: the look-ahead does not consult it, the next-state
+// check needs a state network, the network gate a state-action network.
+static int gate_net_check(const SmEnv* env, RiskCheck mode, const char* who) {
+    if (mode == RISK_LOOKAHEAD || (mode == RISK_NEXT_STATE) == risk_net_is_state(env)) return SM_OK;
+    return fail(SM_ERR_STATE, std::string(who) + (mode == RISK_NEXT_STATE
+                                                      ? ": the next-state check needs a state risk network"
+                                                      : ": the network gate needs a state-action risk network"));
 }
 
 // One env step over the envs [e0, e0 + m) on `stream` with the work lists of slot `chunk` (step_chain): with the gate on
@@ -1895,7 +1919,7 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
     float* exec = nullptr;
     if (gate) {
         if (!buf->obs) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the observation buffer");
-        if (int rc = gate_mode_check(env, "smenv_step")) return rc;
+        if (int rc = gate_net_check(env, env->risk_check, "smenv_step")) return rc;
         if (random_actions) {
             if (!buf->actions) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the action buffer");
             random_actions_kernel<<<(m * env->host_scene.n_joints + 255) / 256, 256, 0, stream>>>(
@@ -1905,16 +1929,18 @@ static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chun
             random_actions = 0;
         }
         exec = env->d_exec + (size_t)e0 * env->host_scene.n_joints;
-        const int rc = env->lookahead_steps > 0
-                           ? lookahead_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr)
-                       : env->next_state
-                           ? next_state_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr)
-                           : gate_launch(env, buf_v, e0, m, chunk, env->gate_threshold, env->d_risk + e0, env->d_risky + e0,
-                                         env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
+        int rc;
+        switch (env->risk_check) {
+        case RISK_LOOKAHEAD: rc = lookahead_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr); break;
+        case RISK_NEXT_STATE: rc = next_state_launch(env, buf_v, e0, m, chunk, step_counter, exec, stream, step_ptr); break;
+        default:
+            rc = gate_launch(env, buf_v, e0, m, chunk, env->gate_threshold, env->d_risk + e0, env->d_risky + e0,
+                             env->d_backup + (size_t)e0 * MLP_MAX_OUT, exec, stream);
+        }
         if (rc) return rc;
     }
     return step_chain(env, buf_v, e0, m, chunk, auto_reset, random_actions, exec, gate ? env->d_risk + e0 : nullptr,
-                      gate ? env->d_risky + e0 : nullptr, step_counter, 0, tk, stream, step_ptr);
+                      gate ? env->d_risky + e0 : nullptr, step_counter, 0, tk, stream, step_ptr, e0);
 }
 
 // The count of the deferred-joint list is cleared by the finish kernel of the previous step; when the number of ranges
@@ -2010,7 +2036,7 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
 struct HostStepKey {
     SmBuffers buf;
     const void* h[4];
-    int auto_reset, chunks, count, pools, start_draw_n, human_external, gate_exact, lookahead, next_state;
+    int auto_reset, chunks, count, pools, start_draw_n, human_external, gate_exact, risk_check, lookahead_k;
     float gate, gate_band;
 };
 
@@ -2085,7 +2111,7 @@ extern "C" int smenv_step_host(SmEnv* env, const SmBuffers* buf, const float* h_
     key.h[0] = h_actions; key.h[1] = h_obs; key.h[2] = h_reward; key.h[3] = h_done;
     key.auto_reset = auto_reset; key.chunks = chunks; key.count = env->count ? 1 : 0; key.pools = env->pools_filled ? 1 : 0; key.gate = env->gate_threshold;
     key.human_external = env->human_external ? 1 : 0; key.gate_exact = env->gate_exact ? 1 : 0; key.gate_band = env->gate_band;
-    key.lookahead = env->lookahead_steps; key.next_state = env->next_state; key.start_draw_n = env->start_draw_n;
+    key.risk_check = env->risk_check; key.lookahead_k = env->lookahead_k; key.start_draw_n = env->start_draw_n;
     if (!env->host_graph || memcmp(&key, env->host_graph_key, sizeof(key)) != 0) {
         if (env->host_graph) { cudaGraphExecDestroy(env->host_graph); env->host_graph = nullptr; }
         const unsigned long long launches0 = env->launches;
@@ -2287,9 +2313,7 @@ extern "C" int smenv_risk_gate(SmEnv* env, const SmBuffers* buf, float threshold
                                SmStream s) {
     if (!env || !buf || !buf->actions || !buf->obs) return fail(SM_ERR_ARG, "smenv_risk_gate: null argument");
     if (!env->net_loaded[0] || !env->net_loaded[1]) return fail(SM_ERR_STATE, "smenv_risk_gate: load both networks first");
-    if (risk_net_is_state(env))
-        return fail(SM_ERR_STATE, "smenv_risk_gate: the loaded risk network is a state network; this call rates (state, "
-                                  "action) pairs");
+    if (int rc = gate_net_check(env, RISK_NETWORK, "smenv_risk_gate")) return rc;
     cudaStream_t stream = (cudaStream_t)s;
     DevLock dev_lock_(env); int rc = activate(env, stream);
     if (rc) return rc;
@@ -2301,10 +2325,8 @@ extern "C" int smenv_set_risk_gate(SmEnv* env, float threshold) {
     if (!env) return fail(SM_ERR_ARG, "smenv_set_risk_gate: null env");
     if (threshold >= 0.0f && (!env->net_loaded[0] || !env->net_loaded[1]))
         return fail(SM_ERR_STATE, "smenv_set_risk_gate: load the risk network and the backup policy first (smenv_mlp_load)");
-    if (threshold >= 0.0f) {
-        const int rc = gate_mode_check(env, "smenv_set_risk_gate");
-        if (rc) return rc;
-    }
+    if (threshold >= 0.0f)
+        if (int rc = gate_net_check(env, env->risk_check, "smenv_set_risk_gate")) return rc;
     env->gate_threshold = threshold >= 0.0f ? threshold : -1.0f;
     return SM_OK;
 }
@@ -2353,18 +2375,19 @@ static int shadow_alloc(SmEnv* env, const char* who) {
 extern "C" int smenv_set_risk_lookahead(SmEnv* env, int backup_steps) {
     if (!env) return fail(SM_ERR_ARG, "smenv_set_risk_lookahead: null env");
     if (backup_steps < 0) return fail(SM_ERR_ARG, "smenv_set_risk_lookahead: backup_steps must be >= 0");
-    if (backup_steps > 0 && !env->net_loaded[SM_NET_BACKUP])
-        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: load the backup policy first (smenv_mlp_load)");
-    if (backup_steps > 0 && env->next_state)
-        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: the next-state check is on (smenv_set_risk_next_state)");
     if (backup_steps > 0) {
-        const int rc = shadow_alloc(env, "smenv_set_risk_lookahead");
-        if (rc) return rc;
-    } else if (env->gate_threshold >= 0.0f && !env->next_state && risk_net_is_state(env)) {
-        return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: the gate is on with a state risk network; switch it off first "
-                                  "(smenv_set_risk_gate)");
+        if (!env->net_loaded[SM_NET_BACKUP])
+            return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: load the backup policy first (smenv_mlp_load)");
+        if (env->risk_check == RISK_NEXT_STATE)
+            return fail(SM_ERR_STATE, "smenv_set_risk_lookahead: the next-state check is on (smenv_set_risk_next_state)");
+        if (int rc = shadow_alloc(env, "smenv_set_risk_lookahead")) return rc;
+        env->risk_check = RISK_LOOKAHEAD;
+    } else if (env->risk_check != RISK_NEXT_STATE) {   // the gate is left in the network mode
+        if (env->gate_threshold >= 0.0f)
+            if (int rc = gate_net_check(env, RISK_NETWORK, "smenv_set_risk_lookahead")) return rc;
+        env->risk_check = RISK_NETWORK;
     }
-    env->lookahead_steps = backup_steps;
+    env->lookahead_k = backup_steps;
     return SM_OK;
 }
 
@@ -2373,18 +2396,16 @@ extern "C" int smenv_set_risk_next_state(SmEnv* env, int enable) {
     if (enable) {
         if (!env->net_loaded[SM_NET_BACKUP])
             return fail(SM_ERR_STATE, "smenv_set_risk_next_state: load the backup policy first (smenv_mlp_load)");
-        if (!risk_net_is_state(env))
-            return fail(SM_ERR_STATE, "smenv_set_risk_next_state: load a state risk network first (smenv_mlp_load, input: "
-                                      "the risk observation)");
-        if (env->lookahead_steps > 0)
+        if (int rc = gate_net_check(env, RISK_NEXT_STATE, "smenv_set_risk_next_state")) return rc;
+        if (env->risk_check == RISK_LOOKAHEAD)
             return fail(SM_ERR_STATE, "smenv_set_risk_next_state: the look-ahead is on (smenv_set_risk_lookahead)");
-        const int rc = shadow_alloc(env, "smenv_set_risk_next_state");
-        if (rc) return rc;
-    } else if (env->gate_threshold >= 0.0f && env->lookahead_steps == 0 && risk_net_is_state(env)) {
-        return fail(SM_ERR_STATE, "smenv_set_risk_next_state: the gate is on with a state risk network; switch it off first "
-                                  "(smenv_set_risk_gate)");
+        if (int rc = shadow_alloc(env, "smenv_set_risk_next_state")) return rc;
+        env->risk_check = RISK_NEXT_STATE;
+    } else if (env->risk_check != RISK_LOOKAHEAD) {   // the gate is left in the network mode
+        if (env->gate_threshold >= 0.0f)
+            if (int rc = gate_net_check(env, RISK_NETWORK, "smenv_set_risk_next_state")) return rc;
+        env->risk_check = RISK_NETWORK;
     }
-    env->next_state = enable != 0;
     return SM_OK;
 }
 
@@ -2414,44 +2435,18 @@ static int pool_compact(SmEnv* env, T* arr, int stride, cudaStream_t stream) {
 }
 
 static int pool_check_launch(SmEnv* env, cudaStream_t stream) {
-    const int P = env->start_pool_n, K = env->init_check_steps, nj = env->host_scene.n_joints;
-    const uint32_t k0 = (uint32_t)env->seed, k1 = (uint32_t)(env->seed >> 32);
+    const int P = env->start_pool_n, K = env->init_check_steps;
     int rc = set_list_layout(env, 1, stream);   // the batches use the work lists of slot 0 over up to n envs
     if (rc) return rc;
     CU(cudaMemsetAsync(env->d_pool_verdict, 0, (size_t)P * sizeof(float), stream));
-    const SmBuffers& sv = env->la_buf;
-    float* shadow_actions = const_cast<float*>(sv.actions);
-    MlpSeg kinem, rest;
-    risk_observation(env, sv.obs, kinem, rest);
     for (int offset = 0; offset < P; offset += env->n) {
         const int B = std::min(env->n, P - offset);
         for (size_t i = 0; i < env->la_allocs.size(); ++i)   // fresh records: reset and draw counters from 0
             CU(cudaMemsetAsync(env->la_allocs[i], 0, env->la_bytes[i], stream));
-        const int* entry = env->d_pool_entry + offset;
-        ResetArgs RA{sv, B, nullptr, env->d_start_pool, P, env->d_target_pool, env->target_pool_n, k0, k1, entry};
-        reset_kernel<<<(B * 32 + 255) / 256, 256, 0, stream>>>(RA);
-        env->launches++;
-        if (env->human) {
-            HumanArgs H;
-            memset(&H, 0, sizeof(H));
-            H.buf = sv; H.n = B; H.env_base = offset; H.k0 = k0; H.k1 = k1;
-            H.start_pool = env->d_hstart_pool; H.start_pool_n = P; H.entry = entry;
-            H.pool_brake = env->d_hpool_brake; H.pool_bcount = env->d_hpool_bcount;
-            H.target_pool = env->d_htarget_pool; H.target_pool_n = env->htarget_pool_n;
-            human_reset_kernel<<<(B * 8 + 255) / 256, 256, 0, stream>>>(H, 0);
-            env->launches++;
-        }
-        CU(cudaGetLastError());
-        for (int i = 0; i < K; ++i) {
-            if ((rc = mlp_launch(env, SM_NET_BACKUP, kinem, rest, MlpSeg{nullptr, 0, 0}, shadow_actions, nj, B, stream)))
-                return rc;
-            if ((rc = step_chain(env, sv, 0, B, 0, 0, 0, nullptr, nullptr, nullptr, SM_POOL_CHECK_STEP0, (uint32_t)i, false,
-                                 stream, nullptr, offset)))
-                return rc;
-            lookahead_latch_kernel<<<(B + 255) / 256, 256, 0, stream>>>(env->d_pool_verdict + offset, sv.done, sv.term_reason, B);
-            env->launches++;
-        }
-        CU(cudaGetLastError());
+        if ((rc = reset_launch(env, env->la_buf, B, nullptr, env->d_pool_entry + offset, offset, P, stream))) return rc;
+        if ((rc = shadow_rollout(env, env->la_buf, 0, B, 0, K, false, SM_POOL_CHECK_STEP0, nullptr, offset,
+                                 env->d_pool_verdict + offset, stream)))
+            return rc;
     }
     pool_partition_kernel<<<1, SM_PARTITION_THREADS, 0, stream>>>(env->d_pool_verdict, P, env->d_pool_dest, env->d_pool_dest + P);
     env->launches++;

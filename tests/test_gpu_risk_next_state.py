@@ -349,3 +349,98 @@ def test_refusals(state_nets):
     with pytest.raises(cabi.SmEnvError):
         la.set_risk_next_state(True)
     la.close()
+
+
+# The gate's mode against the loaded risk network (smenv.h): every row starts in the network mode with the gate off and
+# the network S (state) or SA (state-action, the shipped one) loaded, runs its setup, then the call under test.  Columns:
+# setup, call, refused, and whether a following step_random() runs.  Under risk_state_config 4 both kinds load.
+MODE_TABLE = [
+    # set_risk_gate(t >= 0): refused in the network mode with S and in the next-state mode without S
+    (["SA"], "gate", False, True),
+    (["S"], "gate", True, True),
+    (["S", "next_state", "SA"], "gate", True, True),
+    (["S", "next_state"], "gate", False, True),
+    (["S", "lookahead"], "gate", False, True),
+    (["SA", "lookahead"], "gate", False, True),
+    # set_risk_gate(None): never refused
+    (["SA", "gate", "S"], "gate_off", False, True),
+    (["S", "next_state", "gate", "SA"], "gate_off", False, True),
+    # set_risk_lookahead(K > 0): refused in the next-state mode
+    (["S", "next_state"], "lookahead", True, True),
+    (["S", "next_state", "gate"], "lookahead", True, True),
+    (["SA"], "lookahead", False, True),
+    (["SA", "gate", "S"], "lookahead", False, True),
+    (["S", "lookahead", "gate"], "lookahead", False, True),
+    # set_risk_lookahead(0): refused when it leaves the gate on in the network mode with S
+    (["S", "lookahead", "gate"], "lookahead_off", True, True),
+    (["SA", "lookahead", "gate", "S"], "lookahead_off", True, True),
+    (["SA", "gate", "S"], "lookahead_off", True, False),
+    (["SA", "lookahead", "gate"], "lookahead_off", False, True),
+    (["S", "lookahead"], "lookahead_off", False, True),
+    (["S", "next_state", "gate"], "lookahead_off", False, True),
+    (["S", "next_state", "gate", "SA"], "lookahead_off", False, False),
+    # set_risk_next_state(1): refused without S and in the look-ahead mode
+    (["SA"], "next_state", True, True),
+    (["S", "lookahead"], "next_state", True, True),
+    (["S", "lookahead", "gate"], "next_state", True, True),
+    (["S"], "next_state", False, True),
+    (["SA", "gate", "S"], "next_state", False, True),
+    # set_risk_next_state(0): refused when it leaves the gate on in the network mode with S
+    (["S", "next_state", "gate"], "next_state_off", True, True),
+    (["SA", "gate", "S"], "next_state_off", True, False),
+    (["S", "next_state", "gate", "SA"], "next_state_off", False, True),
+    (["S", "lookahead", "gate"], "next_state_off", False, True),
+    (["S", "next_state"], "next_state_off", False, True),
+    # risk_gate: refused with S, whatever the mode
+    (["S"], "risk_gate", True, True),
+    (["S", "next_state"], "risk_gate", True, True),
+    (["SA"], "risk_gate", False, True),
+    (["SA", "lookahead"], "risk_gate", False, True),
+    # the step with the gate on: refused in the network mode with S and in the next-state mode without S
+    (["SA", "gate", "S"], None, False, False),
+    (["S", "next_state", "gate", "SA"], None, False, False),
+    (["SA", "lookahead", "gate", "S"], None, False, True),
+]
+
+
+def test_mode_and_network_table(state_nets):
+    from safemotionsrisk_b200.vec_env import SafeMotionsVecEnv
+    shipped = os.path.join(os.path.dirname(os.path.abspath(abi.__file__)), "assets", "networks_space.npz")
+    nets = {"S": state_nets["space_bm"], "SA": shipped}
+    env = SafeMotionsVecEnv(num_envs=64, config=space_backup_config(ball_machine_mode=True, risk_config_dir=nets["S"],
+                                                                    risk_threshold=0.5, risk_state_config=4), seed=1)
+    env.reset()
+    calls = {"gate": lambda: env.set_risk_gate(0.5), "gate_off": lambda: env.set_risk_gate(None),
+             "lookahead": lambda: env.set_risk_lookahead(5), "lookahead_off": lambda: env.set_risk_lookahead(0),
+             "next_state": lambda: env.set_risk_next_state(True), "next_state_off": lambda: env.set_risk_next_state(False),
+             "S": lambda: env.load_networks(nets["S"]), "SA": lambda: env.load_networks(nets["SA"]),
+             "risk_gate": lambda: env.risk_gate(0.5)}
+
+    def refuses(fn):
+        try:
+            fn()
+        except cabi.SmEnvError:
+            return True
+        torch.cuda.synchronize()
+        return False
+
+    for setup, call, refused, steps in MODE_TABLE:
+        row = "{} then {}".format(setup, call)
+        env.set_risk_gate(None)            # with the gate off, both off-switches are accepted in every mode
+        env.set_risk_next_state(False)
+        env.set_risk_lookahead(0)
+        for op in setup:
+            calls[op]()
+        if call is not None:
+            assert refuses(calls[call]) == refused, row
+        assert refuses(env.step_random) != steps, row
+    env.close()
+    # without the networks the gate and both modes are refused
+    bare = SafeMotionsVecEnv(num_envs=64, config=space_backup_config(ball_machine_mode=True), seed=1)
+    for call in (lambda: bare.set_risk_gate(0.5), lambda: bare.set_risk_lookahead(5),
+                 lambda: bare.set_risk_next_state(True)):
+        assert refuses(call)
+    for call in (lambda: bare.set_risk_gate(None), lambda: bare.set_risk_lookahead(0),
+                 lambda: bare.set_risk_next_state(False)):
+        assert not refuses(call)
+    bare.close()

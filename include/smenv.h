@@ -441,9 +441,12 @@ int smenv_kernel_times(SmEnv* env, double* ms_out /* SM_K_COUNT */, int* steps_o
 enum SmNet { SM_NET_RISK = 0, SM_NET_BACKUP = 1, SM_NET_HUMAN = 2, SM_NET_COUNT = 3 };
 int smenv_mlp_load(SmEnv* env, int which, int n_tc, const int32_t* dims, int hidden_act, int out_act,
                    const float* weights);
-/* out[n][out_stride] = net([in0 row, in1 row]) for n rows; all device pointers (in1 may be NULL with in1_w = 0). */
+/* out[n][out_stride] = net([in0 row, in1 row]) for n rows; all device pointers (in1 may be NULL with in1_w = 0).  Every
+ * output of the network is written: SM_ERR_ARG if out_stride is smaller than its output count. */
 int smenv_mlp_forward(SmEnv* env, int which, const float* in0, int in0_w, const float* in1, int in1_w, float* out,
                       int out_stride, int n, SmStream stream);
+/* Input and output widths of the loaded network `which` (either pointer may be NULL); SM_ERR_STATE if none is loaded. */
+int smenv_mlp_shape(SmEnv* env, int which, int* n_in, int* n_out);
 /* Risk gate on buf->actions in place: risk(obs, action) >= threshold replaces the env's action by the backup policy's
  * (obs = buf->obs, the observation the action was computed from).  risk_out [N] / risky_out [N] may be NULL.
  * SM_ERR_STATE if the loaded risk network is a state network (see smenv_set_risk_next_state). */
@@ -510,7 +513,9 @@ int smenv_initial_backup_check_counts(SmEnv* env, int* checked, int* passed);
  * (safe_motions_base.py:1597-1603, actions.py:328-333).  exact = 0: both networks on the tensor cores only.
  * band <= 0 keeps the current band (default 0.01; the fp16 error around the reference's thresholds is < 4e-3). */
 int smenv_set_gate_exact(SmEnv* env, int exact, float band);
-/* The loaded network `which` in float32 on the CUDA cores for n rows (parity hook of the exact gate). */
+/* The loaded network `which` in float32 on the CUDA cores for n rows (parity hook of the exact gate): the first n_out
+ * outputs of every row.  SM_ERR_STATE if the network is not loaded; SM_ERR_ARG if n_out exceeds its output count or
+ * out_stride < n_out. */
 int smenv_mlp_forward_exact(SmEnv* env, int which, const float* in0, int in0_w, const float* in1, int in1_w, float* out,
                             int out_stride, int n_out, int n, SmStream stream);
 /* Writes the U(-1,1) actions smenv_step_random would use for the next step into buf->actions (so that the gate can be

@@ -45,3 +45,53 @@ def gate(w, obs, action, threshold, n_joints=7):
     out = action.copy()
     out[risky] = backup_forward(w, obs[risky], n_joints)
     return out, risk, risky
+
+
+# ---------------------------------------------------------------------------------------------- float64 references
+# Generic networks: `layers` is a list of (kernel [in][out], bias [out]) pairs, the hidden layers followed by the output
+# layer; hidden is "selu" or "swish", out is "sigmoid" or "tanh".
+
+def shipped_layers(w, net):
+    """Layer list of a shipped network: net = "risk", "backup" or "human"."""
+    names = ["dense_{}".format(i) for i in range(4)] if net == "risk" else ["fc_1", "fc_2", "fc_out"]
+    return [(w["{}/{}/kernel".format(net, n)], w["{}/{}/bias".format(net, n)]) for n in names]
+
+
+def _act64(x, kind):
+    if kind == "selu":
+        return 1.0507009873554805 * np.where(x > 0, x, 1.6732632423543772 * np.expm1(np.minimum(x, 0)))
+    if kind == "swish":
+        return x / (1 + np.exp(-x))
+    if kind == "sigmoid":
+        return 1 / (1 + np.exp(-x))
+    if kind == "tanh":
+        return np.tanh(x)
+    raise ValueError(kind)
+
+
+def _f16(x):
+    return np.asarray(x, dtype=np.float64).astype(np.float16).astype(np.float64)
+
+
+def forward64(layers, x, hidden="selu", out="sigmoid"):
+    """Plain float64 forward pass (the float32 parameters widened exactly)."""
+    h = np.asarray(x, dtype=np.float64)
+    for k, b in layers[:-1]:
+        h = _act64(h @ np.asarray(k, np.float64) + np.asarray(b, np.float64), hidden)
+    k, b = layers[-1]
+    return _act64(h @ np.asarray(k, np.float64) + np.asarray(b, np.float64), out)
+
+
+def forward_tc(layers, x, hidden="selu", out="sigmoid"):
+    """float64 forward pass that rounds where mlp_kernel (smenv_mlp.cuh) rounds, and nowhere else: the inputs and the
+    kernels of the hidden (tensor-core) layers to fp16 (round to nearest even); products summed in float64, the float32
+    bias added and the activation applied in float64; a hidden activation that feeds another tensor-core layer to fp16.
+    The last hidden activation stays unrounded: the kernel keeps it in fp32 registers and contracts it with the float32
+    output kernel on the CUDA cores."""
+    h = _f16(x)
+    for i, (k, b) in enumerate(layers[:-1]):
+        h = _act64(h @ _f16(k) + np.asarray(b, np.float64), hidden)
+        if i < len(layers) - 2:
+            h = _f16(h)
+    k, b = layers[-1]
+    return _act64(h @ np.asarray(k, np.float64) + np.asarray(b, np.float64), out)

@@ -211,5 +211,5 @@ EXPORTED_SYMBOLS = [
     "smenv_set_seed", "smenv_set_risk_gate", "smenv_set_human_actions_external", "smenv_set_human_state",
     "smenv_human_pool_sizes", "smenv_copy_human_pools", "smenv_measure_fma_peaks", "smenv_launch_config", "smenv_set_gate_exact", "smenv_mlp_forward_exact",
     "smenv_set_risk_lookahead", "smenv_set_risk_next_state", "smenv_set_initial_backup_check",
-    "smenv_initial_backup_check_counts",
+    "smenv_initial_backup_check_counts", "smenv_mlp_shape",
 ]

@@ -52,6 +52,7 @@ def load():
     lib.smenv_launch_config.argtypes = [vp, C.POINTER(i32)]
     lib.smenv_set_gate_exact.argtypes = [vp, i32, C.c_float]
     lib.smenv_mlp_forward_exact.argtypes = [vp, i32, vp, i32, vp, i32, vp, i32, i32, i32, vp]
+    lib.smenv_mlp_shape.argtypes = [vp, i32, C.POINTER(i32), C.POINTER(i32)]
     lib.smenv_set_seed.argtypes = [vp, u64]
     lib.smenv_debug_build_lut.argtypes = [vp, i32, i32, vp, i32]
     lib.smenv_debug_lut_cell.argtypes = [C.c_float, C.c_float, C.c_float, i32]

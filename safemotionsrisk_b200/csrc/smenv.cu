@@ -1438,6 +1438,8 @@ static int mlp_launch(SmEnv* env, int which, MlpSeg s0, MlpSeg s1, MlpSeg s2, fl
     if (!env->net_loaded[which]) return fail(SM_ERR_STATE, "network not loaded (smenv_mlp_load)");
     const MlpNet& net = env->nets[which];
     if (s0.w + s1.w + s2.w != net.n_in) return fail(SM_ERR_ARG, "network input width does not match the loaded weights");
+    // the kernel writes all net.n_out outputs of a row: a narrower row would overrun the caller's buffer
+    if (out_stride < net.n_out) return fail(SM_ERR_ARG, "output row stride is smaller than the loaded network's output count");
     MlpArgs M;
     M.net = net; M.n = n; M.out = out; M.out_stride = out_stride;
     const MlpSeg segs[3] = {s0, s1, s2};
@@ -1456,6 +1458,9 @@ static int mlp_launch(SmEnv* env, int which, MlpSeg s0, MlpSeg s1, MlpSeg s2, fl
 static int mlp_exact_launch(SmEnv* env, int which, MlpSeg s0, MlpSeg s1, MlpSeg s2, const int* rows, const int* n_rows,
                             int max_rows, float* out, int out_stride, int n_write, cudaStream_t stream) {
     if (!env->net_loaded[which]) return fail(SM_ERR_STATE, "network not loaded (smenv_mlp_load)");
+    // outputs past net.n_out would read w_out columns past out_pad (and past the allocation at its last row)
+    if (n_write < 1 || n_write > env->nets[which].n_out) return fail(SM_ERR_ARG, "more outputs requested than the loaded network has");
+    if (out_stride < n_write) return fail(SM_ERR_ARG, "output row stride is smaller than the number of outputs written");
     MlpExactArgs X;
     memset(&X, 0, sizeof(X));
     X.net = env->nets[which]; X.rows = rows; X.n_rows = n_rows; X.n_rows_host = max_rows;
@@ -2523,9 +2528,18 @@ extern "C" int smenv_mlp_forward_exact(SmEnv* env, int which, const float* in0, 
     cudaStream_t stream = (cudaStream_t)s;
     DevLock dev_lock_(env); int rc = activate(env, stream);
     if (rc) return rc;
+    if (!env->net_loaded[which]) return fail(SM_ERR_STATE, "network not loaded (smenv_mlp_load)");
     if (in0_w + (in1 ? in1_w : 0) != env->nets[which].n_in) return fail(SM_ERR_ARG, "network input width does not match the loaded weights");
     return mlp_exact_launch(env, which, MlpSeg{in0, in0_w, in0_w}, MlpSeg{in1, in1 ? in1_w : 0, in1 ? in1_w : 0},
                             MlpSeg{nullptr, 0, 0}, nullptr, nullptr, n, out, out_stride, n_out, stream);
+}
+
+extern "C" int smenv_mlp_shape(SmEnv* env, int which, int* n_in, int* n_out) {
+    if (!env || which < 0 || which >= SM_NET_COUNT) return fail(SM_ERR_ARG, "smenv_mlp_shape: bad argument");
+    if (!env->net_loaded[which]) return fail(SM_ERR_STATE, "network not loaded (smenv_mlp_load)");
+    if (n_in) *n_in = env->nets[which].n_in;
+    if (n_out) *n_out = env->nets[which].n_out;
+    return SM_OK;
 }
 
 extern "C" int smenv_set_seed(SmEnv* env, uint64_t seed) {

@@ -656,8 +656,21 @@ class SafeMotionsVecEnv:
         if self.config.risk_check_initial_backup_trajectory:
             self.set_initial_backup_check(self._initial_backup_steps())
 
+    def mlp_shape(self, which):
+        """(input width, output count) of the loaded network `which` (smenv_mlp_shape)."""
+        n_in, n_out = C.c_int(), C.c_int()
+        cabi.check(self._lib.smenv_mlp_shape(self._handle, which, C.byref(n_in), C.byref(n_out)), "smenv_mlp_shape")
+        return n_in.value, n_out.value
+
+    def _check_n_out(self, which, n_out):
+        have = self.mlp_shape(which)[1]
+        if n_out != have:
+            raise ValueError("network {} has {} outputs, n_out={} was asked for".format(which, have, n_out))
+
     def mlp_forward(self, which, in0, in1=None, n_out=1):
-        """Parity hook: the loaded network `which` (0 risk, 1 backup policy) on caller-supplied rows."""
+        """Parity hook: the loaded network `which` (0 risk, 1 backup policy) on caller-supplied rows; n_out must be the
+        network's output count."""
+        self._check_n_out(which, n_out)
         in0 = torch.as_tensor(in0, dtype=torch.float32, device=self.device).contiguous()
         n = in0.shape[0]
         out = torch.zeros((n, n_out), dtype=torch.float32, device=self.device)
@@ -675,7 +688,9 @@ class SafeMotionsVecEnv:
         cabi.check(self._lib.smenv_set_gate_exact(self._handle, int(bool(exact)), float(band)), "smenv_set_gate_exact")
 
     def mlp_forward_exact(self, which, in0, in1=None, n_out=1):
-        """Parity hook: the loaded network `which` in float32 on the CUDA cores (the exact path of the gate)."""
+        """Parity hook: the loaded network `which` in float32 on the CUDA cores (the exact path of the gate); n_out must
+        be the network's output count."""
+        self._check_n_out(which, n_out)
         in0 = torch.as_tensor(in0, dtype=torch.float32, device=self.device).contiguous()
         n = in0.shape[0]
         out = torch.zeros((n, n_out), dtype=torch.float32, device=self.device)

@@ -338,7 +338,9 @@ typedef struct SmCounters {
     unsigned long long heavy_solves;   /* position bounds that needed the iterative solve */
     unsigned long long aux[6];         /* GJK pairs by iteration count: <= 4, <= 8, <= 12, <= 16, <= 24, more */
     unsigned long long brake_poses;        /* Human: poses the braking-trajectory check visited */
-    unsigned long long brake_pair_bounds;  /* Human: sphere bounds of convex pairs evaluated for those poses */
+    unsigned long long brake_pair_bounds;  /* Human: sphere bounds of convex pairs evaluated by the per-pose pass */
+    unsigned long long brake_spans;        /* Human: spans of consecutive poses the inflated span pass tested */
+    unsigned long long brake_fine_poses;   /* Human: poses of the spans it could not clear, passed to the per-pose pass */
 } SmCounters;
 
 /* Kernels of one step, in launch order (smenv_kernel_times). */
@@ -539,7 +541,9 @@ int smenv_debug_lut_cell(float dx, float dy, float dz, int res);
  * [gp_b0, gp_b0 + gp_nb) on frame gp_fb (human frame index; -1 = world, i.e. the table).  Side A is covered by the capsule
  * of its arm frame (hf_*, arm frames 3, 4, 7, 8 in this order); side B by gp_sb / gp_srb (trunk, frame 0), by the box
  * gp_bmin / gp_bmax (table, world frame) or by its arm frame's capsule.  Against the table the kernel replaces an arm
- * capsule by two spheres of radius hf_cover_rad at 1/4 and 3/4 of its segment. */
+ * capsule by two spheres of radius hf_cover_rad at 1/4 and 3/4 of its segment.  hf_rho[i][j]: a change of joint j by dq
+ * moves every shape centre and both capsule end points of arm frame i by at most |dq| * hf_rho[i][j] (0 for the joints
+ * that do not move the frame); the span pass inflates its volumes by these. */
 typedef struct SmHumanBounds {
     int32_t n_gp;
     int32_t gp_fa[8], gp_fb[8], gp_a0[8], gp_na[8], gp_b0[8], gp_nb[8];
@@ -548,6 +552,7 @@ typedef struct SmHumanBounds {
     float gp_sa[8][6], gp_sra[8], gp_sb[8][6], gp_srb[8]; /* capsules of both sides: segment end points, radius */
     int32_t hf_s0[4], hf_sn[4];                           /* shape range of arm frame i */
     float hf_seg[4][6], hf_rad[4], hf_cover_rad[4];
+    float hf_rho[4][8];
 } SmHumanBounds;
 
 /* Host-only (no GPU needed): the bounding volumes above for a scene with the human enabled, built by the same code as

@@ -67,7 +67,7 @@ class SmHumanBounds(C.Structure):
         ("gp_bmin", (f * 3) * 8), ("gp_bmax", (f * 3) * 8),
         ("gp_sa", (f * 6) * 8), ("gp_sra", f * 8), ("gp_sb", (f * 6) * 8), ("gp_srb", f * 8),
         ("hf_s0", i32 * 4), ("hf_sn", i32 * 4),
-        ("hf_seg", (f * 6) * 4), ("hf_rad", f * 4), ("hf_cover_rad", f * 4)]
+        ("hf_seg", (f * 6) * 4), ("hf_rad", f * 4), ("hf_cover_rad", f * 4), ("hf_rho", (f * 8) * 4)]
     del f
 
 
@@ -198,7 +198,8 @@ class SmCounters(C.Structure):
     _fields_ = [("gjk_calls", C.c_ulonglong), ("gjk_iters", C.c_ulonglong), ("support_dots", C.c_ulonglong),
                 ("distance_items", C.c_ulonglong), ("env_steps", C.c_ulonglong), ("contact_envs", C.c_ulonglong),
                 ("contact_items", C.c_ulonglong), ("reserved", C.c_ulonglong), ("heavy_joints", C.c_ulonglong), ("heavy_solves", C.c_ulonglong), ("aux", C.c_ulonglong * 6),
-                ("brake_poses", C.c_ulonglong), ("brake_pair_bounds", C.c_ulonglong)]
+                ("brake_poses", C.c_ulonglong), ("brake_pair_bounds", C.c_ulonglong), ("brake_spans", C.c_ulonglong),
+                ("brake_fine_poses", C.c_ulonglong)]
 
 
 # every extern "C" symbol include/smenv.h declares

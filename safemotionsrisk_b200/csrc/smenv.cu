@@ -237,7 +237,8 @@ struct SmEnv {
     double* d_hbacc = nullptr;     // [n][SM_HBRAKE_STEPS][8]
     float* d_hposes = nullptr;     // [n][SM_HBRAKE_POSES][8]
     int* d_hbinfo = nullptr;       // [n][4]
-    int* d_hunits = nullptr;       // [0] = count, [1..] = (env << 7 | pose) units of the braking-trajectory pose checks
+    int* d_hunits = nullptr;       // [0] = count, [1..] = spans of poses of the braking-trajectory check (hbp_unit)
+    int* d_hfine = nullptr;        // [0] = count, [1..] = the poses of the spans the span pass could not clear
     float* d_hscratch = nullptr;   // [n][SM_SCRATCH_FLOATS]
     float* d_hpolicy = nullptr;    // [n][16]
     double* d_hstart_pool = nullptr;   // [start_pool_n][SM_HPOOL_STRIDE]
@@ -246,7 +247,8 @@ struct SmEnv {
     double* d_htarget_pool = nullptr;  // [2][htarget_pool_n][4]
     int htarget_pool_n = 0;
     size_t smem_bytes_hplan = 0;
-    int grid_hplan = 0;              // resident CTAs of human_brake_plan_kernel on the device
+    int grid_hplan = 0;              // resident CTAs of human_brake_plan_kernel<false> (per-pose pass) on the device
+    int grid_hplan_span = 0;         // the same for human_brake_plan_kernel<true> (span pass)
     bool time_kernels = false;   // measurement mode (smenv_kernel_timing)
     cudaEvent_t ev[SM_K_COUNT + 1] = {};
     double kernel_ms[SM_K_COUNT] = {};
@@ -442,6 +444,30 @@ static int human_brake_bounds(const SmScene* sc, DevHuman& u, std::vector<short>
         for (int k = 0; k < 6; ++k) u.hf_seg[fi][k] = 0.f;
         u.hf_rad[fi] = 0.f;
         if (!ids.empty()) capsule(ids, u.hf_seg[fi], &u.hf_rad[fi]);
+        // span pass: a change of joint j by dq moves every point it reads in this frame (shape centres, capsule end
+        // points) by at most dq * (largest distance of such a point in the frame + the link offsets from j + 1 to the frame)
+        float cn = 0.f;
+        for (int id : ids)
+            cn = fmaxf(cn, sqrtf((float)(sc->shapes[id].center[0] * sc->shapes[id].center[0] +
+                                         sc->shapes[id].center[1] * sc->shapes[id].center[1] +
+                                         sc->shapes[id].center[2] * sc->shapes[id].center[2])));
+        for (int e = 0; e < 2; ++e) {
+            const float* p = u.hf_seg[fi] + 3 * e;
+            cn = fmaxf(cn, sqrtf(p[0] * p[0] + p[1] * p[1] + p[2] * p[2]));
+        }
+        const int jf = arm_frames[fi] - 101;   // the joint that moves the frame
+        for (int j = 0; j < SM_HUMAN_JOINTS; ++j) {
+            float rho = 0.f;
+            if ((j >> 2) == (jf >> 2) && j <= jf) {
+                rho = cn;
+                for (int i = j + 1; i <= jf; ++i) {
+                    const float t0 = (float)h.joint_t[i][0], t1 = (float)h.joint_t[i][1], t2 = (float)h.joint_t[i][2];
+                    rho += sqrtf(t0 * t0 + t1 * t1 + t2 * t2);
+                }
+                rho *= 1.0f + 1e-5f;
+            }
+            u.hf_rho[fi][j] = rho;
+        }
     }
     for (int g = 0; g < ngp; ++g) {
         const int fa = u.gp_fa[g], fb = u.gp_fb[g];
@@ -740,6 +766,7 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
         if (sc->n_obstacles != 1 || sc->obst_kind[0] != SM_OBST_HUMAN) return fail(SM_ERR_SCENE, "a human scene has the human as its only moving obstacle");
         if (h.brake_checks < 1 || h.brake_checks > 7) return fail(SM_ERR_SCENE, "human brake_checks must be in 1..7");
         if (h.brake_checks * 22 > SM_HBRAKE_POSES) return fail(SM_ERR_SCENE, "too many collision checks per step for the pose buffer");
+        if (num_envs > HBP_MAX_ENVS) return fail(SM_ERR_ARG, "the Human scene supports at most 4194304 envs (unit word of the braking check)");
         for (int j = 0; j < 8; ++j)
             if (h.joint_parent[j] != ((j & 3) == 0 ? 0 : j)) return fail(SM_ERR_SCENE, "the human is expected as two serial arms of four joints");
         env->human = true;
@@ -875,6 +902,8 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
         CU(cudaMemset(env->d_hbinfo, 0, N * 4 * sizeof(int)));
         CU(cudaMalloc((void**)&env->d_hunits, (N * SM_HBRAKE_POSES + 16) * sizeof(int)));
         CU(cudaMemset(env->d_hunits, 0, (N * SM_HBRAKE_POSES + 16) * sizeof(int)));
+        CU(cudaMalloc((void**)&env->d_hfine, (N * SM_HBRAKE_POSES + 16) * sizeof(int)));
+        CU(cudaMemset(env->d_hfine, 0, (N * SM_HBRAKE_POSES + 16) * sizeof(int)));
         CU(cudaMalloc((void**)&env->d_hscratch, N * SM_SCRATCH_FLOATS * sizeof(float)));
         CU(cudaMemset(env->d_hscratch, 0, N * SM_SCRATCH_FLOATS * sizeof(float)));
         CU(cudaMalloc((void**)&env->d_hpolicy, N * 16 * sizeof(float)));
@@ -1063,13 +1092,16 @@ extern "C" int smenv_create(const SmScene* sc, int num_envs, int device, uint64_
         static size_t g_smem_hplan[SM_MAX_DEVICES] = {};   // under the create lock; only ever raised, like the limits above
         size_t& lim = g_smem_hplan[device % SM_MAX_DEVICES];
         if (env->smem_bytes_hplan > lim) {
-            CU(cudaFuncSetAttribute(human_brake_plan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->smem_bytes_hplan));
+            CU(cudaFuncSetAttribute(human_brake_plan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->smem_bytes_hplan));
+            CU(cudaFuncSetAttribute(human_brake_plan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)env->smem_bytes_hplan));
             lim = env->smem_bytes_hplan;
         }
-        int per = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, human_brake_plan_kernel, HBP_THREADS, env->smem_bytes_hplan));
-        if (per < 1) { return fail(SM_ERR_CUDA, "the human's braking-check planning kernel does not fit on an SM"); }
+        int per = 0, per_span = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, human_brake_plan_kernel<false>, HBP_THREADS, env->smem_bytes_hplan));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_span, human_brake_plan_kernel<true>, HBP_THREADS, env->smem_bytes_hplan));
+        if (per < 1 || per_span < 1) { return fail(SM_ERR_CUDA, "the human's braking-check planning kernel does not fit on an SM"); }
         env->grid_hplan = sms * per;
+        env->grid_hplan_span = sms * per_span;
     }
     // big batches step as two env ranges side by side: the latency-bound tails of one range's kernels (the longest
     // position-bound solve, the last GJK pairs) hide behind the other's (Space, 65 536 envs: 799 -> 748 us per step)
@@ -1098,7 +1130,7 @@ extern "C" int smenv_destroy(SmEnv* env) {
     cudaFree(env->d_pool_verdict); cudaFree(env->d_pool_entry); cudaFree(env->d_pool_dest); cudaFree(env->d_pool_scratch);
     cudaFree(env->d_risk); cudaFree(env->d_backup); cudaFree(env->d_exec); cudaFree(env->d_risky); cudaFree(env->d_gate_list);
     cudaFree(env->d_hpairs); cudaFree(env->d_hthresh); cudaFree(env->d_hrange); cudaFree(env->d_hbacc); cudaFree(env->d_hposes);
-    cudaFree(env->d_hbinfo); cudaFree(env->d_hunits); cudaFree(env->d_hscratch); cudaFree(env->d_hpolicy); cudaFree(env->d_hstart_pool); cudaFree(env->d_hpool_brake); cudaFree(env->d_hpool_bcount); cudaFree(env->d_htarget_pool);
+    cudaFree(env->d_hbinfo); cudaFree(env->d_hunits); cudaFree(env->d_hfine); cudaFree(env->d_hscratch); cudaFree(env->d_hpolicy); cudaFree(env->d_hstart_pool); cudaFree(env->d_hpool_brake); cudaFree(env->d_hpool_bcount); cudaFree(env->d_htarget_pool);
     for (int i = 0; i <= SM_K_COUNT; ++i) if (env->ev[i]) cudaEventDestroy(env->ev[i]);
     for (int c = 0; c < 8; ++c) {
         if (env->chunk_streams[c]) cudaStreamDestroy(env->chunk_streams[c]);
@@ -1657,6 +1689,7 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
         HA.poses = env->d_hposes + (size_t)e0 * SM_HBRAKE_POSES * 8;
         HA.binfo = env->d_hbinfo + (size_t)e0 * 4;
         HA.units = env->d_hunits + (size_t)e0 * SM_HBRAKE_POSES + chunk;
+        HA.fine = env->d_hfine + (size_t)e0 * SM_HBRAKE_POSES + chunk;
         HA.hscratch = env->d_hscratch + (size_t)e0 * SM_SCRATCH_FLOATS;
         HA.scratch = scratch;
         HA.items = items; HA.item_count = worklist; HA.capacity = capacity; HA.overflow = worklist + 1;
@@ -1701,12 +1734,16 @@ static int step_chain(SmEnv* env, const SmBuffers& bv, int e0, int m, int chunk,
         env->launches += 5;
         SM_MARK(SM_K_HUMAN_BRAKE_PLAN);
         if (env->host_scene.hu.check_braking) {
-            human_brake_plan_kernel<<<env->grid_hplan, HBP_THREADS, env->smem_bytes_hplan, stream>>>(HA);
+            // span pass over runs of HBP_SPAN poses, then the per-pose pass over the poses of the spans it could not clear
+            human_brake_plan_kernel<true><<<env->grid_hplan_span, HBP_THREADS, env->smem_bytes_hplan, stream>>>(HA);
+            HumanArgs HF = HA;
+            HF.units = HA.fine;
+            human_brake_plan_kernel<false><<<env->grid_hplan, HBP_THREADS, env->smem_bytes_hplan, stream>>>(HF);
             SM_MARK(SM_K_HUMAN_BRAKE_GJK);
             GjkArgs GB;
             GB.items = items; GB.n_items = worklist; GB.capacity = capacity; GB.res = res; GB.counters = env->d_counters;
             launch_gjk(env, GB, stream);
-            env->launches += 2;
+            env->launches += 3;
         }
         else SM_MARK(SM_K_HUMAN_BRAKE_GJK);
         CU(cudaMemsetAsync(worklist, 0, sizeof(int), stream));   // the items of the braking check are consumed
@@ -2210,7 +2247,7 @@ extern "C" int smenv_counters(SmEnv* env, SmCounters* out, int reset) {
     out->env_steps = h[4]; out->contact_envs = h[5]; out->contact_items = h[6]; out->reserved = h[7];
     out->heavy_joints = h[8]; out->heavy_solves = h[9];
     for (int i = 0; i < 6; ++i) out->aux[i] = h[10 + i];
-    out->brake_poses = h[16]; out->brake_pair_bounds = h[17];
+    out->brake_poses = h[16]; out->brake_pair_bounds = h[17]; out->brake_spans = h[18]; out->brake_fine_poses = h[19];
     if (reset) CU(cudaMemset(env->d_counters, 0, sizeof(h)));
     return SM_OK;
 }
@@ -2662,6 +2699,7 @@ extern "C" int smenv_debug_human_bounds(const SmScene* sc, SmHumanBounds* out) {
         const float* s = u.hf_seg[fi];
         const float dx = s[3] - s[0], dy = s[4] - s[1], dz = s[5] - s[2];
         out->hf_cover_rad[fi] = table_cover_radius(u.hf_rad[fi], sqrtf(dx * dx + dy * dy + dz * dz));
+        for (int j = 0; j < SM_HUMAN_JOINTS; ++j) out->hf_rho[fi][j] = u.hf_rho[fi][j];
     }
     return SM_OK;
 }

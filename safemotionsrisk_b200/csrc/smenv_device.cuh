@@ -116,6 +116,7 @@ struct DevHuman {
     // arm frames 3, 4, 7, 8 (index 0..3): their contiguous shape range and a capsule around all of it (frame coordinates)
     int hf_s0[4], hf_sn[4];
     float hf_seg[4][6], hf_rad[4];
+    float hf_rho[4][SM_HUMAN_JOINTS];     // bound on |d point of arm frame i / d q_j| over its shape centres and capsule ends
     double start_box_min[3], start_box_max[3], kinematic_sampling_probability, stay_in_state_probability,
         min_start_static, min_start_self, tp_min_static, tp_min_self;
 };

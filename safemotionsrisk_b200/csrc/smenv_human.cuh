@@ -8,7 +8,9 @@
 //   joint_kernel .. joint_final    safe range of the 8 human joints and the mapped acceleration (set = 1, deferred advance)
 //   human_brake_traj_kernel        braking trajectory that would follow the step, in joint space
 //                                  (ctlp.py:3155-3207, :3467-3507; utils/braking_trajectory_generator.py:44-93)
-//   human_brake_plan_kernel        FK of every checked pose, bounding-volume culling -> GJK_BRAKE items
+//   human_brake_plan_kernel        span pass: one FK per run of HBP_SPAN poses, volumes inflated by the joint motion
+//                                  inside the run; then the per-pose pass over the runs it could not clear: FK of
+//                                  every such pose, bounding-volume culling -> GJK_BRAKE items
 //   gjk_kernel                     "closer than the safety distance?" per item                             (smenv_gjk.cuh)
 //   human_advance_kernel           adapt_action bookkeeping (ctlp.py:3055-3153, :3000-3024), 24 setpoints + tracked pose
 //   human_outcome_kernel           target point reached? (ctlp.py:2787-2821), new knot bookkeeping, new target point from
@@ -32,7 +34,9 @@ struct HumanArgs {
     double* bacc;              // [n][SM_HBRAKE_STEPS][8] braking accelerations of the trajectory under check
     float* poses;              // [n][SM_HBRAKE_POSES][8] poses the check visits
     int* binfo;                // [n][4] braking steps k, poses, timeout, reserved
-    int* units;                // [0] = count, [1..] = env << 7 | pose: the poses the braking-trajectory check has to test
+    int* units;                // [0] = count, [1..] = hbp_unit(env, first pose, poses): the spans of poses the braking-trajectory
+                               // check has to test (human_brake_plan_kernel<true>), or the single poses (<false>)
+    int* fine;                 // [0] = count, [1..] = hbp_unit(env, pose, 1): the poses of the spans the span pass could not clear
     float* hscratch;           // [n][SM_SCRATCH_FLOATS] sub-step poses of the human (tracked, setpoints)
     const float* scratch;      // [n][SM_SCRATCH_FLOATS] sub-step poses of the robot
     GjkItem* items;
@@ -125,6 +129,17 @@ __device__ __forceinline__ double human_braking_acceleration(const JointLim& L, 
     return e;
 }
 
+#ifndef HBP_SPAN
+#define HBP_SPAN 3   /* consecutive poses of a braking trajectory the span pass of human_brake_plan_kernel tests at once */
+#endif
+static_assert(HBP_SPAN >= 1 && HBP_SPAN <= 8, "the unit word holds the pose count of a span in 3 bits");
+static_assert(SM_HBRAKE_POSES <= 128, "the unit word holds the first pose of a span in 7 bits");
+// unit of the braking-trajectory geometry pass: env in the upper 22 bits, n - 1 in bits 7..9, the first pose in bits 0..6
+#define HBP_MAX_ENVS (1 << 22)
+__host__ __device__ __forceinline__ int hbp_unit(int env, int p0, int n) {
+    return (int)(((unsigned)env << 10) | ((unsigned)(n - 1) << 7) | (unsigned)p0);
+}
+
 #ifndef HBT_MIN_BLOCKS
 #define HBT_MIN_BLOCKS 8   /* resident CTAs per SM the register allocation aims for: 64 registers and 220 B of spill, but 32
                               warps instead of 16 hide the FP64 latency chains (Human step 1547 -> 1483 us; 5, 6: no gain, 10, 12: worse) */
@@ -180,20 +195,28 @@ __global__ void __launch_bounds__(128, HBT_MIN_BLOCKS) human_brake_traj_kernel(H
         if (__all_sync(FULL, done)) break;
     }
     const int npc = valid ? (np < SM_HBRAKE_POSES ? np : SM_HBRAKE_POSES) : 0;   // the same in the eight lanes of the env
+    const int nsp = (npc + HBP_SPAN - 1) / HBP_SPAN;
     int base = 0;
     if (valid && j == 0) {
         int* bi = A.binfo + env * 4;
         bi[0] = k; bi[1] = npc; bi[2] = timeout; bi[3] = 0;
         A.res[env * SM_RES_STRIDE + GJK_BRAKE] = SM_RES_NO_CONTACT;
-        if (A.counters && npc > 0) atomicAdd(&A.counters[16], (unsigned long long)npc);
-        if (npc > 0) base = atomicAdd(A.units, npc);
+        if (A.counters && npc > 0) {
+            atomicAdd(&A.counters[16], (unsigned long long)npc);
+            atomicAdd(&A.counters[18], (unsigned long long)nsp);
+        }
+        if (nsp > 0) base = atomicAdd(A.units, nsp);
     }
+    if (t == 0) A.fine[0] = 0;   // the span pass of this step fills the per-pose list afresh
     base = __shfl_sync(FULL, base, lane & 24);
-    for (int p = j; p < npc; p += 8) A.units[1 + base + p] = ((int)env << 7) | p;   // one unit per pose for the geometry pass
+    for (int s = j; s < nsp; s += 8) {   // one unit per span of up to HBP_SPAN consecutive poses for the geometry pass
+        const int p0 = s * HBP_SPAN, n = npc - p0 < HBP_SPAN ? npc - p0 : HBP_SPAN;
+        A.units[1 + base + s] = hbp_unit((int)env, p0, n);
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// geometry of the braking-trajectory check: ONE THREAD PER POSE (the joint-space kernel lists them).  Serial forward
+// geometry of the braking-trajectory check: ONE THREAD PER POSE (the span pass lists them).  Serial forward
 // kinematics of the two arms; as soon as a frame is known, the bounding-sphere centres of its shapes and the end points
 // of its bounding capsule go to the thread's column of a shared-memory table -- every later test reads points by
 // (uniform) index from there, no transform is applied twice.  Then the link-group pairs of get_minimum_distance
@@ -202,6 +225,11 @@ __global__ void __launch_bounds__(128, HBT_MIN_BLOCKS) human_brake_traj_kernel(H
 // are the cross product of two shape ranges, smenv_create checks it) and the separating-axis bound of the distance
 // planning for what is left.  A pair that may be closer than the safety distance becomes a GJK_BRAKE item carrying
 // the pose number.  The trunk does not move: its shapes' world centres are computed once per CTA.
+// In front of it runs the same kernel as a span pass (SPAN = true): one thread per run of up to HBP_SPAN consecutive poses
+// of an env, the FK of the middle pose, the arm frames' volumes grown by how far their points can move inside the run, the
+// same capsule tests and sphere bounds; no axis bound, no items.  The poses of a run with a sphere-bound survivor are
+// listed for the per-pose pass.  A cleared run has no survivor at any of its poses, so the two passes emit the items the
+// per-pose pass alone would.
 // ------------------------------------------------------------------------------------------------------------------
 // squared distance between the segments [p1, q1] and [p2, q2] (Ericson, Real-Time Collision Detection, 5.1.9)
 __device__ __forceinline__ float segment_dist2(V3 p1, V3 q1, V3 p2, V3 q2) {
@@ -249,11 +277,12 @@ __device__ __forceinline__ void hbp_pick(int f, const Xf& F3, const Xf& F4, cons
     out = f < 0 ? world : f == 0 ? B : f == 3 ? F3 : f == 4 ? F4 : f == 7 ? F7 : F8;
 }
 
+template <bool SPAN>
 __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int n_units = A.units[0];
     if (blockIdx.x * HBP_THREADS >= n_units) return;
-    const int tid = threadIdx.x;
+    const int tid = threadIdx.x, lane = tid & 31;
     const int nas = c_sc.hu.n_arm_shapes, soff = c_sc.hu.shape_off;
     float* P = reinterpret_cast<float*>(smem_raw) + tid;                    // this thread's column: P[(slot * 3 + k) * HBP_THREADS]
     float4* TC = reinterpret_cast<float4*>(smem_raw + (size_t)(nas + 8) * 3 * HBP_THREADS * sizeof(float));
@@ -292,15 +321,42 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
         put(nas + 2 * fi + 1, xf_apply(F, sg[3], sg[4], sg[5]));
     };
     unsigned n_bounds = 0;   // sphere bounds of convex pairs evaluated by this thread (counted in the measurement mode)
+    unsigned n_fine = 0;     // span pass: poses this warp passed on to the per-pose pass (lane 31 counts)
 #pragma unroll 1
     for (int u0 = blockIdx.x * HBP_THREADS; u0 < n_units; u0 += gridDim.x * HBP_THREADS) {
         __syncwarp();   // lanes leave the pair loops of the previous pose at different times
         const int u = u0 + tid;
         const bool valid = u < n_units;   // the loops below are uniform over the warp: idle lanes run them on the last pose
-        const int unit = A.units[1 + (valid ? u : n_units - 1)];
-        const int env = unit >> 7, p = unit & 127;
-        const float4* row = reinterpret_cast<const float4*>(A.poses + ((size_t)env * SM_HBRAKE_POSES + p) * 8);
+        const unsigned unit = (unsigned)A.units[1 + (valid ? u : n_units - 1)];
+        const int env = (int)(unit >> 10), p = (int)(unit & 127u);
+        const int np = SPAN ? (int)((unit >> 7) & 7u) + 1 : 1;
+        const float4* row = reinterpret_cast<const float4*>(A.poses + ((size_t)env * SM_HBRAKE_POSES + p + (np - 1) / 2) * 8);
         const float4 r0 = row[0], r1 = row[1];
+        // span pass: the forward kinematics of the middle pose stands for the span; every point of arm frame i lies within
+        // e_i of where it is at any pose of the span (sum_j max_p |q_p,j - q_mid,j| hf_rho[i][j]), so every volume of
+        // the frame grows by e_i.  A span without a sphere-bound survivor has none at any of its poses.
+        float e_f[4] = {0.f, 0.f, 0.f, 0.f};
+        if constexpr (SPAN) {
+            const float4* row0 = reinterpret_cast<const float4*>(A.poses + ((size_t)env * SM_HBRAKE_POSES + p) * 8);
+            float dq[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll 1
+            for (int i = 0; i < np; ++i) {
+                const float4 a = row0[2 * i], b = row0[2 * i + 1];
+                dq[0] = fmaxf(dq[0], fabsf(a.x - r0.x)); dq[1] = fmaxf(dq[1], fabsf(a.y - r0.y));
+                dq[2] = fmaxf(dq[2], fabsf(a.z - r0.z)); dq[3] = fmaxf(dq[3], fabsf(a.w - r0.w));
+                dq[4] = fmaxf(dq[4], fabsf(b.x - r1.x)); dq[5] = fmaxf(dq[5], fabsf(b.y - r1.y));
+                dq[6] = fmaxf(dq[6], fabsf(b.z - r1.z)); dq[7] = fmaxf(dq[7], fabsf(b.w - r1.w));
+            }
+#pragma unroll
+            for (int fi = 0; fi < 4; ++fi) {
+                float e = 0.f;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) e = fmaf(dq[j], c_sc.hu.hf_rho[fi][j], e);
+                e_f[fi] = e * (1.0f + 1e-5f) + 1e-5f;
+            }
+        }
+        // inflation of arm frame fi (uniform index: selects, no local memory)
+        auto infl = [&](int fi) { return fi == 0 ? e_f[0] : fi == 1 ? e_f[1] : fi == 2 ? e_f[2] : e_f[3]; };
         // frames that carry shapes of the check: upper arm (3 / 7) and forearm + hand (4 / 8) of both arms
         Xf F3, F4, F7, F8;
 #if HBP_INTERLEAVE
@@ -344,7 +400,7 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
             const int fa = c_sc.hu.gp_fa[g], fb = c_sc.hu.gp_fb[g];
             const int fia = hbp_frame_index(fa);
             const V3 a0 = get(nas + 2 * fia), a1 = get(nas + 2 * fia + 1);
-            const float ra = c_sc.hu.hf_rad[fia];
+            const float ra = SPAN ? c_sc.hu.hf_rad[fia] + infl(fia) : c_sc.hu.hf_rad[fia];
             bool near_g;
             if (fb < 0) {    // the table's box against two spheres that cover the capsule of side A
                 const V3 dl = a1 - a0;
@@ -360,7 +416,7 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
                 } else {
                     const int fib = hbp_frame_index(fb);
                     b0 = get(nas + 2 * fib); b1 = get(nas + 2 * fib + 1);
-                    rb = c_sc.hu.hf_rad[fib];
+                    rb = SPAN ? c_sc.hu.hf_rad[fib] + infl(fib) : c_sc.hu.hf_rad[fib];
                 }
                 const float l = ra + rb + safety * (1.0f + 1e-5f) + 1e-5f;
                 near_g = segment_dist2(a0, a1, b0, b1) <= l * l;
@@ -368,18 +424,20 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
             near |= (near_g ? 1u : 0u) << g;
         }
         if (!valid) near = 0u;
+        bool flag = false;   // span pass: some pair of the span survives its sphere bound
 #pragma unroll 1
         for (int g = 0; g < c_sc.hu.n_gp; ++g) {
             __syncwarp();
-            if (!((near >> g) & 1u)) continue;
+            if (!((near >> g) & 1u) || flag) continue;
             const int fa = c_sc.hu.gp_fa[g], fb = c_sc.hu.gp_fb[g];
             const int sa0 = c_sc.hu.gp_a0[g], sa1 = sa0 + c_sc.hu.gp_na[g];
             const int sb0 = c_sc.hu.gp_b0[g], nb = c_sc.hu.gp_nb[g];
-            n_bounds += (unsigned)((sa1 - sa0) * nb);
+            const float eb = SPAN && fb > 0 ? infl(hbp_frame_index(fb)) : 0.f;   // trunk and table do not move
+            if (!SPAN) n_bounds += (unsigned)((sa1 - sa0) * nb);
 #pragma unroll 1
             for (int ia = sa0; ia < sa1; ++ia) {
                 const V3 ca = get(ia - soff);
-                const float la = RM[ia - soff] + safety;
+                const float la = SPAN ? RM[ia - soff] + safety + infl(hbp_frame_index(fa)) : RM[ia - soff] + safety;
                 // sphere bound of the nb pairs (ia, sb0 + k): bit k of `hits` = the pair goes on to the axis bound
                 unsigned hits = 0u;
                 if (fb < 0) {              // the table: sphere against its axis-aligned box
@@ -402,29 +460,50 @@ __global__ void __launch_bounds__(HBP_THREADS) human_brake_plan_kernel(HumanArgs
 #pragma unroll 4
                     for (int k = 0; k < nb; ++k) {
                         const V3 d = get(slot0 + k) - ca;
-                        const float l = la + RM[slot0 + k];
+                        const float l = SPAN ? la + RM[slot0 + k] + eb : la + RM[slot0 + k];
                         hits |= (dot(d, d) <= l * l * (1.0f + 1e-5f) ? 1u : 0u) << k;
                     }
                 }
-                while (hits) {             // rare: the frames are picked out of the registers only here
-                    const int ib = sb0 + __ffs(hits) - 1;
-                    hits &= hits - 1u;
-                    Xf TA, TB;
-                    hbp_pick(fa, F3, F4, F7, F8, B, world, TA);
-                    hbp_pick(fb, F3, F4, F7, F8, B, world, TB);
-                    const DevShape& SA = c_sc.shapes[ia];
-                    const DevShape& SB = c_sc.shapes[ib];
-                    const V3 d = xf_apply(TB, SB.cx, SB.cy, SB.cz) - ca;
-                    if (axis_lower_bound_d(SA, SB, TA, TB, d) <= safety) {
-                        const int idx = atomicAdd(A.item_count, 1);
-                        if (idx < A.capacity) write_item(A.items + idx, env, ia, ib, GJK_BRAKE, p + 1, safety, TA, TB);
-                        else atomicAdd(A.overflow, 1);
+                if constexpr (SPAN) {
+                    if (hits) { flag = true; break; }
+                } else {
+                    while (hits) {             // rare: the frames are picked out of the registers only here
+                        const int ib = sb0 + __ffs(hits) - 1;
+                        hits &= hits - 1u;
+                        Xf TA, TB;
+                        hbp_pick(fa, F3, F4, F7, F8, B, world, TA);
+                        hbp_pick(fb, F3, F4, F7, F8, B, world, TB);
+                        const DevShape& SA = c_sc.shapes[ia];
+                        const DevShape& SB = c_sc.shapes[ib];
+                        const V3 d = xf_apply(TB, SB.cx, SB.cy, SB.cz) - ca;
+                        if (axis_lower_bound_d(SA, SB, TA, TB, d) <= safety) {
+                            const int idx = atomicAdd(A.item_count, 1);
+                            if (idx < A.capacity) write_item(A.items + idx, env, ia, ib, GJK_BRAKE, p + 1, safety, TA, TB);
+                            else atomicAdd(A.overflow, 1);
+                        }
                     }
                 }
             }
         }
+        if constexpr (SPAN) {   // every pose of an uncleared span goes to the per-pose pass, warp-aggregated
+            const int cnt = valid && flag ? np : 0;
+            int incl = cnt;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int x = __shfl_up_sync(FULL, incl, o);
+                if (lane >= o) incl += x;
+            }
+            const int total = __shfl_sync(FULL, incl, 31);
+            if (total) {
+                int base = 0;
+                if (lane == 31) { base = atomicAdd(A.fine, total); n_fine += (unsigned)total; }
+                base = __shfl_sync(FULL, base, 31) + incl - cnt;
+                for (int i = 0; i < cnt; ++i) A.fine[1 + base + i] = hbp_unit(env, p + i, 1);
+            }
+        }
     }
     if (A.counters && n_bounds) atomicAdd(&A.counters[17], (unsigned long long)n_bounds);
+    if (A.counters && n_fine) atomicAdd(&A.counters[19], (unsigned long long)n_fine);
 }
 
 // observation of the nested env (observations.py:313-351 with two arms and alternating target points): entries spread over

@@ -437,10 +437,11 @@ int smenv_kernel_times(SmEnv* env, double* ms_out /* SM_K_COUNT */, int* steps_o
  * cores.  which: SM_NET_RISK = risk(obs, action) -> [0, 1]; SM_NET_BACKUP = backup policy, obs -> action mean.
  * dims = { n_in, N_1 .. N_n_tc, n_out }: n_tc hidden Dense layers (widths 16, 32, 48, 64, 128, 192, 256 or 512) and
  * one output Dense layer (n_out <= 16; SM_NET_HUMAN: the human's stochastic policy, means and log-std outputs,
- * ctlp.py:4647-4762).  weights (host, float32, Keras layout): per layer kernel [in][out] row-major
- * followed by its bias.  hidden_act: 0 selu, 1 swish; out_act: 0 sigmoid, 1 tanh.
+ * ctlp.py:4647-4762; SM_NET_AGENT: the policy that acts in the env, see smenv_step_agent).  weights (host, float32,
+ * Keras layout): per layer kernel [in][out] row-major followed by its bias.  hidden_act: 0 selu, 1 swish; out_act:
+ * 0 sigmoid, 1 tanh.
  */
-enum SmNet { SM_NET_RISK = 0, SM_NET_BACKUP = 1, SM_NET_HUMAN = 2, SM_NET_COUNT = 3 };
+enum SmNet { SM_NET_RISK = 0, SM_NET_BACKUP = 1, SM_NET_HUMAN = 2, SM_NET_AGENT = 3, SM_NET_COUNT = 4 };
 int smenv_mlp_load(SmEnv* env, int which, int n_tc, const int32_t* dims, int hidden_act, int out_act,
                    const float* weights);
 /* out[n][out_stride] = net([in0 row, in1 row]) for n rows; all device pointers (in1 may be NULL with in1_w = 0).  Every
@@ -523,6 +524,27 @@ int smenv_mlp_forward_exact(SmEnv* env, int which, const float* in0, int in0_w, 
 /* Writes the U(-1,1) actions smenv_step_random would use for the next step into buf->actions (so that the gate can be
  * applied to them; follow with smenv_step). */
 int smenv_random_actions(SmEnv* env, const SmBuffers* buf, SmStream stream);
+
+/* The agent: the policy that acts in the env (a task policy, or the backup policy as the agent), a Keras fcnet loaded
+ * into slot SM_NET_AGENT with a tanh output layer of 2 n_joints outputs -- the means, then the log-std pre-activations t
+ * (keras_fcnet_last_layer_activation.py:187-202).  smenv_set_agent_head sets the log_std_range of its head:
+ * log_std = lo + (t + 1) / 2 (hi - lo); default -1.375 / 0.0 (the shipped human policy's params.json).  SM_ERR_ARG if
+ * lo > hi. */
+int smenv_set_agent_head(SmEnv* env, float log_std_lo, float log_std_hi);
+/* One env step (as smenv_step) whose proposed actions come from the agent on buf->obs (the full observation, target-point
+ * entries included).  Per env range, before everything else of the step: the agent's network on the tensor cores, then
+ * its DiagGaussian head.  explore != 0: sample = mean + exp(log_std) eps, eps ~ N(0, 1) from the Philox stream (env index,
+ * step counter, joint, 0xA6E7) -- the step counter is the one smenv_step_random would use -- and
+ * logp = -1/2 sum eps^2 - sum log_std - n_joints/2 log(2 pi), RLlib's DiagGaussian log-likelihood of the UNCLIPPED sample
+ * (summed over the joints in order, bit-reproducible).  explore = 0: sample = mean, logp = 0 (RLlib's convention for
+ * explore=False).  buf->actions = clip(sample, -1, 1) (RLlib's clip_actions): with the risk gate on it is the proposal the
+ * gate rates and keeps, as in smenv_step.  Optional device outputs (NULL: not written): sample_out [N][n_joints],
+ * logp_out [N], dist_out [N][2 n_joints] = mean, log_std (RLlib's action_dist_inputs).  In the measurement mode the agent
+ * runs untimed before the timed step.  SM_ERR_ARG if buf->obs or buf->actions is NULL; SM_ERR_STATE if no agent is
+ * loaded, its input width is not the observation size or its output count is not 2 n_joints.  smenv_step_host does not
+ * run the agent. */
+int smenv_step_agent(SmEnv* env, const SmBuffers* buf, int auto_reset, int explore, float* sample_out, float* logp_out,
+                     float* dist_out, SmStream stream);
 
 /* Measured peaks of the FP32 and FP64 FMA pipes of `device` in TFLOP/s (a micro-benchmark of dependent-free FMA chains
  * on all SMs): the denominators of bench.py's roofline for the vector-pipe-bound kernels. */

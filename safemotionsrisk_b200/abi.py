@@ -29,7 +29,7 @@ SM_OBST_NONE, SM_OBST_PLANET, SM_OBST_BALL, SM_OBST_HUMAN = 0, 1, 2, 3
 SM_HUMAN_JOINTS, SM_MAX_OBST_FRAMES, SM_MAX_HLINKS, SM_MAX_HPAIRS, SM_HBRAKE_STEPS, SM_HBRAKE_POSES = 8, 9, 16, 256, 24, 72
 SM_HSTATE_STRIDE, SM_HOBS_STRIDE = 32, 40
 HTP_SAMPLE_NEW, HTP_REACHED, HS_BRAKE_COUNT, HS_DRAWS, HS_BRAKED, HS_STEPS = 10, 11, 24, 25, 26, 27
-SM_NET_RISK, SM_NET_BACKUP, SM_NET_HUMAN = 0, 1, 2
+SM_NET_RISK, SM_NET_BACKUP, SM_NET_HUMAN, SM_NET_AGENT = 0, 1, 2, 3
 
 # termination reasons (safe_motions_base.py:64-70)
 TERMINATION_UNSET = -1
@@ -212,5 +212,5 @@ EXPORTED_SYMBOLS = [
     "smenv_set_seed", "smenv_set_risk_gate", "smenv_set_human_actions_external", "smenv_set_human_state",
     "smenv_human_pool_sizes", "smenv_copy_human_pools", "smenv_measure_fma_peaks", "smenv_launch_config", "smenv_set_gate_exact", "smenv_mlp_forward_exact",
     "smenv_set_risk_lookahead", "smenv_set_risk_next_state", "smenv_set_initial_backup_check",
-    "smenv_initial_backup_check_counts", "smenv_mlp_shape",
+    "smenv_initial_backup_check_counts", "smenv_mlp_shape", "smenv_set_agent_head", "smenv_step_agent",
 ]

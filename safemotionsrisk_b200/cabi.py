@@ -64,6 +64,8 @@ def load():
     lib.smenv_set_initial_backup_check.argtypes = [vp, i32, vp]
     lib.smenv_initial_backup_check_counts.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
     lib.smenv_random_actions.argtypes = [vp, C.POINTER(abi.SmBuffers), vp]
+    lib.smenv_set_agent_head.argtypes = [vp, C.c_float, C.c_float]
+    lib.smenv_step_agent.argtypes = [vp, C.POINTER(abi.SmBuffers), i32, i32, vp, vp, vp, vp]
     lib.smenv_kernel_timing.argtypes = [vp, i32]
     lib.smenv_kernel_times.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(i32), i32]
     if lib.smenv_sizeof_scene() != C.sizeof(abi.SmScene) or lib.smenv_sizeof_shape() != C.sizeof(abi.SmShape):

@@ -212,13 +212,15 @@ struct SmEnv {
     size_t smem_bytes_gjk = 0;
     int grid_gjk = 0;
     int gjk_threads = GJK_THREADS;   // 512 when only one CTA of the GJK kernel fits on an SM
-    MlpNet nets[SM_NET_COUNT];   // risk network, backup policy, human policy (smenv_mlp_load)
+    MlpNet nets[SM_NET_COUNT];   // risk network, backup policy, human policy, agent (smenv_mlp_load)
     bool net_loaded[SM_NET_COUNT] = {};
     std::vector<void*> net_allocs;
     float* d_risk = nullptr;     // [n] risk of the proposed action
     float* d_backup = nullptr;   // [n][MLP_MAX_OUT] action mean of the backup policy
     float* d_exec = nullptr;     // [n][n_joints] actions executed when the gate is on (smenv_set_risk_gate)
     uint8_t* d_risky = nullptr;  // [n] 1 where the gate replaced the action
+    float* d_agent = nullptr;    // [n][MLP_MAX_OUT] outputs of the agent (smenv_step_agent)
+    float agent_lo = -1.375f, agent_hi = 0.0f;   // log_std_range of the agent's head (smenv_set_agent_head)
     float gate_threshold = -1.0f;  // < 0: gate off
     int* d_gate_list = nullptr;    // [0..15] counters (two per env range), then [n] near-threshold rows, [n] risky rows
     int gate_exact = 1;            // re-rate near-threshold rows and compute the backup actions in float32 (smenv_set_gate_exact)
@@ -1129,6 +1131,7 @@ extern "C" int smenv_destroy(SmEnv* env) {
     for (void* q : env->la_allocs) cudaFree(q);
     cudaFree(env->d_pool_verdict); cudaFree(env->d_pool_entry); cudaFree(env->d_pool_dest); cudaFree(env->d_pool_scratch);
     cudaFree(env->d_risk); cudaFree(env->d_backup); cudaFree(env->d_exec); cudaFree(env->d_risky); cudaFree(env->d_gate_list);
+    cudaFree(env->d_agent);
     cudaFree(env->d_hpairs); cudaFree(env->d_hthresh); cudaFree(env->d_hrange); cudaFree(env->d_hbacc); cudaFree(env->d_hposes);
     cudaFree(env->d_hbinfo); cudaFree(env->d_hunits); cudaFree(env->d_hfine); cudaFree(env->d_hscratch); cudaFree(env->d_hpolicy); cudaFree(env->d_hstart_pool); cudaFree(env->d_hpool_brake); cudaFree(env->d_hpool_bcount); cudaFree(env->d_htarget_pool);
     for (int i = 0; i <= SM_K_COUNT; ++i) if (env->ev[i]) cudaEventDestroy(env->ev[i]);
@@ -1950,15 +1953,46 @@ static int gate_net_check(const SmEnv* env, RiskCheck mode, const char* who) {
                                                       : ": the network gate needs a state-action risk network"));
 }
 
-// One env step over the envs [e0, e0 + m) on `stream` with the work lists of slot `chunk` (step_chain): with the gate on
-// (actions.py:303-340) the proposed actions are rated first -- by the risk network, by the look-ahead, or by the state risk
-// network on the simulated next state -- and the backup policy's action is executed where they are risky.
+// What smenv_step_agent asks of the agent: explore or not, and where its samples, log-likelihoods and distribution inputs go
+// (whole-env arrays, each may be NULL).
+struct AgentStep { int explore; float* sample; float* logp; float* dist; };
+
+// The agent proposes the actions of the envs of `bv` (a view of m envs starting at env e0): its network on the full
+// observation bv.obs on the tensor cores, then its DiagGaussian head into bv.actions.  Philox stream (global env index,
+// step counter, joint, 0xA6E7).
+static int agent_launch(SmEnv* env, const SmBuffers& bv, int e0, int m, uint32_t step_counter, const AgentStep& ag,
+                        cudaStream_t stream) {
+    const int nj = env->host_scene.n_joints, ow = env->host_scene.obs_size;
+    float* out = env->d_agent + (size_t)e0 * MLP_MAX_OUT;
+    const MlpSeg none{nullptr, 0, 0};
+    if (int rc = mlp_launch(env, SM_NET_AGENT, MlpSeg{bv.obs, ow, ow}, none, none, out, MLP_MAX_OUT, m, stream)) return rc;
+    AgentArgs A;
+    A.policy_out = out; A.actions = const_cast<float*>(bv.actions);
+    A.sample = ag.sample ? ag.sample + (size_t)e0 * nj : nullptr;
+    A.logp = ag.logp ? ag.logp + e0 : nullptr;
+    A.dist = ag.dist ? ag.dist + (size_t)e0 * 2 * nj : nullptr;
+    A.n = m; A.nj = nj; A.env_base = e0; A.explore = ag.explore;
+    A.step_counter = step_counter; A.k0 = (uint32_t)env->seed; A.k1 = (uint32_t)(env->seed >> 32);
+    A.lo = env->agent_lo; A.span = env->agent_hi - env->agent_lo;
+    agent_action_kernel<<<(m * 8 + 255) / 256, 256, 0, stream>>>(A);
+    env->launches++;
+    CU(cudaGetLastError());
+    return SM_OK;
+}
+
+// One env step over the envs [e0, e0 + m) on `stream` with the work lists of slot `chunk` (step_chain): with an agent
+// (smenv_step_agent) it proposes the actions first; with the gate on (actions.py:303-340) the proposed actions are rated
+// -- by the risk network, by the look-ahead, or by the state risk network on the simulated next state -- and the backup
+// policy's action is executed where they are risky.
 static int step_range(SmEnv* env, const SmBuffers* full, int e0, int m, int chunk, int auto_reset, int random_actions,
-                      uint32_t step_counter, bool tk, cudaStream_t stream, const uint32_t* step_ptr = nullptr) {
+                      uint32_t step_counter, bool tk, cudaStream_t stream, const uint32_t* step_ptr = nullptr,
+                      const AgentStep* agent = nullptr) {
     const SmBuffers buf_v = buffers_at(*full, e0, env->host_scene.n_joints, env->host_scene.obs_size);
     const SmBuffers* buf = &buf_v;
     const bool gate = env->gate_threshold >= 0.0f;
     float* exec = nullptr;
+    if (agent)
+        if (int rc = agent_launch(env, buf_v, e0, m, step_counter, *agent, stream)) return rc;
     if (gate) {
         if (!buf->obs) return fail(SM_ERR_ARG, "smenv_step: the risk gate needs the observation buffer");
         if (int rc = gate_net_check(env, env->risk_check, "smenv_step")) return rc;
@@ -2025,7 +2059,8 @@ static int step_check(SmEnv* env, const SmBuffers* buf, int auto_reset, bool nee
     return SM_OK;
 }
 
-static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int random_actions, SmStream s) {
+static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int random_actions, SmStream s,
+                     const AgentStep* agent = nullptr) {
     int rc = step_check(env, buf, auto_reset, !random_actions);
     if (rc) return rc;
     cudaStream_t stream = (cudaStream_t)s;
@@ -2040,7 +2075,7 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
     if (rc) return rc;
     const uint32_t counter = env->step_counter++;
     if (ranges == 1) {
-        rc = step_range(env, buf, 0, env->n, 0, auto_reset, random_actions, counter, tk, stream);
+        rc = step_range(env, buf, 0, env->n, 0, auto_reset, random_actions, counter, tk, stream, nullptr, agent);
         if (rc) return rc;
     } else {   // env ranges side by side on internal streams: the latency-bound tails of one range hide behind the other
         rc = ensure_chunk_streams(env);
@@ -2051,7 +2086,8 @@ static int step_impl(SmEnv* env, const SmBuffers* buf, int auto_reset, int rando
             const int e0 = c * per, m = e0 + per <= env->n ? per : env->n - e0;
             if (m <= 0) break;
             CU(cudaStreamWaitEvent(env->chunk_streams[c], env->chunk_fork, 0));
-            rc = step_range(env, buf, e0, m, c, auto_reset, random_actions, counter, false, env->chunk_streams[c]);
+            rc = step_range(env, buf, e0, m, c, auto_reset, random_actions, counter, false, env->chunk_streams[c], nullptr,
+                            agent);
             if (rc) return rc;
             CU(cudaEventRecord(env->chunk_done[c], env->chunk_streams[c]));
             CU(cudaStreamWaitEvent(stream, env->chunk_done[c], 0));
@@ -2190,6 +2226,27 @@ extern "C" int smenv_step(SmEnv* env, const SmBuffers* buf, int auto_reset, SmSt
 extern "C" int smenv_step_random(SmEnv* env, const SmBuffers* buf, int auto_reset, SmStream s) {
     return step_impl(env, buf, auto_reset, 1, s);
 }
+extern "C" int smenv_set_agent_head(SmEnv* env, float log_std_lo, float log_std_hi) {
+    if (!env) return fail(SM_ERR_ARG, "smenv_set_agent_head: null env");
+    if (!(log_std_lo <= log_std_hi)) return fail(SM_ERR_ARG, "smenv_set_agent_head: log_std_lo must not exceed log_std_hi");
+    env->agent_lo = log_std_lo; env->agent_hi = log_std_hi;
+    return SM_OK;
+}
+extern "C" int smenv_step_agent(SmEnv* env, const SmBuffers* buf, int auto_reset, int explore, float* sample_out,
+                                float* logp_out, float* dist_out, SmStream s) {
+    if (!env || !buf) return fail(SM_ERR_ARG, "smenv_step_agent: null argument");
+    if (!buf->obs || !buf->actions) return fail(SM_ERR_ARG, "smenv_step_agent: the agent needs the observation and action buffers");
+    if (!env->net_loaded[SM_NET_AGENT]) return fail(SM_ERR_STATE, "smenv_step_agent: no agent loaded (smenv_mlp_load, SM_NET_AGENT)");
+    const MlpNet& net = env->nets[SM_NET_AGENT];
+    if (net.n_in != env->host_scene.obs_size)
+        return fail(SM_ERR_STATE, "smenv_step_agent: the agent takes " + std::to_string(net.n_in) +
+                                      " inputs, the observation has " + std::to_string(env->host_scene.obs_size));
+    if (net.n_out != 2 * env->host_scene.n_joints)
+        return fail(SM_ERR_STATE, "smenv_step_agent: the agent has " + std::to_string(net.n_out) + " outputs, the head needs " +
+                                      std::to_string(2 * env->host_scene.n_joints) + " (means, then log-std)");
+    const AgentStep agent{explore != 0, sample_out, logp_out, dist_out};
+    return step_impl(env, buf, auto_reset, 0, s, &agent);
+}
 
 extern "C" int smenv_safe_range(SmEnv* env, const double* kin, double* lo, double* hi, int32_t* code, int n, SmStream s) {
     if (!env || !kin || !lo || !hi || !code) return fail(SM_ERR_ARG, "smenv_safe_range: null argument");
@@ -2327,6 +2384,7 @@ extern "C" int smenv_mlp_load(SmEnv* env, int which, int n_tc, const int32_t* di
     }
     env->nets[which] = net;
     env->net_loaded[which] = true;
+    if (which == SM_NET_AGENT && !env->d_agent) CU(cudaMalloc((void**)&env->d_agent, (size_t)env->n * MLP_MAX_OUT * sizeof(float)));
     if (!env->d_risk) {
         CU(cudaMalloc((void**)&env->d_risk, (size_t)env->n * sizeof(float)));
         CU(cudaMalloc((void**)&env->d_backup, (size_t)env->n * MLP_MAX_OUT * sizeof(float)));

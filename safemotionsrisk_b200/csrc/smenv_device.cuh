@@ -514,6 +514,18 @@ __device__ __forceinline__ double u01d(uint32_t hi, uint32_t lo) {
     return ((double)(hi >> 5) * 67108864.0 + (double)(lo >> 6)) * (1.0 / 9007199254740992.0);
 }
 
+// One joint of the DiagGaussian head of a Keras-fcnet policy (keras_fcnet_last_layer_activation.py:187-202): the tanh
+// output t of the log-std column is remapped to log_std = lo + (t + 1) / 2 * span (span = hi - lo, the log_std_range of
+// params.json), eps ~ N(0, 1) by Box-Muller from the first two words of a Philox draw; returns the unclipped sample
+// mean + exp(log_std) * eps.  Shared by the human's policy and the agent (the human's actions depend on its exact form).
+__device__ __forceinline__ float diag_gaussian_sample(float mean, float t, float lo, float span, uint4 r, float& log_std,
+                                                      float& eps) {
+    log_std = lo + 0.5f * (t + 1.0f) * span;
+    const float u1 = fmaxf(u01f(r.x), 5.9604645e-8f), u2 = u01f(r.y);
+    eps = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);   // Box-Muller
+    return mean + expf(log_std) * eps;
+}
+
 // per-warp sampling stream: every draw advances the counter; all lanes get the same numbers
 struct Rng {
     uint32_t k0, k1, c0, c1, n;

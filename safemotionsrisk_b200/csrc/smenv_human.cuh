@@ -64,13 +64,13 @@ __global__ void human_action_kernel(HumanArgs A) {
     const int env = t >> 3, j = t & 7;
     if (env >= A.n) return;
     const float* o = A.policy_out + (size_t)env * 16;
-    const float mean = o[j];
-    const float log_std = (float)c_sc.hu.log_std_lo + 0.5f * (o[8 + j] + 1.0f) * (float)(c_sc.hu.log_std_hi - c_sc.hu.log_std_lo);
+    const float mean = o[j], t_log_std = o[8 + j];
     const uint32_t step = A.step_ptr ? __ldg(A.step_ptr) + A.step_offset : A.step_counter;
     const uint4 r = philox((uint32_t)(env + A.env_base), step, (uint32_t)j, 0x4057u, A.k0, A.k1);
-    const float u1 = fmaxf(u01f(r.x), 5.9604645e-8f), u2 = u01f(r.y);
-    const float eps = sqrtf(-2.0f * logf(u1)) * cospif(2.0f * u2);   // Box-Muller
-    A.buf.hactions[(size_t)env * SM_HUMAN_JOINTS + j] = fminf(1.0f, fmaxf(-1.0f, mean + expf(log_std) * eps));
+    float log_std, eps;
+    const float sample = diag_gaussian_sample(mean, t_log_std, (float)c_sc.hu.log_std_lo,
+                                              (float)(c_sc.hu.log_std_hi - c_sc.hu.log_std_lo), r, log_std, eps);
+    A.buf.hactions[(size_t)env * SM_HUMAN_JOINTS + j] = fminf(1.0f, fmaxf(-1.0f, sample));
 }
 
 // ------------------------------------------------------------------------------------------------------------------

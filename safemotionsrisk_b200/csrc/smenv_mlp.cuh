@@ -392,6 +392,52 @@ __global__ void random_actions_kernel(float* actions, int nj, int n, int env_bas
     actions[t] = 2.0f * u01f(r.x) - 1.0f;
 }
 
+// The agent's DiagGaussian head (smenv_step_agent): thread = (env, joint), the eight lanes of an env side by side.
+struct AgentArgs {
+    const float* policy_out;   // [n][MLP_MAX_OUT] tanh outputs of the agent: nj means, then nj log-std pre-activations
+    float* actions;            // [n][nj] clip(sample, -1, 1): what the env executes (or the gate rates)
+    float* sample;             // [n][nj] unclipped sample, or NULL
+    float* logp;               // [n] log-likelihood of the unclipped sample, or NULL
+    float* dist;               // [n][2 nj] mean, log_std, or NULL
+    int n, nj, env_base, explore;
+    uint32_t step_counter, k0, k1;
+    float lo, span;            // log_std = lo + (t + 1) / 2 * span
+};
+
+__global__ void agent_action_kernel(AgentArgs A) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int env = t >> 3, j = t & 7;
+    const bool live = env < A.n && j < A.nj;
+    float eps = 0.0f, log_std = 0.0f;
+    if (live) {
+        const float* o = A.policy_out + (size_t)env * MLP_MAX_OUT;
+        const float mean = o[j];
+        float sample = mean;
+        if (A.explore) {
+            const uint4 r = philox((uint32_t)(env + A.env_base), A.step_counter, (uint32_t)j, 0xA6E7u, A.k0, A.k1);
+            sample = diag_gaussian_sample(mean, o[A.nj + j], A.lo, A.span, r, log_std, eps);
+        } else {
+            log_std = A.lo + 0.5f * (o[A.nj + j] + 1.0f) * A.span;
+        }
+        A.actions[(size_t)env * A.nj + j] = fminf(1.0f, fmaxf(-1.0f, sample));   // RLlib's clip_actions
+        if (A.sample) A.sample[(size_t)env * A.nj + j] = sample;
+        if (A.dist) {
+            A.dist[(size_t)env * 2 * A.nj + j] = mean;
+            A.dist[(size_t)env * 2 * A.nj + A.nj + j] = log_std;
+        }
+    }
+    // DiagGaussian logp of the unclipped sample, summed by lane 0 of the env over the joints in order (bit-reproducible);
+    // explore = 0 reports 0 (RLlib's StochasticSampling with explore=False).  Every lane of the warp takes part.
+    float sq = 0.0f, ls = 0.0f;
+    for (int k = 0; k < A.nj; ++k) {
+        const float e = __shfl_sync(FULL, eps, k, 8), l = __shfl_sync(FULL, log_std, k, 8);
+        sq = fmaf(e, e, sq);
+        ls += l;
+    }
+    if (j == 0 && env < A.n && A.logp)
+        A.logp[env] = A.explore ? -0.5f * sq - ls - 0.91893853320467274f * (float)A.nj : 0.0f;   // 0.5 log(2 pi) per joint
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // Exact (float32, CUDA cores) evaluation of a network on a LIST of rows: the tensor-core pass rates every env with fp16
 // operands; rows whose risk lies within a band around the threshold are re-rated here so that the gate decision equals the

@@ -682,6 +682,97 @@ class SafeMotionsVecEnv:
                                                out.data_ptr(), n_out, n, self._stream()), "smenv_mlp_forward")
         return out
 
+    # ------------------------------------------------------------------ the agent: the policy that acts in the env
+    def load_agent(self, source=None, log_std_range=(-1.375, 0.0), hidden_activation="swish"):
+        """Loads the policy that acts in the env (smenv_mlp_load into SM_NET_AGENT), a Keras fcnet with a DiagGaussian
+        head (keras_fcnet_last_layer_activation.py:86-136, :187-202): hidden Dense layers (swish, or selu), then a tanh
+        Dense layer of 2 n_joints outputs, the means followed by the log-std pre-activations t, remapped to
+        log_std = lo + (t + 1) / 2 (hi - lo) with log_std_range = (lo, hi) (smenv_set_agent_head).  source: an .npz with
+        agent/fc_1/kernel, agent/fc_1/bias, ... agent/fc_out/bias, or None for the scene's packaged backup policy with all
+        its outputs.  The agent sees the full observation (target-point entries included).  Raises ValueError if the
+        input width is not the observation size or the output count is not 2 n_joints."""
+        if hidden_activation not in ("swish", "selu"):
+            raise ValueError("hidden_activation must be 'swish' or 'selu', not {!r}".format(hidden_activation))
+        lo, hi = (float(x) for x in log_std_range)
+        if lo > hi:
+            raise ValueError("log_std_range ({}, {}): the lower end exceeds the upper".format(lo, hi))
+        if source is None:
+            scene = "human" if self.has_human else "ball" if self.config.use_moving_objects else "space"
+            source = os.path.join(os.path.dirname(os.path.abspath(__file__)), "assets", "networks_{}.npz".format(scene))
+            prefix = "backup"
+        else:
+            prefix = "agent"
+        w = np.load(source)
+        names, i = [], 1
+        while "{}/fc_{}/kernel".format(prefix, i) in w.files:
+            names.append("fc_{}".format(i))
+            i += 1
+        names.append("fc_out")
+        if "{}/fc_out/kernel".format(prefix) not in w.files or len(names) < 2:
+            raise ValueError("{}: expected {}/fc_1 ... {}/fc_out kernels and biases".format(source, prefix, prefix))
+        layers = [(w["{}/{}/kernel".format(prefix, k)], w["{}/{}/bias".format(prefix, k)]) for k in names]
+        nj, d = self.scene.n_joints, self.scene.obs_size
+        if layers[0][0].shape[0] != d:
+            raise ValueError("{}: the agent takes {} inputs, the env's observation has {}".format(
+                source, layers[0][0].shape[0], d))
+        if layers[-1][0].shape[1] != 2 * nj:
+            raise ValueError("{}: the agent has {} outputs, its head needs 2 x {} (means, then log-std)".format(
+                source, layers[-1][0].shape[1], nj))
+        dims = np.array([layers[0][0].shape[0]] + [k.shape[1] for k, _ in layers], dtype=np.int32)
+        flat = np.concatenate([np.concatenate([k.astype(np.float32).ravel(), b.astype(np.float32).ravel()])
+                               for k, b in layers])
+        cabi.check(self._lib.smenv_mlp_load(self._handle, abi.SM_NET_AGENT, len(layers) - 1, dims.ctypes.data,
+                                            0 if hidden_activation == "selu" else 1, 1, flat.ctypes.data),
+                   "smenv_mlp_load")
+        cabi.check(self._lib.smenv_set_agent_head(self._handle, lo, hi), "smenv_set_agent_head")
+        n, dev = self.num_envs, self.device
+        self.agent_actions = torch.zeros((n, nj), dtype=torch.float32, device=dev)
+        self.agent_logp = torch.zeros(n, dtype=torch.float32, device=dev)
+        self.agent_dist_inputs = torch.zeros((n, 2 * nj), dtype=torch.float32, device=dev)
+
+    def step_agent(self, explore=True):
+        """One env step whose actions come from the agent (load_agent) on the current observation, on the device
+        (smenv_step_agent).  explore=True samples mean + exp(log_std) eps (Philox normal noise), explore=False takes the
+        mean; the env executes the sample clipped to [-1, 1] (through the risk gate when it is on), and self.actions holds
+        that clipped proposal.  self.agent_actions (the unclipped samples), self.agent_logp (their DiagGaussian
+        log-likelihood; 0 with explore=False) and self.agent_dist_inputs (mean, log_std) describe the step's actions and
+        stay valid until the next step.  Returns what step() returns."""
+        cabi.check(self._lib.smenv_step_agent(self._handle, C.byref(self._buf), int(self.auto_reset), int(bool(explore)),
+                                              self.agent_actions.data_ptr(), self.agent_logp.data_ptr(),
+                                              self.agent_dist_inputs.data_ptr(), self._stream()), "smenv_step_agent")
+        self._after_step()
+        return self._outputs()
+
+    def rollout(self, steps, explore=True):
+        """`steps` calls of step_agent, recorded on the device without a host synchronise, under RLlib's SampleBatch
+        names: obs [T, N, D] (the observation each action was computed from), actions [T, N, n_joints] (unclipped),
+        action_logp [T, N], action_dist_inputs [T, N, 2 n_joints], rewards [T, N], dones [T, N] (bool), risky [T, N]
+        (bool; only while the risk gate is on), and last_obs [N, D], the observation after the last step.  With auto_reset
+        an env that is done starts its next episode in the next row."""
+        T, n, nj, d = int(steps), self.num_envs, self.scene.n_joints, self.scene.obs_size
+        dev = self.device
+        out = dict(obs=torch.empty((T, n, d), dtype=torch.float32, device=dev),
+                   actions=torch.empty((T, n, nj), dtype=torch.float32, device=dev),
+                   action_logp=torch.empty((T, n), dtype=torch.float32, device=dev),
+                   action_dist_inputs=torch.empty((T, n, 2 * nj), dtype=torch.float32, device=dev),
+                   rewards=torch.empty((T, n), dtype=torch.float32, device=dev),
+                   dones=torch.empty((T, n), dtype=torch.bool, device=dev))
+        gate = self._gate_threshold is not None
+        if gate:
+            out["risky"] = torch.empty((T, n), dtype=torch.bool, device=dev)
+        for t in range(T):
+            out["obs"][t].copy_(self.obs)
+            self.step_agent(explore)
+            out["actions"][t].copy_(self.agent_actions)
+            out["action_logp"][t].copy_(self.agent_logp)
+            out["action_dist_inputs"][t].copy_(self.agent_dist_inputs)
+            out["rewards"][t].copy_(self.reward)
+            out["dones"][t].copy_(self.done)
+            if gate:
+                out["risky"][t].copy_(self.info[:, abi.INFO["risky_action"]])
+        out["last_obs"] = self.obs.clone()
+        return out
+
     def set_gate_exact(self, exact=True, band=0.0):
         """Exact gate (default on): rows whose tensor-core risk lies within `band` (default 0.01) of the threshold are
         re-rated in float32 and the backup action of the risky rows is computed in float32 (smenv_set_gate_exact)."""
